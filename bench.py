@@ -2,7 +2,7 @@
 """bench.py — the headline benchmark of the B200-native light-transport path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--workload 4k|config1|config2|config3|config5|1080p|8k]
+                    [--workload 4k|config1|config2|config3|config5|1080p|8k] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -18,7 +18,15 @@ the frame is fixed), with the opaque bands exchanged before the mip chain.
          frame constants go host->device from pinned memory and the tonemapped sRGB8 band comes back.
 `--workload`  4k = BASELINE.json configs[3] (the headline, default); config1/2/3/5 = configs[0]/[1]/[2]/[4] at their
          stated sizes (config5: 8K x 64 orbit views; combine with --view-groups for the 8x1/4x2/2x4/1x8 sweep).
-`sustained`  the same frames back to back for >= --min-seconds (default 2 s) with its own clock summary, next to the K-step burst.
+`--steps K`  the number of timed steps of `value` (and of `e2e`, timed separately through host buffers).
+`sustained`  with --min-seconds S > 0: the same frames back to back for >= S seconds with its own clock summary, next to
+         the K-step burst (off by default, so that K alone sets how many steps are timed).
+`--dump-outputs DIR`  after the timed steps, the frame their last step produced, as a caller of tr_frame receives it:
+         DIR/hdr_rgba.npy (the RGBA16F HDR frame, overflows to inf written as the largest finite half, 65504) and
+         DIR/srgb8_rgba.npy (the tonemapped sRGB8 frame), both widened to float32, of the whole frame (N > 1: stitched from the bands; with several views a step, view groups or
+         --emulate-band: rank 0's rows of the last frame it rendered; --impl reference: the rows of its band).  A frame
+         larger than the 64 MB budget is sampled: DUMP_PIXELS pixels chosen by a fixed seed, so that the same arguments
+         give the same pixels.
 `frame_sha256`  SHA-256 of the whole HDR (RGBA16F) and sRGB8 frame, at N > 1 stitched from the ranks' bands: equal at every N
          <=> N-GPU output == 1-GPU output bitwise, checkable from the JSON lines alone.  `band_hashes` are the per-band
          digests (the N = 1 line carries those of the equal-row splits into 2, 4 and 8); `band_rows` the boundaries used —
@@ -359,6 +367,8 @@ def run_reference(args, wl):
     for _ in range(args.warmup):
         cpu.step()
     times = [cpu.step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cpu.runner.hdr16[cpu.y0:cpu.y1], cpu.runner.srgb8[cpu.y0:cpu.y1])
     total = float(sum(times))
     value = cpu.pixels * args.steps / total / 1e6
     line = {
@@ -382,6 +392,29 @@ def run_reference(args, wl):
 def sha256_rows(arr, y0, y1):
     import hashlib
     return hashlib.sha256(np.ascontiguousarray(arr[y0:y1]).tobytes()).hexdigest()
+
+
+DUMP_BYTES = 64_000_000      # --dump-outputs budget, all files together
+DUMP_PIXELS = 1 << 20        # pixels kept of a frame over the budget (2 x 16 MiB of float32 RGBA)
+DUMP_SEED = 0
+
+
+def dump_outputs(dirname, hdr_bits, srgb):
+    """Writes the frame (RGBA16F bits, sRGB8) as float32 .npy files: whole (H, W, 4) when both fit DUMP_BYTES, else the
+    (DUMP_PIXELS, 4) pixels at the ascending flat indices a generator seeded with DUMP_SEED picks.
+
+    Shaded values beyond the range of the RGBA16F target are stored there as +-inf (sun highlights of the bench scenes
+    reach 5e5); they are written as +-65504, the largest finite half, as the tonemapped frame saturates them at 255."""
+    os.makedirs(dirname, exist_ok=True)
+    half_max = float(np.finfo(np.float16).max)
+    hdr = np.clip(np.ascontiguousarray(hdr_bits).view(np.float16).astype(np.float32), -half_max, half_max)
+    out = np.asarray(srgb, np.float32)
+    h, w = hdr.shape[:2]
+    if 2 * hdr.nbytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, DUMP_PIXELS, replace=False))
+        hdr, out = hdr.reshape(-1, 4)[keep], out.reshape(-1, 4)[keep]
+    np.save(os.path.join(dirname, "hdr_rgba.npy"), hdr)
+    np.save(os.path.join(dirname, "srgb8_rgba.npy"), out)
 
 
 def run_b200(args, wl):
@@ -641,6 +674,7 @@ def run_b200(args, wl):
 
     # ------------------------------------------------------------------ band hashes: N-GPU output == 1-GPU output, from the lines
     band_hashes, frame_sha = None, None
+    frame = None   # rank 0: (RGBA16F bits, sRGB8) of the whole frame of the last step, for --dump-outputs
     if args.views == 1 and not args.emulate_band:
         hdr_bits, srgb = r.read_hdr(), r.read_srgb8()
         mine = {"rows": [int(y0), int(y1)], "hdr_rgba16f": sha256_rows(hdr_bits, y0, y1), "srgb8": sha256_rows(srgb, y0, y1)}
@@ -655,13 +689,19 @@ def run_b200(args, wl):
                     import hashlib
                     frame_sha = {"hdr_rgba16f": hashlib.sha256(b"".join(p[0].tobytes() for p in parts)).hexdigest(),
                                  "srgb8": hashlib.sha256(b"".join(p[1].tobytes() for p in parts)).hexdigest()}
+                    frame = (np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts]))
         else:
+            frame = (hdr_bits, srgb)
             frame_sha = {"hdr_rgba16f": sha256_rows(hdr_bits, 0, H), "srgb8": sha256_rows(srgb, 0, H)}
             band_hashes = {}
             for n in (1, 2, 4, 8):
                 rows = [host.band_rows(H, b, n) for b in range(n)]
                 band_hashes[str(n)] = [{"rows": [int(a), int(b)], "hdr_rgba16f": sha256_rows(hdr_bits, a, b), "srgb8": sha256_rows(srgb, a, b)}
                                        for a, b in rows]
+    if args.dump_outputs and rank == 0:
+        if frame is None:   # several views a step, view groups or an emulated band: rank 0's rows of its last frame
+            frame = (r.read_hdr()[y0:y1], r.read_srgb8()[y0:y1])
+        dump_outputs(args.dump_outputs, *frame)
 
     # ------------------------------------------------------------------ roofline of the dominant pass (rank 0's band)
     line = None
@@ -772,8 +812,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ray-tracing", action="store_true",
                     help="ray-queried shadows on (the reference's --ray-tracing option); off for the headline metric")
-    ap.add_argument("--min-seconds", type=float, default=2.0,
-                    help="also run the timed steps back to back for at least this long and report `sustained` (0 = off)")
+    ap.add_argument("--min-seconds", type=float, default=0.0,
+                    help="also run the timed steps back to back for at least this long and report `sustained` (0 = off, the default)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the frame of the last step to DIR/*.npy (float32; sampled above 64 MB)")
     ap.add_argument("--views", type=int, default=None,
                     help="camera views per step (BASELINE configs[4]: 64 orbit views, the default of --workload config5); a step renders all of them")
     ap.add_argument("--view-groups", type=int, default=1,

@@ -7,6 +7,7 @@ imports this module.  Parity: pinned to the reference's compiled shader modules 
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -18,12 +19,28 @@ _VARIANT = "parity"   # "parity": -O2 -ffp-contract=off (the checker); "o3": -O3
 
 
 def build(force=False, variant="parity"):
-    name = "liboracle.so" if variant == "parity" else "liboracle_o3.so"
-    so = os.path.join(_HERE, name)
+    if variant != "parity":
+        return _build_o3(force)
+    so = os.path.join(_HERE, "liboracle.so")
     srcs = [os.path.join(_HERE, f) for f in os.listdir(_HERE) if f.endswith((".c", ".h")) and not f.startswith("spv_")]
     srcs.append(os.path.join(_HERE, "..", "include", "tr_abi.h"))
     if force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in srcs):
-        subprocess.check_call(["make", "-C", _HERE, "-s", name])
+        subprocess.check_call(["make", "-C", _HERE, "-s", "liboracle.so"])
+    return so
+
+
+_O3_DIR = None
+
+
+def _build_o3(force):
+    """The -O3 -march=native timing variant is built when it is asked for, for the CPU it runs on, in a temporary
+    directory of this process (the source tree may be read-only)."""
+    global _O3_DIR
+    if _O3_DIR is None:
+        _O3_DIR = tempfile.TemporaryDirectory(prefix="tr_oracle_o3_")
+    so = os.path.join(_O3_DIR.name, "liboracle_o3.so")
+    if force or not os.path.exists(so):
+        subprocess.check_call(["make", "-C", _HERE, "-s", so, "O3_SO=" + so])
     return so
 
 
