@@ -540,6 +540,38 @@ enum { TR_BUF_OPAQUE_MIP0 = 0, TR_BUF_HDR = 1, TR_BUF_SRGB8 = 2, TR_BUF_HDR_F32 
 TR_API int32_t tr_device_buffer(tr_ctx* ctx, int32_t what, void** device_ptr, size_t* bytes);
 
 /* ------------------------------------------------------------------ */
+/* Multi-GPU in one process: the reference's host is one thread with   */
+/* one queue (src/main.rs:243, 1290-1294); a group lets that thread     */
+/* drive the bands of one frame on up to 8 contexts.                    */
+/* ------------------------------------------------------------------ */
+/* A group joins n contexts (at most 8) of one host thread into the bands of one frame.  Member k becomes rank k of n with
+ * equal-row bands; its opaque pass stores its band into every member's mip 0 through plain device pointers (peer access
+ * between distinct devices, which tr_group_create enables and leaves enabled), and CUDA events order the members, so no
+ * call waits for the GPU inside a frame.  Contexts may share a device: 2..8 members on one GPU run exactly the code 8 GPUs
+ * run.  Members must be distinct, of one size, and in no communicator (tr_comm_init), peer mapping (tr_peer_attach) or
+ * other group.  While the group lives, tr_frame, tr_shade_opaque, tr_allgather_opaque, tr_set_band, tr_set_bands,
+ * tr_resize, tr_comm_init, tr_peer_attach and tr_destroy on a member return TR_ERR_STATE; uploads,
+ * tr_build_acceleration_structures, tr_set_stream, the timers and every tr_read_* stay per member. */
+typedef struct tr_group tr_group;
+/* the device set-up of src/main.rs:243 (one queue) widened to n contexts; distinct devices without peer access in both
+ * directions -> TR_ERR_UNSUPPORTED */
+TR_API int32_t tr_group_create(tr_ctx* const* ctxs, uint32_t n, tr_group** out_group);
+/* LoopDestroyed clean-up (src/main.rs:1416-1445) of the group only: waits for every member, which then renders the whole
+ * frame again as rank 0 of 1 */
+TR_API int32_t tr_group_destroy(tr_group* g);
+/* tr_set_bands for every member at once: n + 1 ascending row boundaries (0 ... height) */
+TR_API int32_t tr_group_set_bands(tr_group* g, const uint32_t* bounds, uint32_t n_bounds);
+/* swapchain-resize path (src/main.rs:996-1166) on every member; the bands return to equal rows */
+TR_API int32_t tr_group_resize(tr_group* g, uint32_t width, uint32_t height);
+/* one record() (src/main.rs:1551-2263) across the members: params[k] is member k's (its own
+ * acceleration_structure_address when ray queries are on; normally the same camera otherwise) */
+TR_API int32_t tr_group_frame(tr_group* g, const tr_frame_params* params);
+/* fence wait (src/main.rs:1290) on every member */
+TR_API int32_t tr_group_sync(tr_group* g);
+/* the whole sRGB8 frame: every member's band into one width x height x 4 buffer */
+TR_API int32_t tr_group_read_srgb8(tr_group* g, uint8_t* rgba8);
+
+/* ------------------------------------------------------------------ */
 /* Diagnostics (benchmark support; not part of the reference surface)  */
 /* ------------------------------------------------------------------ */
 /* kernels launched by this library in this process so far */

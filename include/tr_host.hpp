@@ -17,6 +17,7 @@
 //   * Renderer: an owning handle of a tr_ctx whose methods return through exceptions, the way every fallible function
 //     of the reference returns anyhow::Result and is propagated with `?` (src/main.rs:93); record() (src/main.rs:1551) is
 //     Renderer::frame.
+//   * RendererGroup: several Renderers of one thread rendering the bands of one frame (tr_group_*), on one or more GPUs.
 //
 // tests/test_host_mirror.py compiles tests/host_mirror_dump.cpp against this header and compares every struct it builds
 // with the Python restatement (transmission_renderer_b200/host.py) the parity tests use: identical bytes wherever no
@@ -408,7 +409,61 @@ public:
     void comm_init(const uint8_t id[TR_NCCL_UNIQUE_ID_BYTES], int32_t rank, int32_t n_ranks) { TR_HOST_CHECK(tr_comm_init(ctx_, id, rank, n_ranks)); }
 
 private:
+    friend class RendererGroup;   // tr_group_resize resizes the members
     tr_ctx* ctx_ = nullptr;
+    uint32_t width_, height_;
+};
+
+// ---- RendererGroup: one Renderer per entry of `devices` (repeats allowed), joined into the bands of one frame
+// (tr_group_*).  The reference's host is one thread with one queue (src/main.rs:243); this is how that thread drives up to 8
+// GPUs.  Uploads and reads go to member(k) as to any Renderer; the frame goes through the group.
+class RendererGroup {
+public:
+    RendererGroup(const std::vector<int32_t>& devices, uint32_t width, uint32_t height, uint32_t flags = 0) : width_(width), height_(height) {
+        if (devices.empty() || devices.size() > 8) throw Error(TR_ERR_INVALID_ARG, "RendererGroup: 1 to 8 devices");
+        members_.reserve(devices.size());
+        for (int32_t d : devices) members_.emplace_back(width, height, d, flags);
+        std::vector<tr_ctx*> ctxs;
+        for (const Renderer& r : members_) ctxs.push_back(r.ctx());
+        TR_HOST_CHECK(tr_group_create(ctxs.data(), (uint32_t)ctxs.size(), &group_));
+    }
+    ~RendererGroup() {   // the group first: a member is not destroyed while it belongs to one
+        if (group_) tr_group_destroy(group_);
+    }
+    RendererGroup(const RendererGroup&) = delete;
+    RendererGroup& operator=(const RendererGroup&) = delete;
+
+    size_t size() const { return members_.size(); }
+    Renderer& member(size_t k) { return members_.at(k); }
+    tr_group* group() const { return group_; }
+
+    void set_bands(const std::vector<uint32_t>& bounds) { TR_HOST_CHECK(tr_group_set_bands(group_, bounds.data(), (uint32_t)bounds.size())); }
+    void resize(uint32_t width, uint32_t height) {   // src/main.rs:996-1166 on every member; equal-row bands again
+        TR_HOST_CHECK(tr_group_resize(group_, width, height));
+        width_ = width;
+        height_ = height;
+        for (Renderer& r : members_) {
+            r.width_ = width;
+            r.height_ = height;
+        }
+    }
+    // record(), src/main.rs:1551-2263, across the members: one camera for all, or one tr_frame_params per member (each with
+    // its own acceleration_structure_address when ray queries are on)
+    void frame(const tr_frame_params& f) { frame(std::vector<tr_frame_params>(members_.size(), f)); }
+    void frame(const std::vector<tr_frame_params>& per_member) {
+        if (per_member.size() != members_.size()) throw Error(TR_ERR_INVALID_ARG, "RendererGroup::frame: one tr_frame_params per member");
+        TR_HOST_CHECK(tr_group_frame(group_, per_member.data()));
+    }
+    void sync() { TR_HOST_CHECK(tr_group_sync(group_)); }
+    std::vector<uint8_t> read_srgb8() {   // the whole frame, every member's band
+        std::vector<uint8_t> out((size_t)width_ * height_ * 4);
+        TR_HOST_CHECK(tr_group_read_srgb8(group_, out.data()));
+        return out;
+    }
+
+private:
+    std::vector<Renderer> members_;
+    tr_group* group_ = nullptr;
     uint32_t width_, height_;
 };
 

@@ -34,6 +34,8 @@ REFERENCE_TYPES = {
     "tr_light_cluster_coefficients": "shared_structs::LightClusterCoefficients", "tr_textures": "shared_structs::Textures",
     "tr_packed_similarity": "shared_structs::PackedSimilarity",
 }
+# opaque handles: only ever behind a pointer
+OPAQUE = {"tr_ctx": "one per GPU / host thread", "tr_group": "contexts of one host thread rendering the bands of one frame"}
 # ABI-own structs: generated as #[repr(C)] below
 OWN_STRUCTS = ["tr_material_params", "tr_basic_brdf_params", "tr_brdf_result", "tr_transmission_btdf_params",
                "tr_ibl_volume_refraction_params", "tr_point_light_params", "tr_point_light_result", "tr_config", "tr_gbuffer_planes",
@@ -68,7 +70,7 @@ def rust_type(ctype):
         return SCALARS[t]
     if t in REFERENCE_TYPES:
         return REFERENCE_TYPES[t]
-    if t == "tr_ctx" or t in OWN_STRUCTS:
+    if t in OPAQUE or t in OWN_STRUCTS:
         return camel(t)
     raise ValueError(f"unmapped C type {ctype!r}")
 
@@ -122,7 +124,8 @@ def generate():
            "// are pinned to the same bytes — so values are passed by pointer without conversion.  INTEGRATION.md maps every call onto the",
            "// place in src/main.rs it replaces.",
            "#![allow(non_camel_case_types, dead_code)]", ""]
-    out.append("#[repr(C)] pub struct TrCtx { _private: [u8; 0] }   // opaque: one per GPU / host thread")
+    for name, what in OPAQUE.items():
+        out.append(f"#[repr(C)] pub struct {camel(name)} {{ _private: [u8; 0] }}   // opaque: {what}")
     out.append("")
     for name in OWN_STRUCTS:
         fields = structs[name]

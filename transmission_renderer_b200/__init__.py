@@ -30,6 +30,8 @@ EXPORTS = [
     "tr_begin_frame", "tr_read_frame_times", "tr_read_pass_totals", "tr_eval_basic_brdf", "tr_eval_transmission_btdf", "tr_eval_point_light", "tr_eval_ibl_volume_refraction",
     "tr_set_bands", "tr_comm_unique_id", "tr_comm_init", "tr_comm_destroy", "tr_peer_export", "tr_peer_attach", "tr_device_buffer",
     "tr_launch_count", "tr_raster_stats", "tr_measure_fp32_peak", "tr_measure_hbm_copy",
+    "tr_group_create", "tr_group_destroy", "tr_group_set_bands", "tr_group_resize", "tr_group_frame", "tr_group_sync",
+    "tr_group_read_srgb8",
 ]
 
 
@@ -61,4 +63,4 @@ def _check(status):
         raise TrError(status, lib().tr_last_error().decode())
 
 
-from .renderer import Renderer  # noqa: E402,F401
+from .renderer import Renderer, RendererGroup  # noqa: E402,F401

@@ -158,13 +158,13 @@ static trd::LutDesc lut_desc(const tr_ctx* c) {
 }
 
 static int slot_of(const tr_ctx* c) { return (int)(c->timing_frame % kTimingRing); }
-static void pass_begin(tr_ctx* c, int pass) {
+void pass_begin(tr_ctx* c, int pass) {
     if (!c->timing) return;
     const int slot = (int)(c->timing_frame % kTimingRing);
     cudaEventRecord(c->ev_begin[slot][pass], c->stream);
     c->ev_used[slot][pass] = true;
 }
-static void pass_end(tr_ctx* c, int pass) {
+void pass_end(tr_ctx* c, int pass) {
     if (!c->timing) return;
     cudaEventRecord(c->ev_end[slot_of(c)][pass], c->stream);
 }
@@ -193,7 +193,7 @@ static int32_t sum_frame_times(tr_ctx* c, int slot, tr_frame_times* out) {
     return first >= 0 ? 1 : 0;
 }
 
-static int32_t check_pc(const tr_ctx* c, const tr_push_constants* pc, const char* who) {
+int32_t check_pc(const tr_ctx* c, const tr_push_constants* pc, const char* who) {
     if (!pc) return fail(TR_ERR_INVALID_ARG, "%s: null push constants", who);
     if (pc->acceleration_structure_address != 0) {  // the `--ray-tracing` variant of the fragment shaders, lib.rs:100-102
         if (!c->accel_blas_valid || pc->acceleration_structure_address != (uint64_t)(uintptr_t)c->accel_tlas.p)
@@ -370,6 +370,91 @@ int32_t check_device_status(tr_ctx* c, const char* who) {
                               "the G-buffer of that frame is incomplete", who, bits);
 }
 
+int32_t resize_frame(tr_ctx* c, uint32_t width, uint32_t height) {
+    c->width = width;
+    c->height = height;
+    c->band_y0 = 0;
+    c->band_y1 = height;
+    c->band_bounds.clear();
+    if (c->n_ranks > 1) {  // a rank of a band-sharded frame keeps its (equal-rows) share of the new frame
+        c->band_y0 = (uint32_t)(((uint64_t)c->rank * height) / c->n_ranks);
+        c->band_y1 = (uint32_t)(((uint64_t)(c->rank + 1) * height) / c->n_ranks);
+    }
+    c->clusters_valid = false;  // main.rs:1113-1121 reruns write_cluster_data on resize
+    return alloc_frame(c);
+}
+
+// ------------------------------------------------------------------ tr_frame in pieces (tr_internal.h)
+int32_t frame_front(tr_ctx* c, const tr_frame_params* f) {
+    timing_next_frame(c);
+    // everything the previous frame read is free from here on: the mark the next frame's uploads wait for (upload_ahead)
+    if (!c->ev_frame_begin) TR_CUDA(cudaEventCreateWithFlags(&c->ev_frame_begin, cudaEventDisableTiming));
+    TR_CUDA(cudaEventRecord(c->ev_frame_begin, c->stream));
+    c->frame_begin_valid = true;
+    c->inst_uploaded = c->lights_uploaded = false;
+    const bool side = c->n_lights && !(f->flags & TR_FRAME_SKIP_VISIBILITY);
+    if (side) {   // K2 beside K1 + K3: fork here, join before the opaque pass reads the light lists
+        if (!c->side_stream) {
+            TR_CUDA(cudaStreamCreateWithFlags(&c->side_stream, cudaStreamNonBlocking));
+            TR_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
+            TR_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
+        }
+        TR_CUDA(cudaEventRecord(c->ev_fork, c->stream));
+        TR_CUDA(cudaStreamWaitEvent(c->side_stream, c->ev_fork, 0));
+        cudaStream_t main_stream = c->stream;
+        c->stream = c->side_stream;            // the pass and its timer events go to the side stream
+        const int32_t st = tr_assign_lights(c, &f->assign_lights);
+        c->stream = main_stream;
+        if (st != TR_OK) return st;
+        TR_CUDA(cudaEventRecord(c->ev_join, c->side_stream));
+    } else if (c->n_lights) {
+        TR_TRY(tr_assign_lights(c, &f->assign_lights));
+    }
+    if (!(f->flags & TR_FRAME_SKIP_VISIBILITY)) {
+        TR_TRY(tr_cull(c, &f->culling));
+        TR_TRY(tr_visibility(c, &f->push_constants));
+    }
+    if (side) TR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_join, 0));
+    return TR_OK;
+}
+
+int32_t shade_opaque(tr_ctx* c, const tr_push_constants* pc) {
+    ShadeLaunch s;
+    TR_TRY(fill_shade(c, pc, TR_LAYER_OPAQUE, &s, "tr_shade_opaque"));
+    uint2* mip0 = c->pyramid.as<uint2>() + c->level_off[0];
+    s.n_opaque = 0;
+    if (c->group) {   // every member's mip 0, this one's included: plain device pointers (same device or peer access)
+        for (int r = 0; r < c->group->n; r++) {
+            const tr_ctx* m = c->group->members[r];
+            s.opaque[s.n_opaque++] = m->pyramid.as<uint2>() + m->level_off[0];
+        }
+    } else if (c->peers_attached) {
+        for (int r = 0; r < c->n_ranks; r++) s.opaque[s.n_opaque++] = reinterpret_cast<uint2*>(c->peer_mip0[r]);
+    } else {
+        s.opaque[s.n_opaque++] = mip0;
+    }
+    pass_begin(c, P_OPAQUE);
+    if (s.shadow_mask) {
+        TR_TRY(launch_shadow_mask(s, c->sm_count, c->stream));
+        TR_TRY(launch_shade_opaque_shadowed(s, c->sm_count, c->stream));
+    } else {
+        TR_TRY(launch_shade_opaque(s, c->sm_count, c->stream));
+    }
+    pass_end(c, P_OPAQUE);
+    c->opaque_valid = true;
+    c->hdr_valid = true;
+    c->mips_valid = false;
+    return TR_OK;
+}
+
+int32_t frame_back(tr_ctx* c, const tr_frame_params* f, cudaEvent_t after_transmission) {
+    TR_TRY(tr_generate_mips(c));
+    if (c->layer[TR_LAYER_TRANSMISSIVE].valid) TR_TRY(tr_shade_transmission(c, &f->push_constants));
+    if (after_transmission) TR_CUDA(cudaEventRecord(after_transmission, c->stream));
+    if (!(f->flags & TR_FRAME_SKIP_TONEMAP)) TR_TRY(tr_tonemap(c, &f->tonemap));
+    return TR_OK;
+}
+
 int32_t comm_allgather_opaque(tr_ctx* c);  // tr_comm.cu
 int32_t comm_barrier(tr_ctx* c);
 void comm_release(tr_ctx* c);
@@ -432,6 +517,7 @@ int32_t tr_create(const tr_config* config, tr_ctx** out_ctx) {
 
 int32_t tr_destroy(tr_ctx* c) {
     if (!c) return TR_OK;
+    TR_NOT_GROUPED(c, "tr_destroy", "tr_group_destroy first");
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     comm_release(c);
@@ -484,24 +570,16 @@ int32_t tr_destroy(tr_ctx* c) {
 
 int32_t tr_resize(tr_ctx* c, uint32_t width, uint32_t height) {
     TR_CHECK_CTX(c);
+    TR_NOT_GROUPED(c, "tr_resize", "tr_group_resize");
     if (width == 0 || height == 0) return fail(TR_ERR_INVALID_ARG, "tr_resize: empty framebuffer");
     TR_CUDA(cudaStreamSynchronize(c->stream));
     if (c->peers_attached) return fail(TR_ERR_STATE, "tr_resize: detach the peer mappings first (tr_comm_destroy); they name the old frame buffers");
-    c->width = width;
-    c->height = height;
-    c->band_y0 = 0;
-    c->band_y1 = height;
-    c->band_bounds.clear();
-    if (c->n_ranks > 1) {  // a rank of a band-sharded frame keeps its (equal-rows) share of the new frame
-        c->band_y0 = (uint32_t)(((uint64_t)c->rank * height) / c->n_ranks);
-        c->band_y1 = (uint32_t)(((uint64_t)(c->rank + 1) * height) / c->n_ranks);
-    }
-    c->clusters_valid = false;  // main.rs:1113-1121 reruns write_cluster_data on resize
-    return alloc_frame(c);
+    return resize_frame(c, width, height);
 }
 
 int32_t tr_set_band(tr_ctx* c, uint32_t y0, uint32_t y1) {
     TR_CHECK_CTX(c);
+    TR_NOT_GROUPED(c, "tr_set_band", "tr_group_set_bands");
     if (y0 >= y1 || y1 > c->height) return fail(TR_ERR_INVALID_ARG, "tr_set_band: [%u,%u) outside the frame", y0, y1);
     c->band_y0 = y0;
     c->band_y1 = y1;
@@ -817,31 +895,13 @@ int32_t tr_visibility(tr_ctx* c, const tr_push_constants* pc) {
 
 int32_t tr_shade_opaque(tr_ctx* c, const tr_push_constants* pc) {
     TR_CHECK_CTX(c);
-    ShadeLaunch s;
-    TR_TRY(fill_shade(c, pc, TR_LAYER_OPAQUE, &s, "tr_shade_opaque"));
-    uint2* mip0 = c->pyramid.as<uint2>() + c->level_off[0];
-    s.n_opaque = 0;
-    if (c->peers_attached) {
-        for (int r = 0; r < c->n_ranks; r++) s.opaque[s.n_opaque++] = reinterpret_cast<uint2*>(c->peer_mip0[r]);
-    } else {
-        s.opaque[s.n_opaque++] = mip0;
-    }
-    pass_begin(c, P_OPAQUE);
-    if (s.shadow_mask) {
-        TR_TRY(launch_shadow_mask(s, c->sm_count, c->stream));
-        TR_TRY(launch_shade_opaque_shadowed(s, c->sm_count, c->stream));
-    } else {
-        TR_TRY(launch_shade_opaque(s, c->sm_count, c->stream));
-    }
-    pass_end(c, P_OPAQUE);
-    c->opaque_valid = true;
-    c->hdr_valid = true;
-    c->mips_valid = false;
-    return TR_OK;
+    TR_NOT_GROUPED(c, "tr_shade_opaque", "tr_group_frame");
+    return shade_opaque(c, pc);
 }
 
 int32_t tr_allgather_opaque(tr_ctx* c) {
     TR_CHECK_CTX(c);
+    TR_NOT_GROUPED(c, "tr_allgather_opaque", "tr_group_frame");
     if (c->n_ranks <= 1) return TR_OK;
     if (!c->opaque_valid) return fail(TR_ERR_STATE, "tr_allgather_opaque: no opaque frame");
     pass_begin(c, P_GATHER);
@@ -904,45 +964,15 @@ int32_t tr_begin_frame(tr_ctx* c) {
 
 int32_t tr_frame(tr_ctx* c, const tr_frame_params* f) {
     TR_CHECK_CTX(c);
+    TR_NOT_GROUPED(c, "tr_frame", "tr_group_frame");
     if (!f) return fail(TR_ERR_INVALID_ARG, "tr_frame: null");
-    timing_next_frame(c);
-    // everything the previous frame read is free from here on: the mark the next frame's uploads wait for (upload_ahead)
-    if (!c->ev_frame_begin) TR_CUDA(cudaEventCreateWithFlags(&c->ev_frame_begin, cudaEventDisableTiming));
-    TR_CUDA(cudaEventRecord(c->ev_frame_begin, c->stream));
-    c->frame_begin_valid = true;
-    c->inst_uploaded = c->lights_uploaded = false;
-    const bool side = c->n_lights && !(f->flags & TR_FRAME_SKIP_VISIBILITY);
-    if (side) {   // K2 beside K1 + K3: fork here, join before the opaque pass reads the light lists
-        if (!c->side_stream) {
-            TR_CUDA(cudaStreamCreateWithFlags(&c->side_stream, cudaStreamNonBlocking));
-            TR_CUDA(cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
-            TR_CUDA(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
-        }
-        TR_CUDA(cudaEventRecord(c->ev_fork, c->stream));
-        TR_CUDA(cudaStreamWaitEvent(c->side_stream, c->ev_fork, 0));
-        cudaStream_t main_stream = c->stream;
-        c->stream = c->side_stream;            // the pass and its timer events go to the side stream
-        const int32_t st = tr_assign_lights(c, &f->assign_lights);
-        c->stream = main_stream;
-        if (st != TR_OK) return st;
-        TR_CUDA(cudaEventRecord(c->ev_join, c->side_stream));
-    } else if (c->n_lights) {
-        TR_TRY(tr_assign_lights(c, &f->assign_lights));
-    }
-    if (!(f->flags & TR_FRAME_SKIP_VISIBILITY)) {
-        TR_TRY(tr_cull(c, &f->culling));
-        TR_TRY(tr_visibility(c, &f->push_constants));
-    }
-    if (side) TR_CUDA(cudaStreamWaitEvent(c->stream, c->ev_join, 0));
+    TR_TRY(frame_front(c, f));
     // peer-store path: a peer's opaque pass writes into THIS rank's mip 0, which the previous frame's transmissive
     // pass may still be sampling -> cross-GPU barrier before anybody starts shading
     if (c->n_ranks > 1 && c->peers_attached) TR_TRY(comm_barrier(c));
-    TR_TRY(tr_shade_opaque(c, &f->push_constants));
+    TR_TRY(shade_opaque(c, &f->push_constants));
     if (c->n_ranks > 1) TR_TRY(tr_allgather_opaque(c));  // NCCL all-gather, or (peer path) the barrier that ends the exchange
-    TR_TRY(tr_generate_mips(c));
-    if (c->layer[TR_LAYER_TRANSMISSIVE].valid) TR_TRY(tr_shade_transmission(c, &f->push_constants));
-    if (!(f->flags & TR_FRAME_SKIP_TONEMAP)) TR_TRY(tr_tonemap(c, &f->tonemap));
-    return TR_OK;
+    return frame_back(c, f, nullptr);
 }
 
 int32_t tr_enable_timing(tr_ctx* c, int32_t enable) {

@@ -70,7 +70,7 @@ int32_t nccl_fail(const char* what, int rc) {
 }
 }  // namespace
 
-static void band_of(const tr_ctx* c, int r, uint32_t* y0, uint32_t* y1) {
+void band_of(const tr_ctx* c, int r, uint32_t* y0, uint32_t* y1) {
     if (c->band_bounds.size() == (size_t)c->n_ranks + 1) {  // caller-balanced bands (tr_set_bands)
         *y0 = c->band_bounds[r];
         *y1 = c->band_bounds[r + 1];
@@ -175,6 +175,7 @@ int32_t tr_comm_init(tr_ctx* c, const uint8_t id[TR_NCCL_UNIQUE_ID_BYTES], int32
     if (!c || !id) return fail(TR_ERR_INVALID_ARG, "tr_comm_init: null");
     if (n_ranks < 1 || n_ranks > kMaxPeers || rank < 0 || rank >= n_ranks)
         return fail(TR_ERR_INVALID_ARG, "tr_comm_init: rank %d of %d (at most %d ranks)", rank, n_ranks, kMaxPeers);
+    TR_NOT_GROUPED(c, "tr_comm_init", "the group's bands (tr_group_set_bands); a group needs no communicator");
     TR_CUDA(cudaSetDevice(c->device));
     c->rank = rank;
     c->n_ranks = n_ranks;
@@ -207,6 +208,7 @@ int32_t tr_comm_destroy(tr_ctx* c) {
 
 int32_t tr_set_bands(tr_ctx* c, const uint32_t* bounds, uint32_t n_bounds) {
     if (!c || !bounds) return fail(TR_ERR_INVALID_ARG, "tr_set_bands: null");
+    TR_NOT_GROUPED(c, "tr_set_bands", "tr_group_set_bands");
     if (n_bounds != (uint32_t)c->n_ranks + 1) return fail(TR_ERR_INVALID_ARG, "tr_set_bands: %u boundaries for %d ranks", n_bounds, c->n_ranks);
     if (bounds[0] != 0 || bounds[c->n_ranks] != c->height) return fail(TR_ERR_INVALID_ARG, "tr_set_bands: the bands must cover rows [0, %u)", c->height);
     for (int r = 0; r < c->n_ranks; r++)
@@ -233,6 +235,7 @@ int32_t tr_peer_export(tr_ctx* c, uint8_t handle[TR_IPC_HANDLE_BYTES]) {
 
 int32_t tr_peer_attach(tr_ctx* c, int32_t rank, int32_t n_ranks, const uint8_t* handles) {
     if (!c || !handles) return fail(TR_ERR_INVALID_ARG, "tr_peer_attach: null");
+    TR_NOT_GROUPED(c, "tr_peer_attach", "tr_group_frame, whose members store into each other's frames directly");
     if (rank != c->rank || n_ranks != c->n_ranks) return fail(TR_ERR_STATE, "tr_peer_attach: call tr_comm_init first with the same rank/size");
     TR_CUDA(cudaSetDevice(c->device));
     for (int r = 0; r < n_ranks; r++) {

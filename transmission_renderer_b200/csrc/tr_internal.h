@@ -34,6 +34,11 @@ void count_launches(int n);  // process-wide count of kernels this library launc
         int32_t _s = (expr);          \
         if (_s != TR_OK) return _s;   \
     } while (0)
+// the frame-wide calls of a group member go through its group (tr_group.cu)
+#define TR_NOT_GROUPED(c, who, instead)                                                                              \
+    do {                                                                                                             \
+        if ((c)->group) return tr::fail(TR_ERR_STATE, "%s: the context is a member of a group; use %s", who, instead); \
+    } while (0)
 
 struct DevBuf {
     void* p = nullptr;
@@ -148,6 +153,16 @@ struct tr_ctx {
     size_t barrier_flags_offset = 0;      // byte offset of the barrier words inside the pyramid allocation
     uint32_t barrier_epoch = 0;
     bool peers_attached = false;
+    tr_group* group = nullptr;            // single-process group this context is rank `rank` of (tr_group.cu)
+};
+
+// tr_group_create: contexts of one host thread joined into the bands of one frame.  Member k is rank k; its opaque pass
+// stores into every member's mip 0 through plain device pointers, and CUDA events order the members (tr_group.cu).
+struct tr_group {
+    int n = 0;
+    tr_ctx* members[tr::kMaxPeers] = {};
+    cudaEvent_t ev_front[tr::kMaxPeers] = {};  // recorded after member k's opaque pass (its band is in every mip 0)
+    cudaEvent_t ev_back[tr::kMaxPeers] = {};   // recorded after member k's transmissive pass (done reading its mip 0)
 };
 
 namespace tr {
@@ -221,5 +236,18 @@ int32_t validate_scene(tr_ctx* c, const char* who);  // instance -> primitive / 
 void mat4_inverse_f64(const tr_mat4& m, tr_mat4* out);
 int32_t ensure_layer(tr_ctx* c, int layer, bool with_position);
 int32_t upload_texture_table(tr_ctx* c);  // descriptor table of the bound images -> device (if it changed)
+void band_of(const tr_ctx* c, int r, uint32_t* y0, uint32_t* y1);   // rows of rank r (tr_comm.cu)
+
+// tr_frame in pieces (tr_api.cu), shared with tr_group_frame (tr_group.cu):
+//   frame_front   per-pass timer mark, ev_frame_begin, K2 on the side stream beside K1 + K3, join
+//   shade_opaque  K4 (tr_shade_opaque without the group check); a group member stores its band into every member's mip 0
+//   frame_back    K5, K6, then records `after_transmission` (if not null) on the context stream, then K7
+int32_t frame_front(tr_ctx* c, const tr_frame_params* f);
+int32_t shade_opaque(tr_ctx* c, const tr_push_constants* pc);
+int32_t frame_back(tr_ctx* c, const tr_frame_params* f, cudaEvent_t after_transmission);
+int32_t check_pc(const tr_ctx* c, const tr_push_constants* pc, const char* who);
+int32_t resize_frame(tr_ctx* c, uint32_t width, uint32_t height);   // tr_resize after its checks
+void pass_begin(tr_ctx* c, int pass);
+void pass_end(tr_ctx* c, int pass);
 
 }  // namespace tr

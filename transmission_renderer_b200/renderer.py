@@ -9,7 +9,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import abi
+from . import abi, host
 
 
 def _lib():
@@ -51,12 +51,13 @@ class Renderer:
         cfg = _Config(self.width, self.height, device, y0, y1, abi.TR_FLAG_HDR_F32_DEBUG if f32_debug else 0)
         _check(_lib().tr_create(C.byref(cfg), C.byref(self._ctx)))
         self.f32_debug = f32_debug
+        self.acceleration_structure_address = 0   # the handle of the last build_acceleration_structures (RendererGroup.frame)
         self._keep = []
 
     # -- lifecycle -------------------------------------------------------------------
     def close(self):
         if self._ctx:
-            _lib().tr_destroy(self._ctx)
+            _check(_lib().tr_destroy(self._ctx))   # refused while the context is a member of a RendererGroup
             self._ctx = C.c_void_p()
 
     def __del__(self):
@@ -130,11 +131,13 @@ class Renderer:
         Returns the handle to put into PushConstants.acceleration_structure_address (src/main.rs:856-859)."""
         a = C.c_uint64(0)
         _check(_lib().tr_build_acceleration_structures(self._ctx, C.byref(a)))
+        self.acceleration_structure_address = a.value
         return a.value
 
     def update_top_level_acceleration_structure(self):
         a = C.c_uint64(0)
         _check(_lib().tr_update_top_level_acceleration_structure(self._ctx, C.byref(a)))
+        self.acceleration_structure_address = a.value
         return a.value
 
     def trace_shadow_rays(self, origins, directions, t_max):
@@ -391,3 +394,134 @@ class Renderer:
         v = C.c_float(0)
         _check(_lib().tr_measure_hbm_copy(self._ctx, C.byref(v)))
         return v.value
+
+
+_BAND_PASSES = ("visibility_ms", "shade_opaque_ms", "shade_transmission_ms", "tonemap_ms")   # a band's own cost (parallel.py)
+
+
+class RendererGroup:
+    """Several `Renderer`s of this thread rendering the bands of ONE frame (tr_group_*): member k renders band k, and its
+    opaque pass stores the band into every member's opaque frame directly.  The members may sit on different devices or on
+    the same one.  The reference's host is one thread with one queue (src/main.rs:243); this is how such a host drives
+    several GPUs.
+
+        with Renderer(w, h, device=0) as a, Renderer(w, h, device=1) as b, RendererGroup([a, b]) as g:
+            g.frame(camera.frame_params())
+            image = g.read_srgb8()
+
+    While the group lives, the members' frame-wide calls (frame, shade_opaque, resize, set_band(s), close ...) raise;
+    uploads, build_acceleration_structures, timers and reads stay per member."""
+
+    def __init__(self, renderers):
+        self.renderers = list(renderers)
+        n = len(self.renderers)
+        ctxs = (C.c_void_p * max(n, 1))(*[r._ctx.value for r in self.renderers])
+        self._g = C.c_void_p()
+        _check(_lib().tr_group_create(ctxs, C.c_uint32(n), C.byref(self._g)))
+        self.width, self.height = self.renderers[0].width, self.renderers[0].height
+        self.bounds = self._equal_bounds()
+
+    def _equal_bounds(self):
+        n = len(self.renderers)
+        return [host.band_rows(self.height, k, n)[0] for k in range(n)] + [self.height]
+
+    # -- lifecycle ---------------------------------------------------------------------------------
+    def close(self):
+        """tr_group_destroy: waits for every member, which renders the whole frame again."""
+        if self._g:
+            st = _lib().tr_group_destroy(self._g)
+            self._g = C.c_void_p()
+            _check(st)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    # -- frame -----------------------------------------------------------------------------------------
+    def set_bands(self, bounds):
+        """n + 1 ascending row boundaries, 0 ... height; member k renders rows [bounds[k], bounds[k+1])."""
+        a = _c(bounds, np.uint32)
+        _check(_lib().tr_group_set_bands(self._g, _p(a), C.c_uint32(len(a))))
+        self.bounds = [int(v) for v in a]
+
+    def resize(self, width, height):
+        """Every member at the new size; the bands return to equal rows."""
+        _check(_lib().tr_group_resize(self._g, C.c_uint32(width), C.c_uint32(height)))
+        for r in self.renderers:
+            r.width, r.height = int(width), int(height)
+        self.width, self.height = int(width), int(height)
+        self.bounds = self._equal_bounds()
+
+    def frame(self, params):
+        """One frame across the members.  `params`: one frame-params struct for all of them, or a list of one per member.
+        A single struct with ray queries on (acceleration_structure_address != 0) gets each member's own handle."""
+        n = len(self.renderers)
+        if isinstance(params, (list, tuple)):
+            if len(params) != n:
+                raise ValueError(f"{len(params)} frame params for {n} members")
+            p = np.zeros(n, dtype=abi.frame_params)   # not np.concatenate: it packs the struct, dropping the ABI's padding
+            for k, q in enumerate(params):
+                p[k] = _c(q, abi.frame_params).reshape(-1)[0]
+        else:
+            one = _c(params, abi.frame_params).reshape(-1)
+            if len(one) != 1:
+                raise ValueError("frame(params): one struct, or a list of one per member")
+            p = np.repeat(one, n)
+            if one["push_constants"]["acceleration_structure_address"][0] != 0:
+                for k, r in enumerate(self.renderers):
+                    p[k]["push_constants"]["acceleration_structure_address"] = r.acceleration_structure_address
+        _check(_lib().tr_group_frame(self._g, _p(p)))
+
+    def sync(self):
+        _check(_lib().tr_group_sync(self._g))
+
+    # -- whole-frame reads ---------------------------------------------------------------------------
+    def read_srgb8(self, out=None):
+        a = np.zeros((self.height, self.width, 4), dtype=np.uint8) if out is None else out
+        assert a.dtype == np.uint8 and a.size == self.width * self.height * 4 and a.flags.c_contiguous
+        _check(_lib().tr_group_read_srgb8(self._g, _p(a)))
+        return a
+
+    def read_hdr(self):
+        """The RGBA16F frame stitched from every member's band."""
+        out = np.zeros((self.height, self.width, 4), dtype=np.uint16)
+        for k, r in enumerate(self.renderers):
+            y0, y1 = self.bounds[k], self.bounds[k + 1]
+            out[y0:y1] = r.read_hdr()[y0:y1]
+        return out
+
+    def pass_totals(self):
+        """Every member's (per-pass ms summed over the frames since its timers were switched on, number of frames)."""
+        return [r.pass_totals() for r in self.renderers]
+
+    def balance_bands(self, run_frames, iterations=4):
+        """Move the band boundaries until every member's band costs about the same: the in-process form of
+        parallel.balance_bands, with the same cost model (parallel.balanced_bounds).  `run_frames()` renders a few group
+        frames.  Returns the final boundaries."""
+        from . import parallel
+        bounds = list(self.bounds)
+        if len(self.renderers) == 1:
+            return bounds
+        for _ in range(iterations):
+            run_frames()             # untimed: the first frames after new boundaries grow buffers
+            self.sync()
+            for r in self.renderers:
+                r.enable_timing(True)
+            run_frames()
+            self.sync()
+            cost = []
+            for r in self.renderers:
+                totals, n = r.pass_totals()
+                r.enable_timing(False)
+                cost.append(sum(totals[k] for k in _BAND_PASSES) / max(n, 1))
+            bounds = parallel.balanced_bounds(bounds, cost)
+            self.set_bands(bounds)
+        return bounds
