@@ -414,6 +414,14 @@ TR_API int32_t tr_build_acceleration_structures(tr_ctx* ctx, uint64_t* address);
 /* update_top_level_acceleration_structure_from_instances (src/acceleration_structures.rs:188-263, src/main.rs:1332-1345):
  * after tr_set_instances.  The handle may change; it is returned again. */
 TR_API int32_t tr_update_top_level_acceleration_structure(tr_ctx* ctx, uint64_t* address);
+/* update_top_level_acceleration_structure_from_instances (src/acceleration_structures.rs:188-263, src/main.rs:1332-1345),
+ * built on the device in stream order: it reads the instance buffer as the context's stream sees it (after any pending
+ * tr_set_instances upload) and returns without waiting for the GPU.  The frame enqueued next traces against it.  Same
+ * handle rules as tr_update_top_level_acceleration_structure; the handle changes only when the number of instances
+ * in the top level grows past what was allocated.  Requires tr_build_acceleration_structures since the last mesh /
+ * primitive upload.  The first call after that build uploads a per-primitive table; later calls do not wait for the
+ * device unless a buffer grows.  Each call launches 19 kernels (tr_launch_count). */
+TR_API int32_t tr_update_top_level_acceleration_structure_async(tr_ctx* ctx, uint64_t* address);
 /* trace_shadow_ray (lighting.rs:97-125) for a batch of rays given in host memory: origins/directions [n*3], t_max [n];
  * lit[i] = 1 when nothing is hit between t_min = 0.001 and t_max[i], else 0. */
 TR_API int32_t tr_trace_shadow_rays(tr_ctx* ctx, uint32_t n, const float* origins, const float* directions,
@@ -421,6 +429,11 @@ TR_API int32_t tr_trace_shadow_rays(tr_ctx* ctx, uint32_t n, const float* origin
 /* Parity hook: the occluded-ray bits the last shading pass of `layer` used, [5][h*w] words (band rows are written):
  * planes 0-3 bit i = the ray towards the i-th light of the pixel's cluster list, plane 4 bit 0 = the sun ray. */
 TR_API int32_t tr_read_shadow_mask(tr_ctx* ctx, int32_t layer, uint32_t* mask);
+/* Parity hook: the top level as built, by either update: node_capacity 64-byte nodes and instance_capacity 64-byte
+ * instance records in leaf order (layouts in csrc/tr_device_accel.cuh: AccelNode, AccelInstance); node 0 is the root.
+ * *n_nodes / *n_instances receive the counts (null arrays: counts only); blocking. */
+TR_API int32_t tr_read_top_level_acceleration_structure(tr_ctx* ctx, void* nodes, uint32_t node_capacity, uint32_t* n_nodes,
+                                                       void* instances, uint32_t instance_capacity, uint32_t* n_instances);
 
 /* ------------------------------------------------------------------ */
 /* Per-frame passes, in record() order (src/main.rs:1551-2263).        */

@@ -384,6 +384,18 @@ public:
         TR_HOST_CHECK(tr_build_acceleration_structures(ctx_, &address));
         return address;
     }
+    // update_top_level_acceleration_structure_from_instances, src/acceleration_structures.rs:188-263: after set_instances
+    uint64_t update_top_level_acceleration_structure() {
+        uint64_t address = 0;
+        TR_HOST_CHECK(tr_update_top_level_acceleration_structure(ctx_, &address));
+        return address;
+    }
+    // the same, built on the device in stream order without waiting for the GPU (the per-frame form, src/main.rs:1263-1345)
+    uint64_t update_top_level_acceleration_structure_async() {
+        uint64_t address = 0;
+        TR_HOST_CHECK(tr_update_top_level_acceleration_structure_async(ctx_, &address));
+        return address;
+    }
     // record(), src/main.rs:1551-2263
     void frame(const tr_frame_params& f) { TR_HOST_CHECK(tr_frame(ctx_, &f)); }
     void sync() { TR_HOST_CHECK(tr_sync(ctx_)); }

@@ -129,3 +129,10 @@ def default_material(n=1):
     m["specular_factor"] = 1.0
     m["specular_colour_factor"] = (1.0, 1.0, 1.0, 0.0)
     return m
+
+# the top level as tr_read_top_level_acceleration_structure returns it (csrc/tr_device_accel.cuh AccelNode, AccelInstance);
+# c0 / c1 >= 0: inner node, < 0: leaf ~(first | (count - 1) << 28)
+accel_node = _dt([("lo0", VEC3, 0), ("hi0", VEC3, 12), ("lo1", VEC3, 24), ("hi1", VEC3, 36), ("c0", "<i4", 48), ("c1", "<i4", 52),
+                  ("pad", ("<u4", (2,)), 56)], 64)
+accel_instance = _dt([("translation", VEC3, 0), ("inv_scale", "<f4", 12), ("conj_rotation", VEC4, 16), ("lo", VEC3, 32),
+                      ("hi", VEC3, 44), ("blas_root", "<u4", 56), ("tri_base", "<u4", 60)], 64)

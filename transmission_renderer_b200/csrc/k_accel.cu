@@ -5,10 +5,11 @@
 //   build_top_level_acceleration_structure_from_instances                      :106-186  (instances, PREFER_FAST_TRACE)
 //   update_top_level_acceleration_structure_from_instances                     :188-263  (after an instance moved)
 //   the instance filter `draw_buffer_index < 2`           src/main.rs:614-625
-// The reference hands both builds to the Vulkan driver; here they are binned-SAH builds on the host (a few hundred
-// thousand triangles and ten thousand instances take milliseconds, and they run at load time or when an instance
-// moves, not per frame).  What the trees must guarantee is in tr_device_accel.cuh: inner boxes are exact unions and the
-// depth of either level stays below kAccelStack.
+// The reference hands both builds to the Vulkan driver; here they are binned-SAH builds on the host, run at load time
+// and by tr_update_top_level_acceleration_structure, which reads the instances back and waits for the GPU.  When
+// instances move every frame (the reference's --rotate-model), tr_update_top_level_acceleration_structure_async rebuilds
+// the top level on the device in stream order instead (k_accel_device.cu).  What the trees must guarantee is in
+// tr_device_accel.cuh: inner boxes are exact unions and the depth of either level stays below kAccelStack.
 #include <algorithm>
 #include <cmath>
 #include <cstring>

@@ -526,7 +526,7 @@ int32_t tr_destroy(tr_ctx* c) {
                       &c->draws[2], &c->draws[3], &c->work_prefix, &c->slot_z, &c->slot_first, &c->block_entry, &c->chunk_spheres, &c->prim_chunk_base, &c->cluster_aabbs, &c->cluster_counts,
                       &c->cluster_indices, &c->vis[0], &c->vis[1], &c->bin_entries, &c->bin_state, &c->tri_records, &c->dev_status, &c->band_list, &c->hdr, &c->hdr_f32, &c->pyramid,
                       &c->srgb8, &c->mip_counter, &c->shade_counter, &c->accel_tlas, &c->accel_blas, &c->accel_inst, &c->accel_tris,
-                      &c->shadow_mask[0], &c->shadow_mask[1]};
+                      &c->accel_prim_table, &c->accel_scratch, &c->shadow_mask[0], &c->shadow_mask[1]};
     for (DevBuf* b : bufs) b->release();
     for (DevBuf& b : c->tex_data) b.release();
     c->tex_table.release();
@@ -806,6 +806,7 @@ int32_t tr_build_acceleration_structures(tr_ctx* c, uint64_t* address) {
     TR_CHECK_CTX(c);
     if (!address) return fail(TR_ERR_INVALID_ARG, "tr_build_acceleration_structures: null");
     *address = 0;
+    c->accel_prim_table_valid = false;   // the device builder's primitive table follows the new bottom level
     TR_TRY(accel_build(c));
     *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
     return TR_OK;
@@ -815,6 +816,31 @@ int32_t tr_update_top_level_acceleration_structure(tr_ctx* c, uint64_t* address)
     TR_CHECK_CTX(c);
     TR_TRY(accel_build_tlas(c));
     if (address) *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
+    return TR_OK;
+}
+
+int32_t tr_update_top_level_acceleration_structure_async(tr_ctx* c, uint64_t* address) {
+    TR_CHECK_CTX(c);
+    TR_TRY(accel_build_tlas_async(c));
+    if (address) *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
+    return TR_OK;
+}
+
+int32_t tr_read_top_level_acceleration_structure(tr_ctx* c, void* nodes, uint32_t node_capacity, uint32_t* n_nodes, void* instances,
+                                                 uint32_t instance_capacity, uint32_t* n_instances) {
+    TR_CHECK_CTX(c);
+    if (!c->accel_blas_valid || !c->accel_tlas_valid)
+        return fail(TR_ERR_STATE, "tr_read_top_level_acceleration_structure: acceleration structures not built");
+    const uint32_t m = c->accel_n_instances, nn = m >= 2 ? m - 1 : 1;   // a binary tree over m leaves, or the one root
+    if (n_nodes) *n_nodes = nn;
+    if (n_instances) *n_instances = m;
+    if ((nodes && node_capacity < nn) || (instances && instance_capacity < m))
+        return fail(TR_ERR_INVALID_ARG, "tr_read_top_level_acceleration_structure: capacity %u nodes / %u instances < %u / %u",
+                    node_capacity, instance_capacity, nn, m);
+    if (nodes) TR_CUDA(cudaMemcpyAsync(nodes, c->accel_tlas.p, (size_t)nn * sizeof(trd::AccelNode), cudaMemcpyDeviceToHost, c->stream));
+    if (instances && m)
+        TR_CUDA(cudaMemcpyAsync(instances, c->accel_inst.p, (size_t)m * sizeof(trd::AccelInstance), cudaMemcpyDeviceToHost, c->stream));
+    TR_CUDA(cudaStreamSynchronize(c->stream));
     return TR_OK;
 }
 

@@ -44,7 +44,15 @@ struct AccelDesc {
 
 constexpr float kShadowTMin = 0.001f;      // lighting.rs:109
 constexpr float kSunTMax = 10000.0f;       // lighting.rs:31, 163
-constexpr int kAccelStack = 64;            // the builder bounds the depth of either level (k_accel.cu)
+// Traversal stack.  A push onto a full stack is dropped (sp < kAccelStack), which would lose a subtree and give a wrong bit,
+// not an error, so every builder bounds the depth of its trees below it:
+//   k_accel.cu (host, both levels): median splits below depth 28, so depth <= 28 + log2(n) < 64.
+//   k_accel_device.cu (device, top level): a radix tree over keys (30-bit Morton code, position); positions break ties, so
+//   the keys are distinct 54-bit strings (tr_set_instances keeps n below 2^24).  Every inner node splits its range at the
+//   first bit where its keys differ, so a child's common prefix is strictly longer than its parent's; the prefixes run
+//   from 0 to 53 bits, so a root-to-leaf path has at most 54 inner nodes and the depth is <= 55 < 64
+//   (tests/test_gpu_accel_update.py checks it on equal codes, geometric chains and wide scale ranges).
+constexpr int kAccelStack = 64;
 
 struct AccelRay {
     float o[3], d[3], inv[3];

@@ -120,6 +120,11 @@ struct tr_ctx {
     bool accel_blas_valid = false, accel_tlas_valid = false;
     std::vector<float> h_prim_box;                                  // object-space box per primitive (lo, hi)
     std::vector<uint32_t> h_prim_root, h_prim_tri_base, h_prim_bucket;
+    // the device builder of the top level (k_accel_device.cu): per-primitive table, uploaded on the first update after
+    // tr_build_acceleration_structures, and the builder's scratch (grow-only)
+    tr::DevBuf accel_prim_table, accel_scratch;
+    std::vector<uint8_t> h_accel_prims;   // the table's host copy (the source of its upload)
+    bool accel_prim_table_valid = false;
 
     // timing (profiling.rs zone taxonomy)
     bool timing = false;
@@ -214,6 +219,9 @@ int32_t launch_shadow_mask(const ShadeLaunch& p, int sm_count, cudaStream_t s);
 trd::AccelDesc accel_desc(const tr_ctx* c);
 int32_t accel_build(tr_ctx* c);       // bottom-level structures of every primitive, then the top level
 int32_t accel_build_tlas(tr_ctx* c);  // top level only (instances moved)
+// the top level built on the device in stream order (k_accel_device.cu); launches kAsyncTlasLaunches kernels
+int32_t accel_build_tlas_async(tr_ctx* c);
+constexpr int kAsyncTlasLaunches = 19;
 int32_t launch_trace_rays(tr_ctx* c, uint32_t n, const float* d_origins, const float* d_directions, const float* d_t_max, uint8_t* d_lit);
 int32_t launch_generate_mips(uint2* pyramid, uint32_t levels, const uint32_t* w, const uint32_t* h, const uint32_t* off,
                              uint32_t* counter, int sm_count, cudaStream_t s);

@@ -140,6 +140,26 @@ class Renderer:
         self.acceleration_structure_address = a.value
         return a.value
 
+    def update_top_level_acceleration_structure_async(self):
+        """The same update built on the device in stream order: returns without waiting for the GPU; the next frame
+        traces against it."""
+        a = C.c_uint64(0)
+        _check(_lib().tr_update_top_level_acceleration_structure_async(self._ctx, C.byref(a)))
+        self.acceleration_structure_address = a.value
+        return a.value
+
+    def read_top_level_acceleration_structure(self):
+        """(nodes, instances): the top level as built, abi.accel_node (node 0 is the root) and abi.accel_instance in
+        leaf order."""
+        nn, ni = C.c_uint32(0), C.c_uint32(0)
+        _check(_lib().tr_read_top_level_acceleration_structure(self._ctx, None, C.c_uint32(0), C.byref(nn), None, C.c_uint32(0),
+                                                                C.byref(ni)))
+        nodes = np.zeros(nn.value, dtype=abi.accel_node)
+        inst = np.zeros(ni.value, dtype=abi.accel_instance)
+        _check(_lib().tr_read_top_level_acceleration_structure(self._ctx, _p(nodes), C.c_uint32(len(nodes)), C.byref(nn),
+                                                                _p(inst) if len(inst) else None, C.c_uint32(len(inst)), C.byref(ni)))
+        return nodes, inst
+
     def trace_shadow_rays(self, origins, directions, t_max):
         """(n,3), (n,3), (n,) -> (n,) uint8: 1 = lit, 0 = occluded (trace_shadow_ray, lighting.rs:97-125)."""
         o, d = _c(origins, np.float32).reshape(-1, 3), _c(directions, np.float32).reshape(-1, 3)
