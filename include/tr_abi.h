@@ -398,6 +398,24 @@ TR_API int32_t tr_set_texture(tr_ctx* ctx, uint32_t index, const uint8_t* const*
 /* vertex bindings 0..2 + index buffer (pipelines.rs:291-307, main.rs:2516-2557). */
 TR_API int32_t tr_set_mesh(tr_ctx* ctx, const float* positions, const float* normals, const float* uvs,
                            uint32_t n_vertices, const uint32_t* indices, uint32_t n_indices);
+/* Vertex animation (skinning, morph targets, cloth, procedural displacement computed on the host): replaces the positions and
+ * normals [n*3] of vertices [first_vertex, first_vertex + n) of the mesh of tr_set_mesh; indices, uvs and the vertex count
+ * stay.  Stream-ordered on the context stream: the frame enqueued before the call sees the old vertices, the next one the new.
+ * Sources follow the upload rule (pageable: copied during the call; page-locked: read in stream order).  On the device, in
+ * stream order, it recomputes the culling spheres of the binning pass and, once tr_build_acceleration_structures has run,
+ * refits the bottom-level structures (same topology, new boxes and triangles); the top level then needs an update
+ * (tr_update_top_level_acceleration_structure(_async)) before the next traced frame, which otherwise fails with
+ * TR_ERR_STATE, as after tr_set_instances.  The handle does not change.  No wait for the device.  No allocation either,
+ * except in the first call after tr_set_mesh / tr_set_primitives when no tr_cull has run since: that call sizes the
+ * culling-sphere buffers for the new chunk count (grow-only), as the next tr_cull would.
+ * PrimitiveInfo.packed_bounding_sphere stays the caller's: for a deforming mesh it must hold every pose.
+ * No mesh: TR_ERR_STATE; a range past the vertex count, or a null pointer with n > 0: TR_ERR_INVALID_ARG; n = 0: nothing.
+ * Each call launches 1 kernel, plus 2 with built acceleration structures (tr_launch_count). */
+TR_API int32_t tr_update_mesh_vertices(tr_ctx* ctx, uint32_t first_vertex, uint32_t n, const float* positions, const float* normals);
+/* Parity hook: the culling spheres of the binning pass, one float4 (object-space centre xyz, radius w) per 64 consecutive
+ * triangles of every primitive, primitive after primitive; computed first if no tr_cull has needed them yet.  *n_spheres
+ * receives the count (0 when a primitive leaves the index buffer: the test is off); null array: count only; blocking. */
+TR_API int32_t tr_read_chunk_spheres(tr_ctx* ctx, float* spheres, uint32_t capacity, uint32_t* n_spheres);
 
 /* ------------------------------------------------------------------ */
 /* Ray-queried shadows — the `--ray-tracing` option (src/main.rs:84,   */
@@ -419,8 +437,8 @@ TR_API int32_t tr_update_top_level_acceleration_structure(tr_ctx* ctx, uint64_t*
  * tr_set_instances upload) and returns without waiting for the GPU.  The frame enqueued next traces against it.  Same
  * handle rules as tr_update_top_level_acceleration_structure; the handle changes only when the number of instances
  * in the top level grows past what was allocated.  Requires tr_build_acceleration_structures since the last mesh /
- * primitive upload.  The first call after that build uploads a per-primitive table; later calls do not wait for the
- * device unless a buffer grows.  Each call launches 19 kernels (tr_launch_count). */
+ * primitive upload.  A call does not wait for the device unless a buffer grows.  Each call launches 19 kernels
+ * (tr_launch_count). */
 TR_API int32_t tr_update_top_level_acceleration_structure_async(tr_ctx* ctx, uint64_t* address);
 /* trace_shadow_ray (lighting.rs:97-125) for a batch of rays given in host memory: origins/directions [n*3], t_max [n];
  * lit[i] = 1 when nothing is hit between t_min = 0.001 and t_max[i], else 0. */
@@ -434,6 +452,13 @@ TR_API int32_t tr_read_shadow_mask(tr_ctx* ctx, int32_t layer, uint32_t* mask);
  * *n_nodes / *n_instances receive the counts (null arrays: counts only); blocking. */
 TR_API int32_t tr_read_top_level_acceleration_structure(tr_ctx* ctx, void* nodes, uint32_t node_capacity, uint32_t* n_nodes,
                                                        void* instances, uint32_t instance_capacity, uint32_t* n_instances);
+/* Parity hook: the bottom-level structures of every primitive, as built or as refitted by tr_update_mesh_vertices:
+ * node_capacity 64-byte nodes (AccelNode; the trees one after the other in primitive order, each root first) and
+ * tri_capacity triangles of three float4 (x, y, z, 0) each, in leaf order, primitive after primitive.  Leaf references
+ * count triangles from the first triangle of their primitive.  Counts into *n_nodes / *n_tris (null arrays: counts only);
+ * blocking. */
+TR_API int32_t tr_read_bottom_level_acceleration_structures(tr_ctx* ctx, void* nodes, uint32_t node_capacity, uint32_t* n_nodes,
+                                                           void* tris, uint32_t tri_capacity, uint32_t* n_tris);
 
 /* ------------------------------------------------------------------ */
 /* Per-frame passes, in record() order (src/main.rs:1551-2263).        */

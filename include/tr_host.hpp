@@ -360,6 +360,13 @@ public:
             throw Error(TR_ERR_INVALID_ARG, "Renderer::set_mesh: positions / normals / uvs disagree about the vertex count");
         TR_HOST_CHECK(tr_set_mesh(ctx_, positions.data(), normals.data(), uvs.data(), (uint32_t)(positions.size() / 3), indices.data(), (uint32_t)indices.size()));
     }
+    // vertex animation: positions and normals of vertices [first_vertex, first_vertex + n) in stream order; with ray queries,
+    // update the top level (update_top_level_acceleration_structure_async) before the next frame
+    void update_mesh_vertices(const std::vector<float>& positions, const std::vector<float>& normals, uint32_t first_vertex = 0) {
+        if (positions.size() % 3 || normals.size() != positions.size())
+            throw Error(TR_ERR_INVALID_ARG, "Renderer::update_mesh_vertices: positions / normals disagree about the vertex count");
+        TR_HOST_CHECK(tr_update_mesh_vertices(ctx_, first_vertex, (uint32_t)(positions.size() / 3), positions.data(), normals.data()));
+    }
     void set_instances(const std::vector<tr_instance>& v) { TR_HOST_CHECK(tr_set_instances(ctx_, v.data(), (uint32_t)v.size())); }
     void set_primitives(const std::vector<tr_primitive_info>& v) { TR_HOST_CHECK(tr_set_primitives(ctx_, v.data(), (uint32_t)v.size())); }
     void set_materials(const std::vector<tr_material_info>& v) { TR_HOST_CHECK(tr_set_materials(ctx_, v.data(), (uint32_t)v.size())); }

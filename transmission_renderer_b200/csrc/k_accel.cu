@@ -8,8 +8,9 @@
 // The reference hands both builds to the Vulkan driver; here they are binned-SAH builds on the host, run at load time
 // and by tr_update_top_level_acceleration_structure, which reads the instances back and waits for the GPU.  When
 // instances move every frame (the reference's --rotate-model), tr_update_top_level_acceleration_structure_async rebuilds
-// the top level on the device in stream order instead (k_accel_device.cu).  What the trees must guarantee is in
-// tr_device_accel.cuh: inner boxes are exact unions and the depth of either level stays below kAccelStack.
+// the top level on the device in stream order instead (k_accel_device.cu), and tr_update_mesh_vertices refits the bottom
+// level there from the parent links and triangle sources this build uploads (k_mesh_update.cu).  What the trees must
+// guarantee is in tr_device_accel.cuh: inner boxes are exact unions and the depth of either level stays below kAccelStack.
 #include <algorithm>
 #include <cmath>
 #include <cstring>
@@ -229,6 +230,10 @@ int32_t accel_build_tlas(tr_ctx* c) {
     std::vector<tr_instance> inst(c->n_instances);
     if (c->n_instances)
         TR_CUDA(cudaMemcpyAsync(inst.data(), c->instances.p, sizeof(tr_instance) * c->n_instances, cudaMemcpyDeviceToHost, c->stream));
+    // the primitive boxes: the device table is their source of truth (a bottom-level refit rewrites them in stream order)
+    std::vector<TlasPrim> prims(c->n_primitives);
+    if (c->n_primitives)
+        TR_CUDA(cudaMemcpyAsync(prims.data(), c->accel_prim_table.p, sizeof(TlasPrim) * c->n_primitives, cudaMemcpyDeviceToHost, c->stream));
     TR_CUDA(cudaStreamSynchronize(c->stream));
     std::vector<AccelInstance> records;
     std::vector<Item> items;
@@ -243,9 +248,10 @@ int32_t accel_build_tlas(tr_ctx* c) {
         r.inv_scale = 1.0f / scale;
         r.qx = -s.rotation.x; r.qy = -s.rotation.y; r.qz = -s.rotation.z; r.qw = s.rotation.w;
         Box w = box_empty();
-        const float* ob = &c->h_prim_box[(size_t)p * 6];
+        const float* lo = prims[p].lo;
+        const float* hi = prims[p].hi;
         for (int k = 0; k < 8; k++) {  // Similarity * Vec3 (shared-structs lib.rs:216-220) on the eight corners
-            const H3 corner = h3(k & 1 ? ob[3] : ob[0], k & 2 ? ob[4] : ob[1], k & 4 ? ob[5] : ob[2]);
+            const H3 corner = h3(k & 1 ? hi[0] : lo[0], k & 2 ? hi[1] : lo[1], k & 4 ? hi[2] : lo[2]);
             const H3 wp = hadd(h3(r.tx, r.ty, r.tz), hscale(hquat_mul(s.rotation.x, s.rotation.y, s.rotation.z, s.rotation.w, corner), scale));
             const float q[3] = {wp.x, wp.y, wp.z};
             box_grow(w, q);
@@ -282,7 +288,8 @@ int32_t accel_build(tr_ctx* c) {
 
     std::vector<AccelNode> nodes;
     std::vector<float4> tris;
-    c->h_prim_box.assign((size_t)c->n_primitives * 6, 0.0f);
+    std::vector<uint32_t> tri_src;                       // first index of every leaf-order triangle (the refit's gather)
+    std::vector<TlasPrim> table(c->n_primitives);
     c->h_prim_root.assign(c->n_primitives, 0u);
     c->h_prim_tri_base.assign(c->n_primitives, 0u);
     c->h_prim_bucket.assign(c->n_primitives, 0u);
@@ -308,22 +315,40 @@ int32_t accel_build(tr_ctx* c) {
             box_union(pb, b);
             items.push_back(Item{b, t});
         }
-        memcpy(&c->h_prim_box[(size_t)p * 6], pb.lo, 12);
-        memcpy(&c->h_prim_box[(size_t)p * 6 + 3], pb.hi, 12);
         c->h_prim_root[p] = build_tree(nodes, items, 4);
-        for (const Item& it : items)  // triangles in leaf order
+        for (const Item& it : items) {  // triangles in leaf order
+            tri_src.push_back(pr.first_index + it.id * 3);
             for (int k = 0; k < 3; k++) {
                 const float* v = &pos[(size_t)idx[pr.first_index + it.id * 3 + k] * 3];
                 tris.push_back(make_float4(v[0], v[1], v[2], 0.0f));
             }
+        }
+        memcpy(table[p].lo, pb.lo, 12);
+        memcpy(table[p].hi, pb.hi, 12);
+        table[p].blas_root = c->h_prim_root[p];
+        table[p].tri_base = c->h_prim_tri_base[p];
+        table[p].keep = pr.draw_buffer_index < 2u && nt != 0u;
     }
+    // the refit's parent links: -1 at a root (build_tree appends every tree in preorder, children after their parent)
+    std::vector<int32_t> parent(nodes.size(), -1);
+    for (size_t i = 0; i < nodes.size(); i++)
+        for (int32_t ch : {nodes[i].c0, nodes[i].c1})
+            if (ch >= 0) parent[ch] = (int32_t)i;
     if (c->h_prim_tris.size() != c->n_primitives) {
         c->h_prim_tris.resize(c->n_primitives);
         for (uint32_t p = 0; p < c->n_primitives; p++) c->h_prim_tris[p] = prims[p].index_count / 3;
     }
     TR_TRY(upload_vec(c, c->accel_blas, nodes.data(), nodes.size() * sizeof(AccelNode)));
     TR_TRY(upload_vec(c, c->accel_tris, tris.data(), tris.size() * sizeof(float4)));
+    TR_TRY(upload_vec(c, c->accel_prim_table, table.data(), table.size() * sizeof(TlasPrim)));
+    // refit tables (k_mesh_update.cu): parents [nodes], arrival counters [nodes], triangle sources [triangles]
+    const size_t nn = nodes.size(), nt = tri_src.size();
+    TR_TRY(c->accel_refit.ensure((nn * 2 + nt) * 4));
+    TR_CUDA(cudaMemcpyAsync(c->accel_refit.p, parent.data(), nn * 4, cudaMemcpyHostToDevice, c->stream));
+    if (nt) TR_CUDA(cudaMemcpyAsync(c->accel_refit.as<uint32_t>() + nn * 2, tri_src.data(), nt * 4, cudaMemcpyHostToDevice, c->stream));
     TR_CUDA(cudaStreamSynchronize(c->stream));
+    c->accel_blas_nodes = (uint32_t)nn;
+    c->accel_n_tris = (uint32_t)nt;
     c->accel_blas_valid = true;
     return accel_build_tlas(c);
 }

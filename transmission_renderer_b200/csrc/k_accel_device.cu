@@ -26,14 +26,6 @@ constexpr int kRadixPasses = 4;        // 30-bit codes in 8-bit digits
 constexpr int kScanThreads = 1024;
 static_assert(kTile == kRadix, "the histogram kernel keeps one digit per thread");
 
-struct TlasPrim {  // what the top level needs of a primitive (k_accel.cu keeps it on the host as h_prim_*)
-    float lo[3], hi[3];       // object-space box
-    uint32_t blas_root, tri_base;
-    uint32_t keep;            // draw_buffer_index < 2 and at least one triangle (src/main.rs:614-625)
-    uint32_t pad[3];
-};
-static_assert(sizeof(TlasPrim) == 48, "TlasPrim");
-
 __device__ __forceinline__ uint32_t keep_of(const tr_instance* inst, const TlasPrim* prims, uint32_t i) {
     return prims[inst[i].primitive_id].keep;
 }
@@ -323,8 +315,8 @@ __global__ void __launch_bounds__(kTile) tlas_boxes_kernel(const AccelInstance* 
 namespace tr {
 
 // Host side: the top-level count, the instance checks and the buffer sizes come from what the host holds; nothing
-// waits for the device unless a buffer grows (or on the first call after tr_build_acceleration_structures, which
-// uploads the primitive table).
+// waits for the device unless a buffer grows.  The primitive table is on the device since tr_build_acceleration_structures
+// (k_accel.cu accel_build), and a bottom-level refit keeps its boxes current (k_mesh_update.cu).
 int32_t accel_build_tlas_async(tr_ctx* c) {
     if (!c->accel_blas_valid)
         return fail(TR_ERR_STATE, "top-level build: bottom-level structures missing (tr_build_acceleration_structures)");
@@ -335,22 +327,6 @@ int32_t accel_build_tlas_async(tr_ctx* c) {
         if (p >= c->n_primitives) return fail(TR_ERR_INVALID_ARG, "top-level build: instance %u refers to primitive %u of %u", i, p, c->n_primitives);
         if (c->h_prim_bucket[p] >= 2u || c->h_prim_tris[p] == 0u) continue;
         m++;
-    }
-    if (!c->accel_prim_table_valid) {
-        c->h_accel_prims.assign((size_t)c->n_primitives * sizeof(TlasPrim), 0);
-        TlasPrim* t = reinterpret_cast<TlasPrim*>(c->h_accel_prims.data());
-        for (uint32_t p = 0; p < c->n_primitives; p++) {
-            for (int k = 0; k < 3; k++) {
-                t[p].lo[k] = c->h_prim_box[(size_t)p * 6 + k];
-                t[p].hi[k] = c->h_prim_box[(size_t)p * 6 + 3 + k];
-            }
-            t[p].blas_root = c->h_prim_root[p];
-            t[p].tri_base = c->h_prim_tri_base[p];
-            t[p].keep = c->h_prim_bucket[p] < 2u && c->h_prim_tris[p] != 0u;
-        }
-        TR_TRY(c->accel_prim_table.ensure(c->h_accel_prims.size()));
-        TR_CUDA(cudaMemcpyAsync(c->accel_prim_table.p, c->h_accel_prims.data(), c->h_accel_prims.size(), cudaMemcpyHostToDevice, c->stream));
-        c->accel_prim_table_valid = true;
     }
 
     // scratch: records [m], keys [2][m], values [2][m], parents [2m], arrivals [m], digit counts [kRadix][tiles of m],

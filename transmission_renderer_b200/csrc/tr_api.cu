@@ -200,7 +200,7 @@ int32_t check_pc(const tr_ctx* c, const tr_push_constants* pc, const char* who) 
             return fail(TR_ERR_INVALID_ARG, "%s: acceleration_structure_address is not the handle of tr_build_acceleration_structures "
                         "(or the mesh / primitives changed since)", who);
         if (!c->accel_tlas_valid)
-            return fail(TR_ERR_STATE, "%s: instances changed since the top-level structure was built "
+            return fail(TR_ERR_STATE, "%s: instances or mesh vertices changed since the top-level structure was built "
                         "(tr_update_top_level_acceleration_structure)", who);
     }
     if (pc->framebuffer_size.x != c->width || pc->framebuffer_size.y != c->height)
@@ -300,49 +300,28 @@ int32_t validate_scene(tr_ctx* c, const char* who) {
 
 // A bounding sphere (object space) per TR_CHUNK_TRIS consecutive triangles of every primitive: the binning pass tests it
 // against the frustum and the band before it touches the chunk's vertices.  Centre = centre of the chunk's box, radius = the
-// farthest vertex (double, rounded up).  Without a mesh, or with a primitive that leaves the index buffer, the test is off.
+// farthest vertex (double, rounded up); computed on the device in stream order (k_mesh_update.cu), so tr_update_mesh_vertices
+// can redo it every frame.  Without a mesh, or with a primitive that leaves the index buffer, the test is off.
 int32_t ensure_chunks(tr_ctx* c) {
     if (c->chunks_valid) return TR_OK;
-    std::vector<uint32_t> base((size_t)c->n_primitives + 1, 0u);
-    std::vector<float> spheres;
-    bool ok = c->n_indices != 0 && c->h_indices.size() == c->n_indices && c->h_positions.size() == (size_t)c->n_vertices * 3;
+    std::vector<uint32_t>& base = c->h_chunk_base;   // kept: the source of an upload that does not wait
+    base.assign((size_t)c->n_primitives + 1, 0u);
+    uint32_t n = 0;
+    bool ok = c->n_indices != 0;
     for (uint32_t p = 0; ok && p < c->n_primitives; p++) {
         const uint64_t first = c->h_prim_first[p], tris = c->h_prim_count[p] / 3;
         if (first + tris * 3 > c->n_indices) { ok = false; break; }   // validate_scene reports it
-        base[p] = (uint32_t)(spheres.size() / 4);
-        for (uint64_t t0 = 0; t0 < tris; t0 += TR_CHUNK_TRIS) {
-            const uint64_t t1 = std::min<uint64_t>(t0 + TR_CHUNK_TRIS, tris);
-            double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-            for (uint64_t i = first + t0 * 3; i < first + t1 * 3; i++)
-                for (int k = 0; k < 3; k++) {
-                    const double v = c->h_positions[(size_t)c->h_indices[i] * 3 + k];
-                    lo[k] = std::min(lo[k], v);
-                    hi[k] = std::max(hi[k], v);
-                }
-            const double cx = 0.5 * (lo[0] + hi[0]), cy = 0.5 * (lo[1] + hi[1]), cz = 0.5 * (lo[2] + hi[2]);
-            double r2 = 0.0;
-            for (uint64_t i = first + t0 * 3; i < first + t1 * 3; i++) {
-                const float* v = &c->h_positions[(size_t)c->h_indices[i] * 3];
-                const double dx = v[0] - cx, dy = v[1] - cy, dz = v[2] - cz;
-                r2 = std::max(r2, dx * dx + dy * dy + dz * dz);
-            }
-            const float fc[3] = {(float)cx, (float)cy, (float)cz};
-            // the centre was rounded to float: widen the radius by that much and by its own rounding
-            const double shift = fabs(fc[0] - cx) + fabs(fc[1] - cy) + fabs(fc[2] - cz);
-            float r = (float)((sqrt(r2) + shift) * (1.0 + 1e-6));
-            if (!(r == r) || !std::isfinite(r)) r = INFINITY;   // non-finite vertices: never culled
-            spheres.insert(spheres.end(), {fc[0], fc[1], fc[2], r});
-        }
+        base[p] = n;
+        n += (uint32_t)((tris + TR_CHUNK_TRIS - 1) / TR_CHUNK_TRIS);
     }
-    base[c->n_primitives] = (uint32_t)(spheres.size() / 4);
+    base[c->n_primitives] = n;
     TR_TRY(c->prim_chunk_base.ensure(base.size() * 4));
-    TR_TRY(c->chunk_spheres.ensure(std::max<size_t>(spheres.size() * 4, 16)));
+    TR_TRY(c->chunk_spheres.ensure(std::max<size_t>((size_t)n * 16, 16)));
     TR_CUDA(cudaMemcpyAsync(c->prim_chunk_base.p, base.data(), base.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    if (ok && !spheres.empty()) TR_CUDA(cudaMemcpyAsync(c->chunk_spheres.p, spheres.data(), spheres.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    TR_CUDA(cudaStreamSynchronize(c->stream));   // the sources are locals
+    c->n_chunks = ok ? n : 0u;
     c->chunk_cull = ok && !getenv("TR_NO_CHUNK_CULL");
     c->chunks_valid = true;
-    return TR_OK;
+    return launch_chunk_spheres(c);
 }
 
 // Upper bound of the visibility work list (every instance visible), recomputed after an instance / primitive upload.
@@ -526,7 +505,7 @@ int32_t tr_destroy(tr_ctx* c) {
                       &c->draws[2], &c->draws[3], &c->work_prefix, &c->slot_z, &c->slot_first, &c->block_entry, &c->chunk_spheres, &c->prim_chunk_base, &c->cluster_aabbs, &c->cluster_counts,
                       &c->cluster_indices, &c->vis[0], &c->vis[1], &c->bin_entries, &c->bin_state, &c->tri_records, &c->dev_status, &c->band_list, &c->hdr, &c->hdr_f32, &c->pyramid,
                       &c->srgb8, &c->mip_counter, &c->shade_counter, &c->accel_tlas, &c->accel_blas, &c->accel_inst, &c->accel_tris,
-                      &c->accel_prim_table, &c->accel_scratch, &c->shadow_mask[0], &c->shadow_mask[1]};
+                      &c->accel_prim_table, &c->accel_scratch, &c->accel_refit, &c->shadow_mask[0], &c->shadow_mask[1]};
     for (DevBuf* b : bufs) b->release();
     for (DevBuf& b : c->tex_data) b.release();
     c->tex_table.release();
@@ -793,11 +772,41 @@ int32_t tr_set_mesh(tr_ctx* c, const float* positions, const float* normals, con
     TR_TRY(upload(c, c->mesh_idx, indices, (size_t)n_indices * 4));
     c->n_vertices = n_vertices;
     c->n_indices = n_indices;
-    c->h_positions.assign(positions, positions + (size_t)n_vertices * 3);
-    c->h_indices.assign(indices, indices + n_indices);
     c->chunks_valid = false;
     c->scene_checked = false;
     c->accel_blas_valid = c->accel_tlas_valid = false;
+    return TR_OK;
+}
+
+// Vertex animation: the positions and normals of [first_vertex, first_vertex + n) in stream order on the context stream (not
+// the run-ahead upload stream: the frame in flight reads these buffers), then everything that depends on the positions, on
+// the device: the chunk spheres and, once built, the bottom-level trees (refit; the top level needs an update after it).
+int32_t tr_update_mesh_vertices(tr_ctx* c, uint32_t first_vertex, uint32_t n, const float* positions, const float* normals) {
+    TR_CHECK_CTX(c);
+    if (!c->mesh_pos.p) return fail(TR_ERR_STATE, "tr_update_mesh_vertices: no mesh (tr_set_mesh)");
+    if ((uint64_t)first_vertex + n > c->n_vertices)
+        return fail(TR_ERR_INVALID_ARG, "tr_update_mesh_vertices: vertices [%u, %u + %u) of %u", first_vertex, first_vertex, n, c->n_vertices);
+    if (n == 0) return TR_OK;
+    if (!positions || !normals) return fail(TR_ERR_INVALID_ARG, "tr_update_mesh_vertices: null");
+    TR_CUDA(cudaMemcpyAsync(c->mesh_pos.as<float>() + (size_t)first_vertex * 3, positions, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+    TR_CUDA(cudaMemcpyAsync(c->mesh_nrm.as<float>() + (size_t)first_vertex * 3, normals, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+    if (c->chunks_valid) TR_TRY(launch_chunk_spheres(c));
+    else TR_TRY(ensure_chunks(c));
+    if (c->accel_blas_valid) {
+        TR_TRY(accel_refit_blas(c));
+        c->accel_tlas_valid = false;   // the top level holds the old primitive boxes: it needs an update, as after tr_set_instances
+    }
+    return TR_OK;
+}
+
+int32_t tr_read_chunk_spheres(tr_ctx* c, float* spheres, uint32_t capacity, uint32_t* n_spheres) {
+    TR_CHECK_CTX(c);
+    TR_TRY(ensure_chunks(c));
+    const uint32_t n = c->n_chunks;
+    if (n_spheres) *n_spheres = n;
+    if (spheres && capacity < n) return fail(TR_ERR_INVALID_ARG, "tr_read_chunk_spheres: capacity %u < %u", capacity, n);
+    if (spheres && n) TR_CUDA(cudaMemcpyAsync(spheres, c->chunk_spheres.p, (size_t)n * 16, cudaMemcpyDeviceToHost, c->stream));
+    TR_CUDA(cudaStreamSynchronize(c->stream));
     return TR_OK;
 }
 
@@ -806,7 +815,6 @@ int32_t tr_build_acceleration_structures(tr_ctx* c, uint64_t* address) {
     TR_CHECK_CTX(c);
     if (!address) return fail(TR_ERR_INVALID_ARG, "tr_build_acceleration_structures: null");
     *address = 0;
-    c->accel_prim_table_valid = false;   // the device builder's primitive table follows the new bottom level
     TR_TRY(accel_build(c));
     *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
     return TR_OK;
@@ -840,6 +848,23 @@ int32_t tr_read_top_level_acceleration_structure(tr_ctx* c, void* nodes, uint32_
     if (nodes) TR_CUDA(cudaMemcpyAsync(nodes, c->accel_tlas.p, (size_t)nn * sizeof(trd::AccelNode), cudaMemcpyDeviceToHost, c->stream));
     if (instances && m)
         TR_CUDA(cudaMemcpyAsync(instances, c->accel_inst.p, (size_t)m * sizeof(trd::AccelInstance), cudaMemcpyDeviceToHost, c->stream));
+    TR_CUDA(cudaStreamSynchronize(c->stream));
+    return TR_OK;
+}
+
+int32_t tr_read_bottom_level_acceleration_structures(tr_ctx* c, void* nodes, uint32_t node_capacity, uint32_t* n_nodes, void* tris,
+                                                     uint32_t tri_capacity, uint32_t* n_tris) {
+    TR_CHECK_CTX(c);
+    if (!c->accel_blas_valid)
+        return fail(TR_ERR_STATE, "tr_read_bottom_level_acceleration_structures: acceleration structures not built");
+    const uint32_t nn = c->accel_blas_nodes, nt = c->accel_n_tris;
+    if (n_nodes) *n_nodes = nn;
+    if (n_tris) *n_tris = nt;
+    if ((nodes && node_capacity < nn) || (tris && tri_capacity < nt))
+        return fail(TR_ERR_INVALID_ARG, "tr_read_bottom_level_acceleration_structures: capacity %u nodes / %u triangles < %u / %u",
+                    node_capacity, tri_capacity, nn, nt);
+    if (nodes && nn) TR_CUDA(cudaMemcpyAsync(nodes, c->accel_blas.p, (size_t)nn * sizeof(trd::AccelNode), cudaMemcpyDeviceToHost, c->stream));
+    if (tris && nt) TR_CUDA(cudaMemcpyAsync(tris, c->accel_tris.p, (size_t)nt * 3 * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
     TR_CUDA(cudaStreamSynchronize(c->stream));
     return TR_OK;
 }

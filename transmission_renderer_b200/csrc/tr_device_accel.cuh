@@ -33,6 +33,14 @@ struct AccelInstance {  // 64 B, stored in top-level leaf order
 };
 static_assert(sizeof(AccelInstance) == 64, "AccelInstance");
 
+struct TlasPrim {  // what the top level needs of a primitive: the per-primitive table on the device (k_accel_device.cu)
+    float lo[3], hi[3];       // object-space box; a bottom-level refit rewrites it (k_mesh_update.cu)
+    uint32_t blas_root, tri_base;
+    uint32_t keep;            // draw_buffer_index < 2 and at least one triangle (src/main.rs:614-625)
+    uint32_t pad[3];
+};
+static_assert(sizeof(TlasPrim) == 48, "TlasPrim");
+
 struct AccelDesc {
     const float4* tlas_nodes;  // AccelNode[]; node 0 is the root
     const float4* blas_nodes;  // AccelNode[] of all primitives

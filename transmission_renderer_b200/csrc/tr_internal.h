@@ -90,10 +90,10 @@ struct tr_ctx {
     uint32_t* d_cull_scalars = nullptr;     // [0] n_visible [1] visible triangles [2..5] draw_counts [6,7] ~min/max bits of slot_z
     std::vector<uint32_t> h_prim_tris, h_inst_prim;  // host copies: triangles per primitive, primitive of each instance
     // cluster culling in the binning pass (k_visibility.cu): a bounding sphere per 64 consecutive triangles of every primitive,
-    // built on the host when the mesh or the primitives change (ensure_chunks)
-    std::vector<float> h_positions;
-    std::vector<uint32_t> h_indices;
+    // computed on the device when the mesh or the primitives change (ensure_chunks) and after every tr_update_mesh_vertices
     tr::DevBuf chunk_spheres, prim_chunk_base;   // float4 (object-space centre, radius) per chunk; first chunk of each primitive
+    std::vector<uint32_t> h_chunk_base;          // the host copy of prim_chunk_base (the source of its upload)
+    uint32_t n_chunks = 0;                       // spheres in chunk_spheres (0 when a primitive leaves the index buffer)
     bool chunks_valid = false, chunk_cull = false;
     std::vector<uint32_t> h_inst_mat, h_prim_first, h_prim_count;  // material of each instance; index range of each primitive
     std::vector<uint32_t> band_bounds;  // n_ranks + 1 row boundaries when the caller balances the bands itself (tr_set_bands)
@@ -118,13 +118,15 @@ struct tr_ctx {
     tr::DevBuf accel_tlas, accel_blas, accel_inst, accel_tris, shadow_mask[2];
     uint32_t accel_n_instances = 0;
     bool accel_blas_valid = false, accel_tlas_valid = false;
-    std::vector<float> h_prim_box;                                  // object-space box per primitive (lo, hi)
     std::vector<uint32_t> h_prim_root, h_prim_tri_base, h_prim_bucket;
-    // the device builder of the top level (k_accel_device.cu): per-primitive table, uploaded on the first update after
-    // tr_build_acceleration_structures, and the builder's scratch (grow-only)
+    // per-primitive table (trd::TlasPrim: object-space box, root, first triangle), uploaded by tr_build_acceleration_structures;
+    // the device builder of the top level reads it (k_accel_device.cu), and so does the host one, for the boxes that a
+    // bottom-level refit rewrites.  Then the device builder's scratch (grow-only).
     tr::DevBuf accel_prim_table, accel_scratch;
-    std::vector<uint8_t> h_accel_prims;   // the table's host copy (the source of its upload)
-    bool accel_prim_table_valid = false;
+    // bottom-level refit after tr_update_mesh_vertices (k_mesh_update.cu): parent of every node (-1 at a root), arrival
+    // counters, and the first index of every leaf-order triangle
+    tr::DevBuf accel_refit;
+    uint32_t accel_blas_nodes = 0, accel_n_tris = 0;
 
     // timing (profiling.rs zone taxonomy)
     bool timing = false;
@@ -222,6 +224,11 @@ int32_t accel_build_tlas(tr_ctx* c);  // top level only (instances moved)
 // the top level built on the device in stream order (k_accel_device.cu); launches kAsyncTlasLaunches kernels
 int32_t accel_build_tlas_async(tr_ctx* c);
 constexpr int kAsyncTlasLaunches = 19;
+// tr_update_mesh_vertices (k_mesh_update.cu): the chunk spheres in one launch, the bottom-level refit in two
+int32_t launch_chunk_spheres(tr_ctx* c);
+int32_t accel_refit_blas(tr_ctx* c);
+constexpr int kChunkSphereLaunches = 1;
+constexpr int kRefitLaunches = 2;
 int32_t launch_trace_rays(tr_ctx* c, uint32_t n, const float* d_origins, const float* d_directions, const float* d_t_max, uint8_t* d_lit);
 int32_t launch_generate_mips(uint2* pyramid, uint32_t levels, const uint32_t* w, const uint32_t* h, const uint32_t* off,
                              uint32_t* counter, int sm_count, cudaStream_t s);
@@ -239,7 +246,7 @@ int32_t launch_eval_ibl(uint32_t n, const trd::mat4& pv, const tr_ibl_volume_ref
 
 int32_t check_device_status(tr_ctx* c, const char* who);
 int32_t ensure_tri_bound(tr_ctx* c, const char* who);   // max_triangles: the work list's upper bound
-int32_t ensure_chunks(tr_ctx* c);   // (re)builds chunk_spheres / prim_chunk_base after a mesh or primitive upload
+int32_t ensure_chunks(tr_ctx* c);   // (re)builds chunk_spheres / prim_chunk_base after a mesh or primitive upload, in stream order
 int32_t validate_scene(tr_ctx* c, const char* who);  // instance -> primitive / material ids, primitive index ranges  // sticky device-side error bits -> TR_ERR_STATE
 void mat4_inverse_f64(const tr_mat4& m, tr_mat4* out);
 int32_t ensure_layer(tr_ctx* c, int layer, bool with_position);

@@ -125,6 +125,25 @@ class Renderer:
         p, n, u, i = _c(positions, np.float32), _c(normals, np.float32), _c(uvs, np.float32), _c(indices, np.uint32)
         _check(_lib().tr_set_mesh(self._ctx, _p(p), _p(n), _p(u), C.c_uint32(len(p)), _p(i), C.c_uint32(i.size)))
 
+    def update_mesh_vertices(self, positions, normals, first_vertex=0):
+        """New positions and normals ((n, 3) float32 each) for vertices [first_vertex, first_vertex + n) of the mesh, in
+        stream order: the culling spheres and, once built, the bottom-level acceleration structures follow on the device.
+        After it, a traced frame needs a top-level update first.  Page-locked arrays are read in stream order."""
+        p, n = _c(positions, np.float32).reshape(-1, 3), _c(normals, np.float32).reshape(-1, 3)
+        if len(p) != len(n):
+            raise ValueError(f"update_mesh_vertices: {len(p)} positions but {len(n)} normals")
+        _check(_lib().tr_update_mesh_vertices(self._ctx, C.c_uint32(first_vertex), C.c_uint32(len(p)), _p(p) if len(p) else None,
+                                              _p(n) if len(n) else None))
+
+    def read_chunk_spheres(self):
+        """(n, 4) float32: the binning pass's culling spheres (object-space centre, radius), one per 64 consecutive
+        triangles of every primitive, primitive after primitive."""
+        n = C.c_uint32(0)
+        _check(_lib().tr_read_chunk_spheres(self._ctx, None, C.c_uint32(0), C.byref(n)))
+        out = np.zeros((n.value, 4), np.float32)
+        _check(_lib().tr_read_chunk_spheres(self._ctx, _p(out) if len(out) else None, C.c_uint32(len(out)), C.byref(n)))
+        return out
+
     # -- ray-queried shadows (`--ray-tracing`, src/main.rs:577-658) ---------------------------
     def build_acceleration_structures(self):
         """Bottom-level structures of every primitive + the top level over the instances with draw_buffer_index < 2.
@@ -159,6 +178,20 @@ class Renderer:
         _check(_lib().tr_read_top_level_acceleration_structure(self._ctx, _p(nodes), C.c_uint32(len(nodes)), C.byref(nn),
                                                                 _p(inst) if len(inst) else None, C.c_uint32(len(inst)), C.byref(ni)))
         return nodes, inst
+
+    def read_bottom_level_acceleration_structure(self):
+        """(nodes, tris): every primitive's tree, abi.accel_node, one after the other in primitive order (each root first),
+        and the triangles in leaf order, (n, 3, 4) float32 (x, y, z, 0); leaf references count from the primitive's first
+        triangle."""
+        nn, nt = C.c_uint32(0), C.c_uint32(0)
+        _check(_lib().tr_read_bottom_level_acceleration_structures(self._ctx, None, C.c_uint32(0), C.byref(nn), None, C.c_uint32(0),
+                                                                    C.byref(nt)))
+        nodes = np.zeros(nn.value, dtype=abi.accel_node)
+        tris = np.zeros((nt.value, 3, 4), np.float32)
+        _check(_lib().tr_read_bottom_level_acceleration_structures(self._ctx, _p(nodes) if len(nodes) else None, C.c_uint32(len(nodes)),
+                                                                    C.byref(nn), _p(tris) if len(tris) else None, C.c_uint32(len(tris)),
+                                                                    C.byref(nt)))
+        return nodes, tris
 
     def trace_shadow_rays(self, origins, directions, t_max):
         """(n,3), (n,3), (n,) -> (n,) uint8: 1 = lit, 0 = occluded (trace_shadow_ray, lighting.rs:97-125)."""
