@@ -429,6 +429,14 @@ TR_API int32_t tr_read_chunk_spheres(tr_ctx* ctx, float* spheres, uint32_t capac
  * (src/main.rs:856-859); passing it to tr_frame / tr_shade_* turns the shadow rays on, 0 leaves them off.
  * Rebinding the mesh or the primitives invalidates it. */
 TR_API int32_t tr_build_acceleration_structures(tr_ctx* ctx, uint64_t* address);
+/* build_acceleration_structures_from_primitives + build_top_level_acceleration_structure_from_instances
+ * (src/acceleration_structures.rs:6-186), built on the device in stream order: the contract of
+ * tr_build_acceleration_structures (same handle rules, errors, invalidation and read-back hooks), but it reads the
+ * positions, indices and instances as the context stream sees them (it may follow tr_set_mesh, tr_update_mesh_vertices or
+ * tr_set_instances directly), never waits for the device and allocates only when a buffer grows.  The trees differ from
+ * the host build's (H-PLOC, single-triangle leaves: 64 B of nodes per triangle); every ray's result does not.  After
+ * refits, it is the cheap rebuild from the current pose. */
+TR_API int32_t tr_build_acceleration_structures_async(tr_ctx* ctx, uint64_t* address);
 /* update_top_level_acceleration_structure_from_instances (src/acceleration_structures.rs:188-263, src/main.rs:1332-1345):
  * after tr_set_instances.  The handle may change; it is returned again. */
 TR_API int32_t tr_update_top_level_acceleration_structure(tr_ctx* ctx, uint64_t* address);

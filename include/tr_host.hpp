@@ -391,6 +391,12 @@ public:
         TR_HOST_CHECK(tr_build_acceleration_structures(ctx_, &address));
         return address;
     }
+    // the same, built on the device in stream order without waiting for the GPU (also the rebuild after refits)
+    uint64_t build_acceleration_structures_async() {
+        uint64_t address = 0;
+        TR_HOST_CHECK(tr_build_acceleration_structures_async(ctx_, &address));
+        return address;
+    }
     // update_top_level_acceleration_structure_from_instances, src/acceleration_structures.rs:188-263: after set_instances
     uint64_t update_top_level_acceleration_structure() {
         uint64_t address = 0;

@@ -151,24 +151,6 @@ __global__ void __launch_bounds__(kScanThreads) tlas_bounds_kernel(const AccelIn
     }
 }
 
-__device__ __forceinline__ uint32_t spread10(uint32_t x) {  // 10 bits -> every third bit of 30
-    x &= 0x3ffu;
-    x = (x | (x << 16)) & 0x030000ffu;
-    x = (x | (x << 8)) & 0x0300f00fu;
-    x = (x | (x << 4)) & 0x030c30c3u;
-    x = (x | (x << 2)) & 0x09249249u;
-    return x;
-}
-
-// 10 bits per axis.  A zero, infinite or NaN extent, or a NaN centroid, quantises to 0 instead of an undefined
-// conversion: the codes only shape the tree, never the result.
-__device__ __forceinline__ uint32_t quantise(float c, float lo, float ext) {
-    const float t = (ext > 0.0f && ext <= 3.4e38f) ? (c - lo) / ext * 1024.0f : 0.0f;
-    if (!(t >= 0.0f)) return 0u;
-    if (t >= 1023.0f) return 1023u;
-    return (uint32_t)t;
-}
-
 __global__ void __launch_bounds__(kTile) tlas_codes_kernel(const AccelInstance* __restrict__ rec, uint32_t m, const float* __restrict__ bounds,
                                                            uint32_t* __restrict__ keys, uint32_t* __restrict__ vals) {
     const uint32_t i = blockIdx.x * kTile + threadIdx.x;
@@ -313,6 +295,8 @@ __global__ void __launch_bounds__(kTile) tlas_boxes_kernel(const AccelInstance* 
 }  // namespace
 
 namespace tr {
+
+void launch_block_scan(uint32_t* data, uint32_t len, cudaStream_t s) { tlas_scan_kernel<<<1, kScanThreads, 0, s>>>(data, len); }
 
 // Host side: the top-level count, the instance checks and the buffer sizes come from what the host holds; nothing
 // waits for the device unless a buffer grows.  The primitive table is on the device since tr_build_acceleration_structures

@@ -505,7 +505,7 @@ int32_t tr_destroy(tr_ctx* c) {
                       &c->draws[2], &c->draws[3], &c->work_prefix, &c->slot_z, &c->slot_first, &c->block_entry, &c->chunk_spheres, &c->prim_chunk_base, &c->cluster_aabbs, &c->cluster_counts,
                       &c->cluster_indices, &c->vis[0], &c->vis[1], &c->bin_entries, &c->bin_state, &c->tri_records, &c->dev_status, &c->band_list, &c->hdr, &c->hdr_f32, &c->pyramid,
                       &c->srgb8, &c->mip_counter, &c->shade_counter, &c->accel_tlas, &c->accel_blas, &c->accel_inst, &c->accel_tris,
-                      &c->accel_prim_table, &c->accel_scratch, &c->accel_refit, &c->shadow_mask[0], &c->shadow_mask[1]};
+                      &c->accel_prim_table, &c->accel_scratch, &c->accel_build_scratch, &c->accel_refit, &c->shadow_mask[0], &c->shadow_mask[1]};
     for (DevBuf* b : bufs) b->release();
     for (DevBuf& b : c->tex_data) b.release();
     c->tex_table.release();
@@ -640,10 +640,12 @@ int32_t tr_set_primitives(tr_ctx* c, const tr_primitive_info* prims, uint32_t n)
     c->h_prim_tris.resize(n);
     c->h_prim_first.resize(n);
     c->h_prim_count.resize(n);
+    c->h_prim_bucket.resize(n);
     for (uint32_t i = 0; i < n; i++) {
         c->h_prim_tris[i] = prims[i].index_count / 3u;
         c->h_prim_first[i] = prims[i].first_index;
         c->h_prim_count[i] = prims[i].index_count;
+        c->h_prim_bucket[i] = prims[i].draw_buffer_index;
     }
     c->scene_checked = false;
     c->tri_bound_valid = false;
@@ -816,6 +818,15 @@ int32_t tr_build_acceleration_structures(tr_ctx* c, uint64_t* address) {
     if (!address) return fail(TR_ERR_INVALID_ARG, "tr_build_acceleration_structures: null");
     *address = 0;
     TR_TRY(accel_build(c));
+    *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
+    return TR_OK;
+}
+
+int32_t tr_build_acceleration_structures_async(tr_ctx* c, uint64_t* address) {
+    TR_CHECK_CTX(c);
+    if (!address) return fail(TR_ERR_INVALID_ARG, "tr_build_acceleration_structures_async: null");
+    *address = 0;
+    TR_TRY(accel_build_async(c));
     *address = (uint64_t)(uintptr_t)c->accel_tlas.p;
     return TR_OK;
 }

@@ -118,7 +118,7 @@ struct tr_ctx {
     tr::DevBuf accel_tlas, accel_blas, accel_inst, accel_tris, shadow_mask[2];
     uint32_t accel_n_instances = 0;
     bool accel_blas_valid = false, accel_tlas_valid = false;
-    std::vector<uint32_t> h_prim_root, h_prim_tri_base, h_prim_bucket;
+    std::vector<uint32_t> h_prim_root, h_prim_tri_base, h_prim_bucket;   // h_prim_bucket: draw_buffer_index (tr_set_primitives)
     // per-primitive table (trd::TlasPrim: object-space box, root, first triangle), uploaded by tr_build_acceleration_structures;
     // the device builder of the top level reads it (k_accel_device.cu), and so does the host one, for the boxes that a
     // bottom-level refit rewrites.  Then the device builder's scratch (grow-only).
@@ -127,6 +127,8 @@ struct tr_ctx {
     // counters, and the first index of every leaf-order triangle
     tr::DevBuf accel_refit;
     uint32_t accel_blas_nodes = 0, accel_n_tris = 0;
+    // the scratch of the bottom level built on the device (k_accel_build.cu), grow-only
+    tr::DevBuf accel_build_scratch;
 
     // timing (profiling.rs zone taxonomy)
     bool timing = false;
@@ -224,6 +226,11 @@ int32_t accel_build_tlas(tr_ctx* c);  // top level only (instances moved)
 // the top level built on the device in stream order (k_accel_device.cu); launches kAsyncTlasLaunches kernels
 int32_t accel_build_tlas_async(tr_ctx* c);
 constexpr int kAsyncTlasLaunches = 19;
+// the bottom level built on the device in stream order, then the top level (k_accel_build.cu); launches
+// async_blas_launches(n_primitives) + kAsyncTlasLaunches kernels
+int32_t accel_build_async(tr_ctx* c);
+int async_blas_launches(uint32_t n_primitives);
+void launch_block_scan(uint32_t* data, uint32_t len, cudaStream_t s);   // exclusive, one block (k_accel_device.cu)
 // tr_update_mesh_vertices (k_mesh_update.cu): the chunk spheres in one launch, the bottom-level refit in two
 int32_t launch_chunk_spheres(tr_ctx* c);
 int32_t accel_refit_blas(tr_ctx* c);

@@ -153,6 +153,14 @@ class Renderer:
         self.acceleration_structure_address = a.value
         return a.value
 
+    def build_acceleration_structures_async(self):
+        """The same structures built on the device in stream order: returns the handle without waiting for the GPU and
+        reads the mesh and instances as the stream sees them (also the rebuild after update_mesh_vertices refits)."""
+        a = C.c_uint64(0)
+        _check(_lib().tr_build_acceleration_structures_async(self._ctx, C.byref(a)))
+        self.acceleration_structure_address = a.value
+        return a.value
+
     def update_top_level_acceleration_structure(self):
         a = C.c_uint64(0)
         _check(_lib().tr_update_top_level_acceleration_structure(self._ctx, C.byref(a)))
