@@ -7,18 +7,14 @@ import time
 import numpy as np
 import pytest
 
+from accel_checks import ACCEL_STACK, ASYNC_TLAS_LAUNCHES
+from accel_checks import _check_blas, _deform, _hold, _pinned, _random_rays, _records_key, _reference, _surface_rays, _tree_checks, _upload_scene
 from pipeline import REL_L2_TOL, rel_l2
-from test_gpu_accel_update import _hold, _tree_checks
-from test_gpu_mesh_update import _check_blas, _deform, _pinned, _records_key
-from test_gpu_shadows import _random_rays, _reference, _upload_scene
-from test_oracle_shadows import _surface_rays
 from transmission_renderer_b200 import Renderer, RendererGroup, TrError, abi, host, scenes
 
 pytestmark = pytest.mark.gpu
 f32 = np.float32
 TR_ERR_INVALID_ARG, TR_ERR_STATE = -1, -6
-ACCEL_STACK = 64               # kAccelStack, tr_device_accel.cuh
-ASYNC_TLAS_LAUNCHES = 19       # kAsyncTlasLaunches
 
 
 def _async_build_launches(n_prims):

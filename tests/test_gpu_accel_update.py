@@ -6,69 +6,14 @@ import time
 import numpy as np
 import pytest
 
+from accel_checks import ACCEL_STACK, ASYNC_TLAS_LAUNCHES as ASYNC_UPDATE_LAUNCHES
+from accel_checks import _hold, _pinned, _random_rays, _reference, _surface_rays, _tree_checks, _upload_scene
 from pipeline import REL_L2_TOL, rel_l2
-from test_gpu_shadows import _random_rays, _reference, _upload_scene
-from test_oracle_shadows import _surface_rays
 from transmission_renderer_b200 import Renderer, RendererGroup, TrError, abi, host, scenes
 
 pytestmark = pytest.mark.gpu
 f32 = np.float32
 TR_ERR_INVALID_ARG, TR_ERR_STATE = -1, -6
-ASYNC_UPDATE_LAUNCHES = 19     # count, scan, records, bounds, codes, 4 x (histogram, scan, scatter), hierarchy, boxes
-ACCEL_STACK = 64               # kAccelStack, tr_device_accel.cuh
-
-
-def _tree_checks(nodes, inst):
-    """Every leaf once, every inner box the exact union of its subtree; returns the depth (inner nodes on the longest path)."""
-    m = len(inst)
-    if m == 0:
-        assert len(nodes) == 1 and nodes["c0"][0] == -1 and nodes["c1"][0] == -1
-        assert np.all(np.isinf(nodes["lo0"])) and np.all(np.isinf(nodes["lo1"]))
-        return 1
-    seen = np.zeros(m, np.int64)
-    depth = 0
-
-    def box_of(c):   # (lo, hi) of a child reference
-        if c < 0:
-            code = ~int(c) & 0xFFFFFFFF
-            first, count = code & 0x0FFFFFFF, (code >> 28) + 1
-            seen[first:first + count] += 1
-            return inst["lo"][first:first + count].min(0), inst["hi"][first:first + count].max(0)
-        return walk(c)
-
-    stack_boxes = {}
-
-    def walk(root):   # iterative post-order: (node, depth, children done)
-        nonlocal depth
-        todo = [(root, 1, False)]
-        while todo:
-            n, d, done = todo.pop()
-            depth = max(depth, d)
-            kids = [int(nodes["c0"][n]), int(nodes["c1"][n])]
-            if m == 1 and n == 0:
-                kids = kids[:1]
-            if not done:
-                todo.append((n, d, True))
-                for c in kids:
-                    if c >= 0:
-                        todo.append((c, d + 1, False))
-                continue
-            lo, hi = [], []
-            for k, c in enumerate(kids):
-                b = stack_boxes.pop(c) if c >= 0 else box_of(c)
-                want_lo, want_hi = nodes["lo0" if k == 0 else "lo1"][n], nodes["hi0" if k == 0 else "hi1"][n]
-                assert np.array_equal(want_lo, b[0]) and np.array_equal(want_hi, b[1]), \
-                    f"node {n} child {k}: box is not the union of its subtree"
-                lo.append(b[0])
-                hi.append(b[1])
-            stack_boxes[n] = (np.min(lo, 0), np.max(hi, 0))
-        return stack_boxes.pop(root)
-
-    walk(0)
-    if m == 1:
-        assert np.all(np.isinf(nodes["lo1"][0])) and np.all(np.isinf(nodes["hi1"][0]))
-    assert (seen == 1).all(), "a top-level instance is missing or repeated"
-    return depth
 
 
 def _same_records(a, b):
@@ -205,14 +150,6 @@ def _rotated_frames(instances, n_frames):
     return out
 
 
-def _pinned(like):
-    import torch
-    t = torch.empty(len(like) * abi.instance.itemsize, dtype=torch.uint8).pin_memory()
-    a = t.numpy().view(abi.instance)
-    a[:] = like
-    return t, a
-
-
 def test_animation_matches_host_update(oracle, ggx_lut):
     """8 frames in which every instance rotates: async update (pinned uploads, no sync between frames) against the host
     update, masks of both layers, HDR and sRGB8 equal frame by frame; the last frame against the oracle."""
@@ -259,13 +196,6 @@ def test_animation_matches_host_update(oracle, ggx_lut):
     ref = _reference(oracle, ggx_lut, s2, oracle.Accel(s2["mesh"], s2["instances"], s2["primitives"]))
     assert (want[-1][0] != oracle.shadow_mask_frame(ref["g0"], ref["scene"])).sum() == 0
     assert rel_l2(last32[..., :3], ref["t32"][..., :3]) < REL_L2_TOL
-
-
-def _hold(stream, seconds):
-    import torch
-    clock_khz = getattr(torch.cuda.get_device_properties(0), "clock_rate", 0) or 2_100_000
-    with torch.cuda.stream(stream):
-        torch.cuda._sleep(int(seconds * clock_khz * 1e3))   # >= `seconds`: the cycles at the highest clock
 
 
 def test_async_update_does_not_block(ggx_lut):

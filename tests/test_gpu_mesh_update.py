@@ -8,18 +8,15 @@ import time
 import numpy as np
 import pytest
 
+from accel_checks import MESH_UPDATE_LAUNCHES, MESH_UPDATE_LAUNCHES_NO_ACCEL
+from accel_checks import _check_blas, _deform, _hold, _pinned, _random_rays, _records_key, _reference, _surface_rays, _upload_scene
 from pipeline import REL_L2_TOL, rel_l2
-from test_gpu_accel_update import _hold
-from test_gpu_shadows import _random_rays, _reference, _upload_scene
-from test_oracle_shadows import _surface_rays
 from transmission_renderer_b200 import Renderer, RendererGroup, TrError, abi, host, scenes
 
 pytestmark = pytest.mark.gpu
 f32 = np.float32
 TR_ERR_INVALID_ARG, TR_ERR_STATE = -1, -6
 CHUNK = 64                     # TR_CHUNK_TRIS
-MESH_UPDATE_LAUNCHES = 3       # chunk spheres; with built acceleration structures also the refit's gather and boxes
-MESH_UPDATE_LAUNCHES_NO_ACCEL = 1
 
 
 # ---------------------------------------------------------------------------------------------------------- restatements
@@ -61,24 +58,6 @@ def _chunk_spheres(pos, idx, prims):
     return np.array(out, f32).reshape(-1, 4)
 
 
-def _deform(mesh, k, first=0, last=None, amp=0.04):
-    """Vertices [first, last) displaced along their normals by a moving sine, normals tilted with it: (positions, normals)
-    of the range and the whole new mesh."""
-    last = len(mesh["positions"]) if last is None else last
-    p = mesh["positions"][first:last].astype(np.float64)
-    n = mesh["normals"][first:last].astype(np.float64)
-    a = amp * np.sin(3.0 * p[:, 0] + 2.0 * p[:, 2] + 0.9 * k)
-    newp = (p + a[:, None] * n).astype(f32)
-    newn = n + 0.2 * np.cos(2.0 * p[:, 1] + 0.7 * k)[:, None] * np.array([0.3, 0.0, -0.2])
-    newn = (newn / np.linalg.norm(newn, axis=1, keepdims=True)).astype(f32)
-    full = dict(mesh)
-    full["positions"] = mesh["positions"].copy()
-    full["normals"] = mesh["normals"].copy()
-    full["positions"][first:last] = newp
-    full["normals"][first:last] = newn
-    return newp, newn, full
-
-
 def _vertex_ranges(s):
     """[first vertex, end) of every primitive of a MeshSet scene (from its index ranges)."""
     idx = s["mesh"]["indices"]
@@ -87,12 +66,6 @@ def _vertex_ranges(s):
         sl = idx[int(p["first_index"]):int(p["first_index"]) + int(p["index_count"])]
         out.append((int(sl.min()), int(sl.max()) + 1))
     return out
-
-
-def _pinned(a):
-    import torch
-    t = torch.from_numpy(np.ascontiguousarray(a)).pin_memory()
-    return t, t.numpy()
 
 
 def _fresh(w, h, lut, s, mesh, accel=True, f32_debug=False):
@@ -209,77 +182,6 @@ def test_raster_path_matches_fresh_context(oracle, ggx_lut):
 
 
 # ---------------------------------------------------------------------------------------------------------- 3. refit
-def _blas_layout(nodes, prims):
-    """(root node, first triangle) of every primitive: the trees lie one after the other in preorder."""
-    roots, bases, root, base = [], [], 0, 0
-    for p in prims:
-        roots.append(root)
-        bases.append(base)
-        base += int(p["index_count"]) // 3
-        todo, count = [root], 0
-        while todo:
-            n = todo.pop()
-            count += 1
-            for c in (int(nodes["c0"][n]), int(nodes["c1"][n])):
-                if c >= 0:
-                    todo.append(c)
-        root += count
-    assert root == len(nodes)
-    return roots, bases
-
-
-def _check_blas(nodes, tris, prims, mesh):
-    """Per primitive: the triangles are the mesh's, as a multiset; every box is the exact union of its subtree (a zero may
-    carry either sign)."""
-    pos, idx = mesh["positions"], mesh["indices"]
-    roots, bases = _blas_layout(nodes, prims)
-    inf = np.float32(np.inf)
-    for p, (root, base) in enumerate(zip(roots, bases)):
-        nt = int(prims["index_count"][p]) // 3
-        want = pos[idx[int(prims["first_index"][p]):int(prims["first_index"][p]) + nt * 3]].reshape(nt, 9)
-        got = tris[base:base + nt, :, :3].reshape(nt, 9)
-        assert (tris[base:base + nt, :, 3] == 0).all()
-        key = lambda a: np.sort(np.ascontiguousarray(a + f32(0)).view(np.dtype((np.void, 36))).reshape(-1))
-        assert key(got).tobytes() == key(want).tobytes(), f"primitive {p}: triangles differ"
-        end = roots[p + 1] if p + 1 < len(roots) else len(nodes)
-        boxes = {}
-
-        def leaf(c):
-            code = ~c & 0xFFFFFFFF
-            first, count = code & 0x0FFFFFFF, (code >> 28) + 1
-            t = tris[base + first:base + first + count, :, :3].reshape(-1, 3)
-            return t.min(0), t.max(0)
-
-        for n in range(end - 1, root - 1, -1):   # children after their parent
-            c0, c1 = int(nodes["c0"][n]), int(nodes["c1"][n])
-            if c0 == c1:                           # the special roots
-                assert n == root
-                assert np.all(nodes["lo1"][n] == inf) and np.all(nodes["hi1"][n] == -inf)
-                if nt == 0:
-                    assert np.all(nodes["lo0"][n] == inf) and np.all(nodes["hi0"][n] == -inf)
-                else:
-                    lo, hi = leaf(c0)
-                    assert np.array_equal(nodes["lo0"][n], lo) and np.array_equal(nodes["hi0"][n], hi)
-                continue
-            los, his = [], []
-            for k, c in enumerate((c0, c1)):
-                lo, hi = leaf(c) if c < 0 else boxes.pop(c)
-                assert np.array_equal(nodes["lo0" if k == 0 else "lo1"][n], lo), f"primitive {p} node {n} child {k}"
-                assert np.array_equal(nodes["hi0" if k == 0 else "hi1"][n], hi), f"primitive {p} node {n} child {k}"
-                los.append(lo)
-                his.append(hi)
-            boxes[n] = np.min(los, 0), np.max(his, 0)
-
-
-def _records_key(inst):
-    """Top-level records as a multiset, blas_root left out (a fresh build makes other trees), +0 for -0."""
-    rec = inst.copy()
-    for f in ("translation", "inv_scale", "conj_rotation", "lo", "hi"):
-        rec[f] = rec[f] + f32(0)
-    rec["blas_root"] = 0
-    return np.sort(np.frombuffer(rec.tobytes(), np.dtype((np.void, 64))))
-
-
 @pytest.mark.parametrize("kind", ["shadow", "instanced"])
 def test_refit(oracle, ggx_lut, kind):
     w, h = 320, 180

@@ -4,32 +4,12 @@ HDR tolerance, the call-order rules of the handle."""
 import numpy as np
 import pytest
 
-from pipeline import REL_L2_TOL, gpu_setup, oracle_cluster_lights, oracle_scene, rel_l2
-from test_oracle_shadows import _surface_rays
+from accel_checks import _random_rays, _reference, _surface_rays, _upload_scene
+from pipeline import REL_L2_TOL, rel_l2
 from transmission_renderer_b200 import Renderer, TrError, abi, host, scenes
 
 pytestmark = pytest.mark.gpu
 f32 = np.float32
-
-
-def _upload_scene(r, lut, s):
-    gpu_setup(r, lut, s["uniforms"], s["materials"], s["lights"])
-    r.set_instances(s["instances"])
-    r.set_primitives(s["primitives"])
-    m = s["mesh"]
-    r.set_mesh(m["positions"], m["normals"], m["uvs"], m["indices"])
-    r.build_clusters(s["camera"].write_cluster_data())
-
-
-def _random_rays(rng, n, lo, hi):
-    o = rng.uniform(lo, hi, (n, 3)).astype(f32)
-    d = rng.normal(size=(n, 3))
-    d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(f32)
-    d[::7, rng.integers(0, 3)] = 0.0
-    d[::11] = np.sign(d[::11]) * (np.abs(d[::11]) > 0.5)
-    t = rng.uniform(0.5, 60, n).astype(f32)
-    ok = np.linalg.norm(d, axis=1) > 0
-    return o[ok], d[ok], t[ok]
 
 
 @pytest.mark.parametrize("kind", ["shadow", "instanced"])
@@ -55,20 +35,6 @@ def test_ray_batches_bit_exact(oracle, ggx_lut, kind):
     assert 0.02 < 1 - ref.mean() < 0.98 and 0.02 < 1 - ref_p.mean() < 0.98
     sub = slice(0, 20000)
     assert np.array_equal(got[sub], acc.trace(o[sub], d[sub], t[sub], brute=True))
-
-
-def _reference(oracle, lut, s, accel):
-    cam = s["camera"]
-    pc = cam.push_constants()
-    _, visible = oracle.frustum_culling(s["instances"], s["primitives"], cam.culling())
-    g0, g1 = oracle.visibility(s["mesh"], s["instances"], s["primitives"], visible, pc)
-    _, cc, ci = oracle_cluster_lights(oracle, cam, s["uniforms"], s["lights"])
-    sc = oracle_scene(pc, s["uniforms"], s["materials"], s["lights"], cc, ci)
-    sc["accel"] = accel
-    o32, o16 = oracle.shade_opaque_frame(g0, sc)
-    levels = oracle.build_pyramid(o16)
-    t32, t16 = oracle.shade_transmission_frame(g1, sc, levels, lut, o32, o16)
-    return dict(g0=g0, g1=g1, scene=sc, o32=o32, o16=o16, t32=t32)
 
 
 @pytest.mark.parametrize("size", [(640, 360), (333, 187)])

@@ -4,6 +4,7 @@ effect on a shaded frame."""
 import numpy as np
 import pytest
 
+from accel_checks import _surface_rays
 from pipeline import oracle_cluster_lights, oracle_scene
 from transmission_renderer_b200 import abi, host, scenes
 
@@ -59,24 +60,6 @@ def test_instance_transform_and_top_level_filter(oracle):
         assert acc.n_instances == (1 if casts else 0)
         lit = acc.trace(np.zeros((1, 3), f32), np.array([(0, 1, 0)], f32), np.array([10.0], f32))[0]
         assert lit == (0 if casts else 1)
-
-
-def _surface_rays(s, oracle, n, rng):
-    """Rays as the shaders cast them: from points on the visible surfaces towards the lights and the sun."""
-    cam = s["camera"]
-    _, visible = oracle.frustum_culling(s["instances"], s["primitives"], cam.culling())
-    g0, _ = oracle.visibility(s["mesh"], s["instances"], s["primitives"], visible, cam.push_constants())
-    ys, xs = np.nonzero(g0["depth"] > 0)
-    pick = rng.choice(len(ys), n)
-    ys, xs = ys[pick], xs[pick]
-    inv = np.linalg.inv(cam.proj_view.astype(np.float64))
-    ndc = np.stack([(xs + 0.5) / cam.width * 2 - 1, (ys + 0.5) / cam.height * 2 - 1, g0["depth"][ys, xs], np.ones(n)], 1)
-    h = ndc @ inv.T
-    pos = (h[:, :3] / h[:, 3:]).astype(f32)
-    lp = s["lights"]["position_and_spotlight_epsilon"][rng.integers(0, len(s["lights"]), n), :3]
-    vec = lp - pos
-    dist = np.linalg.norm(vec, axis=1).astype(f32)
-    return pos, (vec / dist[:, None]).astype(f32), dist
 
 
 def test_tree_walk_equals_the_definition(oracle):

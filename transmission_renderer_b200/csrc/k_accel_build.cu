@@ -31,22 +31,17 @@
 #include <algorithm>
 #include <cstdlib>
 
-#include "tr_device_accel.cuh"
+#include "tr_device_build.cuh"
 #include "tr_internal.h"
 
 using namespace trd;
 
 namespace {
 
-constexpr int kThreads = 256;          // items per block of every per-item kernel
-constexpr int kRadixBits = 8;
-constexpr int kRadix = 1 << kRadixBits;
-constexpr int kScanThreads = 1024;
 constexpr int kScanChunk = kScanThreads * 4;   // entries per block of the two-level scan
 constexpr int kPlocRadius = 8;
 constexpr int kPlocThreshold = 16;     // two children's lists of at most 16 clusters fill a warp
 constexpr uint32_t kInvalid = 0xffffffffu;
-static_assert(kThreads == kRadix, "the histogram kernel keeps one digit per thread");
 static_assert(2 * kPlocThreshold <= 32, "a node's two cluster lists fit in one warp");
 
 struct BuildPrim {             // per primitive, assembled on the device (build_init_kernel)
@@ -81,53 +76,13 @@ __device__ __forceinline__ Cluster load_cluster(const float4* cbox, uint32_t id)
 
 // the primitive owning triangle g: the last whose tri_base <= g (primitives without triangles share their successor's)
 __device__ __forceinline__ uint32_t prim_of(const BuildPrim* bp, uint32_t n_prims, uint32_t g) {
-    uint32_t lo = 0, hi = n_prims;
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (__ldg(&bp[mid].tri_base) <= g) lo = mid;
-        else hi = mid;
-    }
-    return lo;
+    return last_at_most(n_prims, g, [&](uint32_t p) { return __ldg(&bp[p].tri_base); });
 }
 
-struct Tri {
-    float4 v[3];
-};
-
-__device__ __forceinline__ Tri load_tri(const float* pos, const uint32_t* idx, uint32_t first) {
-    Tri t;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        const uint32_t v = __ldg(idx + first + k);
-        t.v[k] = make_float4(__ldg(pos + (size_t)v * 3), __ldg(pos + (size_t)v * 3 + 1), __ldg(pos + (size_t)v * 3 + 2), 0.0f);
-    }
-    return t;
-}
-
-// the triangle's box as the host folds it (box_grow per vertex), and its leaf box (box_union into an empty box), as
-// k_mesh_update.cu leaf_box does
-__device__ __forceinline__ void tri_box(const Tri& t, float* tlo, float* thi) {
-    const float inf = __int_as_float(0x7f800000);
-    tlo[0] = tlo[1] = tlo[2] = inf;
-    thi[0] = thi[1] = thi[2] = -inf;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        tlo[0] = fminf(tlo[0], t.v[k].x); thi[0] = fmaxf(thi[0], t.v[k].x);
-        tlo[1] = fminf(tlo[1], t.v[k].y); thi[1] = fmaxf(thi[1], t.v[k].y);
-        tlo[2] = fminf(tlo[2], t.v[k].z); thi[2] = fmaxf(thi[2], t.v[k].z);
-    }
-}
-
-__device__ __forceinline__ Cluster leaf_cluster(const Tri& t) {
-    const float inf = __int_as_float(0x7f800000);
-    float tlo[3], thi[3];
-    tri_box(t, tlo, thi);
+__device__ __forceinline__ Cluster leaf_cluster(const Tri& t) {   // a leaf of one triangle
     Cluster c;
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        c.lo[k] = fminf(fminf(inf, tlo[k]), thi[k]);
-        c.hi[k] = fmaxf(fmaxf(-inf, tlo[k]), thi[k]);
-    }
+    empty_box(c.lo, c.hi);
+    fold_tri(t, c.lo, c.hi);
     c.inner = 0;
     c.tris = 1;
     return c;
@@ -144,9 +99,9 @@ enum { W_COUNTER = 0, W_START = 1 };
 
 // Launch 1: per primitive, its triangles and its node count; their exclusive scans (launches 2 and 3) are the first
 // triangle and the root of every primitive, the offsets the host computes on its own for its checks and handles.
-__global__ void __launch_bounds__(kThreads) build_counts_kernel(const tr_primitive_info* __restrict__ prims, uint32_t n_prims,
-                                                                uint32_t* __restrict__ tri_base, uint32_t* __restrict__ node_base) {
-    const uint32_t p = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_counts_kernel(const tr_primitive_info* __restrict__ prims, uint32_t n_prims,
+                                                             uint32_t* __restrict__ tri_base, uint32_t* __restrict__ node_base) {
+    const uint32_t p = blockIdx.x * kTile + threadIdx.x;
     if (p >= n_prims) return;
     const uint32_t nt = prims[p].index_count / 3u;
     tri_base[p] = nt;
@@ -156,17 +111,17 @@ __global__ void __launch_bounds__(kThreads) build_counts_kernel(const tr_primiti
 // Launch 4: per primitive, its BuildPrim, the centroid bounds and depth start empty, and the nt <= 1 trees are written whole (build_tree:
 // the empty root, or the leaf wrapped in a root whose second box is empty).  Per cluster id, no parent; per sorted
 // position, the leaf is its own cluster list and no thread has reached its parent boundary yet.
-__global__ void __launch_bounds__(kThreads) build_init_kernel(const tr_primitive_info* __restrict__ prims, const uint32_t* __restrict__ tri_base,
-                                                              const uint32_t* __restrict__ node_base, BuildPrim* __restrict__ bp,
-                                                              uint32_t n_prims, uint32_t n,
-                                                              const float* __restrict__ pos, const uint32_t* __restrict__ idx,
-                                                              uint32_t* __restrict__ pbounds, uint32_t* __restrict__ pdepth,
-                                                              uint32_t* __restrict__ words, int32_t* __restrict__ tparent,
-                                                              uint32_t* __restrict__ cidx, int32_t* __restrict__ pidx,
-                                                              AccelNode* __restrict__ nodes, float4* __restrict__ tris,
-                                                              int32_t* __restrict__ parent, uint32_t* __restrict__ arrivals,
-                                                              uint32_t* __restrict__ tri_src, TlasPrim* __restrict__ table) {
-    const uint32_t i = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_init_kernel(const tr_primitive_info* __restrict__ prims, const uint32_t* __restrict__ tri_base,
+                                                           const uint32_t* __restrict__ node_base, BuildPrim* __restrict__ bp,
+                                                           uint32_t n_prims, uint32_t n,
+                                                           const float* __restrict__ pos, const uint32_t* __restrict__ idx,
+                                                           uint32_t* __restrict__ pbounds, uint32_t* __restrict__ pdepth,
+                                                           uint32_t* __restrict__ words, int32_t* __restrict__ tparent,
+                                                           uint32_t* __restrict__ cidx, int32_t* __restrict__ pidx,
+                                                           AccelNode* __restrict__ nodes, float4* __restrict__ tris,
+                                                           int32_t* __restrict__ parent, uint32_t* __restrict__ arrivals,
+                                                           uint32_t* __restrict__ tri_src, TlasPrim* __restrict__ table) {
+    const uint32_t i = blockIdx.x * kTile + threadIdx.x;
     if (i < 3 * n) tparent[i] = -1;
     if (i < n) {
         cidx[i] = i;
@@ -189,35 +144,18 @@ __global__ void __launch_bounds__(kThreads) build_init_kernel(const tr_primitive
     b.pad[0] = b.pad[1] = b.pad[2] = 0u;
     bp[i] = b;
     if (b.nt >= 2) return;
-    const float inf = __int_as_float(0x7f800000);
-    TlasPrim tp;
-    tp.lo[0] = tp.lo[1] = tp.lo[2] = inf;
-    tp.hi[0] = tp.hi[1] = tp.hi[2] = -inf;
-    tp.blas_root = b.node_base;
-    tp.tri_base = b.tri_base;
-    tp.keep = b.keep;
-    tp.pad[0] = tp.pad[1] = tp.pad[2] = 0u;
-    AccelNode r;
-    for (int k = 0; k < 3; k++) {
-        r.lo0[k] = r.lo1[k] = inf;
-        r.hi0[k] = r.hi1[k] = -inf;
-    }
-    r.c0 = r.c1 = ~0;
-    r.pad[0] = r.pad[1] = 0u;
+    float lo[3], hi[3];
+    empty_box(lo, hi);
     if (b.nt == 1) {
         const Tri t = load_tri(pos, idx, b.first_index);
-        const Cluster c = leaf_cluster(t);
-        for (int k = 0; k < 3; k++) {
-            r.lo0[k] = tp.lo[k] = c.lo[k];
-            r.hi0[k] = tp.hi[k] = c.hi[k];
-        }
+        fold_tri(t, lo, hi);
         for (int k = 0; k < 3; k++) tris[(size_t)b.tri_base * 3 + k] = t.v[k];
         tri_src[b.tri_base] = b.first_index;
     }
-    nodes[b.node_base] = r;
+    nodes[b.node_base] = special_root(lo, hi);
     parent[b.node_base] = -1;
     arrivals[b.node_base] = 0u;
-    table[i] = tp;
+    table[i] = make_tlas_prim(lo, hi, b.node_base, b.tri_base, b.keep);
 }
 
 __device__ __forceinline__ void centroid(const Tri& t, float* c) {   // lo + hi, as build_range
@@ -227,10 +165,10 @@ __device__ __forceinline__ void centroid(const Tri& t, float* c) {   // lo + hi,
 }
 
 // Launch 2: every primitive's centroid bounds (NaN centroids left out)
-__global__ void __launch_bounds__(kThreads) build_bounds_kernel(const BuildPrim* __restrict__ bp, uint32_t n_prims, uint32_t n,
-                                                                const float* __restrict__ pos, const uint32_t* __restrict__ idx,
-                                                                uint32_t* __restrict__ pbounds) {
-    const uint32_t g = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_bounds_kernel(const BuildPrim* __restrict__ bp, uint32_t n_prims, uint32_t n,
+                                                             const float* __restrict__ pos, const uint32_t* __restrict__ idx,
+                                                             uint32_t* __restrict__ pbounds) {
+    const uint32_t g = blockIdx.x * kTile + threadIdx.x;
     if (g >= n) return;
     const uint32_t p = prim_of(bp, n_prims, g);
     const BuildPrim b = bp[p];
@@ -244,11 +182,11 @@ __global__ void __launch_bounds__(kThreads) build_bounds_kernel(const BuildPrim*
 }
 
 // Launch 3: keys (primitive << 30 | code) and values (triangle) in the initial order, which is (primitive, position)
-__global__ void __launch_bounds__(kThreads) build_codes_kernel(const BuildPrim* __restrict__ bp, uint32_t n_prims, uint32_t n,
-                                                               const float* __restrict__ pos, const uint32_t* __restrict__ idx,
-                                                               const uint32_t* __restrict__ pbounds, uint64_t* __restrict__ keys,
-                                                               uint32_t* __restrict__ vals) {
-    const uint32_t g = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_codes_kernel(const BuildPrim* __restrict__ bp, uint32_t n_prims, uint32_t n,
+                                                            const float* __restrict__ pos, const uint32_t* __restrict__ idx,
+                                                            const uint32_t* __restrict__ pbounds, uint64_t* __restrict__ keys,
+                                                            uint32_t* __restrict__ vals) {
+    const uint32_t g = blockIdx.x * kTile + threadIdx.x;
     if (g >= n) return;
     const uint32_t p = prim_of(bp, n_prims, g);
     const BuildPrim b = bp[p];
@@ -264,45 +202,8 @@ __global__ void __launch_bounds__(kThreads) build_codes_kernel(const BuildPrim* 
     vals[g] = g;
 }
 
-// Stable LSD radix sort, one 8-bit digit per pass: per-tile digit counts laid out digit-major (their exclusive scan is the
-// first output slot of (digit, tile)), a two-level scan, and a scatter that keeps the input order within a digit.
-__global__ void __launch_bounds__(kThreads) build_histogram_kernel(const uint64_t* __restrict__ keys, uint32_t n, int shift,
-                                                                   uint32_t* __restrict__ hist) {
-    __shared__ uint32_t h[kRadix];
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t i = blockIdx.x * kThreads + threadIdx.x;
-    if (i < n) atomicAdd(&h[(uint32_t)(keys[i] >> shift) & (kRadix - 1)], 1u);
-    __syncthreads();
-    hist[(size_t)threadIdx.x * gridDim.x + blockIdx.x] = h[threadIdx.x];
-}
-
-// block-wide exclusive scan of one value per thread; returns the total in *total
-__device__ __forceinline__ uint32_t block_scan(uint32_t v, uint32_t* warp_sum, uint32_t* total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t x = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-        if (lane >= o) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-        uint32_t s = lane < (int)(blockDim.x >> 5) ? warp_sum[lane] : 0u;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, s, o);
-            if (lane >= o) s += y;
-        }
-        warp_sum[lane] = s;
-    }
-    __syncthreads();
-    const uint32_t excl = (warp ? warp_sum[warp - 1] : 0u) + x - v;
-    *total = warp_sum[(blockDim.x >> 5) - 1];
-    return excl;
-}
-
+// The two-level scan of the radix sort's digit counts (tr_device_build.cuh): the sum of every chunk of kScanChunk
+// entries, their one-block scan, then every chunk scanned from its offset.
 __global__ void __launch_bounds__(kScanThreads) build_chunk_sums_kernel(const uint32_t* __restrict__ data, uint32_t len,
                                                                         uint32_t* __restrict__ sums) {
     __shared__ uint32_t warp_sum[32];
@@ -329,23 +230,6 @@ __global__ void __launch_bounds__(kScanThreads) build_scan_kernel(uint32_t* __re
         if (base + k < len) data[base + k] = x;
         x += v[k];
     }
-}
-
-__global__ void __launch_bounds__(kThreads) build_scatter_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ vals,
-                                                                 uint32_t n, int shift, const uint32_t* __restrict__ offset,
-                                                                 uint64_t* __restrict__ keys_out, uint32_t* __restrict__ vals_out) {
-    __shared__ uint32_t digit[kThreads];
-    const uint32_t i = blockIdx.x * kThreads + threadIdx.x;
-    const uint64_t key = i < n ? keys[i] : 0ull;
-    const uint32_t d = i < n ? (uint32_t)(key >> shift) & (kRadix - 1) : 0xffffffffu;
-    digit[threadIdx.x] = d;
-    __syncthreads();
-    if (i >= n) return;
-    uint32_t rank = 0;
-    for (uint32_t j = 0; j < threadIdx.x; j++) rank += digit[j] == d;
-    const uint32_t dst = offset[(size_t)d * gridDim.x + blockIdx.x] + rank;
-    keys_out[dst] = key;
-    vals_out[dst] = vals[i];
 }
 
 // The boundary between sorted positions i and i + 1 of one primitive's segment [lo, hi]: the keys (code, position - lo)
@@ -445,13 +329,13 @@ __device__ __forceinline__ void ploc_merge(uint32_t l, uint32_t r, uint32_t spli
 // One thread per sorted position of the primitives being built (pass 0: every primitive of >= 2 triangles; pass 1: those
 // deeper than `depth_limit`, with threshold 1, i.e. the radix tree).  Apetrei's climb: at a boundary the left child leaves
 // its l, the right child its r; the second to arrive takes the other's and owns the parent.
-__global__ void __launch_bounds__(kThreads) build_hploc_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ vals,
-                                                               uint32_t n, const BuildPrim* __restrict__ bp, const float* __restrict__ pos,
-                                                               const uint32_t* __restrict__ idx, const uint32_t* __restrict__ pdepth,
-                                                               uint32_t depth_limit, int pass, int32_t* pidx, uint32_t* cidx,
-                                                               float4* cbox, int32_t* __restrict__ tparent, Temp* __restrict__ tnode,
-                                                               uint32_t* __restrict__ tprim, uint32_t* counter) {
-    const uint32_t s = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_hploc_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ vals,
+                                                            uint32_t n, const BuildPrim* __restrict__ bp, const float* __restrict__ pos,
+                                                            const uint32_t* __restrict__ idx, const uint32_t* __restrict__ pdepth,
+                                                            uint32_t depth_limit, int pass, int32_t* pidx, uint32_t* cidx,
+                                                            float4* cbox, int32_t* __restrict__ tparent, Temp* __restrict__ tnode,
+                                                            uint32_t* __restrict__ tprim, uint32_t* counter) {
+    const uint32_t s = blockIdx.x * kTile + threadIdx.x;
     if (s >= n) return;
     const uint32_t p = (uint32_t)(__ldg(keys + s) >> 30);
     const BuildPrim b = bp[p];
@@ -487,15 +371,15 @@ __global__ void __launch_bounds__(kThreads) build_hploc_kernel(const uint64_t* _
 // (1 for the parent, plus the inner nodes of the left sibling for a right child) and the triangle offset (the left
 // sibling's triangles).  It writes the node, the triangles of its leaf children, the refit tables and, at a root, the
 // primitive's TlasPrim.  Pass 0 records every primitive's depth (inner nodes on the longest path).
-__global__ void __launch_bounds__(kThreads) build_place_kernel(uint32_t n, const uint32_t* __restrict__ words, const Temp* __restrict__ tnode,
-                                                               const int32_t* __restrict__ tparent, const uint32_t* __restrict__ tprim,
-                                                               const float4* __restrict__ cbox, const BuildPrim* __restrict__ bp,
-                                                               const uint32_t* __restrict__ vals, const float* __restrict__ pos,
-                                                               const uint32_t* __restrict__ idx, int pass, uint32_t* __restrict__ pdepth,
-                                                               AccelNode* __restrict__ nodes, float4* __restrict__ tris,
-                                                               int32_t* __restrict__ parent, uint32_t* __restrict__ arrivals,
-                                                               uint32_t* __restrict__ tri_src, TlasPrim* __restrict__ table) {
-    const uint32_t t = words[W_START] + blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_place_kernel(uint32_t n, const uint32_t* __restrict__ words, const Temp* __restrict__ tnode,
+                                                            const int32_t* __restrict__ tparent, const uint32_t* __restrict__ tprim,
+                                                            const float4* __restrict__ cbox, const BuildPrim* __restrict__ bp,
+                                                            const uint32_t* __restrict__ vals, const float* __restrict__ pos,
+                                                            const uint32_t* __restrict__ idx, int pass, uint32_t* __restrict__ pdepth,
+                                                            AccelNode* __restrict__ nodes, float4* __restrict__ tris,
+                                                            int32_t* __restrict__ parent, uint32_t* __restrict__ arrivals,
+                                                            uint32_t* __restrict__ tri_src, TlasPrim* __restrict__ table) {
+    const uint32_t t = words[W_START] + blockIdx.x * kTile + threadIdx.x;
     if (t >= words[W_COUNTER]) return;
     uint32_t pre = 0, toff = 0, depth = 1;
     uint32_t x = n + t;
@@ -542,25 +426,21 @@ __global__ void __launch_bounds__(kThreads) build_place_kernel(uint32_t n, const
     arrivals[self] = 0u;
     if (pre == 0) {   // the root
         parent[self] = -1;
-        TlasPrim tp;
+        float lo[3], hi[3];
         for (int k = 0; k < 3; k++) {
-            tp.lo[k] = fminf(k0.lo[k], k1.lo[k]);
-            tp.hi[k] = fmaxf(k0.hi[k], k1.hi[k]);
+            lo[k] = fminf(k0.lo[k], k1.lo[k]);
+            hi[k] = fmaxf(k0.hi[k], k1.hi[k]);
         }
-        tp.blas_root = b.node_base;
-        tp.tri_base = b.tri_base;
-        tp.keep = b.keep;
-        tp.pad[0] = tp.pad[1] = tp.pad[2] = 0u;
-        table[prim] = tp;
+        table[prim] = make_tlas_prim(lo, hi, b.node_base, b.tri_base, b.keep);
     }
     if (pass == 0) atomicMax(&pdepth[prim], depth);
 }
 
 // Between the passes: the positions of every primitive deeper than the limit start over, and pass 1's ids follow pass 0's
-__global__ void __launch_bounds__(kThreads) build_reset_kernel(const uint64_t* __restrict__ keys, uint32_t n, const uint32_t* __restrict__ pdepth,
-                                                               uint32_t depth_limit, uint32_t* __restrict__ words, uint32_t* __restrict__ cidx,
-                                                               int32_t* __restrict__ pidx) {
-    const uint32_t s = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kTile) build_reset_kernel(const uint64_t* __restrict__ keys, uint32_t n, const uint32_t* __restrict__ pdepth,
+                                                            uint32_t depth_limit, uint32_t* __restrict__ words, uint32_t* __restrict__ cidx,
+                                                            int32_t* __restrict__ pidx) {
+    const uint32_t s = blockIdx.x * kTile + threadIdx.x;
     if (s == 0) words[W_START] = words[W_COUNTER];
     if (s >= n || pdepth[(uint32_t)(keys[s] >> 30)] <= depth_limit) return;
     cidx[s] = s;
@@ -599,20 +479,19 @@ int32_t accel_build_async(tr_ctx* c) {
         nn += nt > 1 ? nt - 1 : 1;
     }
     if (n >= (1u << 29)) return fail(TR_ERR_UNSUPPORTED, "%s: %llu triangles (at most 2^29 - 1)", who, (unsigned long long)n);
-    const uint32_t nc = n ? (uint32_t)n : 1u, tiles = (nc + kThreads - 1) / kThreads, hist_len = kRadix * tiles,
+    const uint32_t nc = n ? (uint32_t)n : 1u, tiles = (nc + kTile - 1) / kTile, hist_len = kRadix * tiles,
                    chunks = (hist_len + kScanChunk - 1) / kScanChunk;
 
     // scratch: primitives [np], centroid bounds [6 np], depths [np], words [4], keys [2][n] (8 B), values [2][n], digit
     // counts [hist_len], chunk sums [chunks], cluster lists [n], boundary slots [n], cluster boxes [3n] (32 B), parents of
     // clusters [3n], nodes made [2n] (16 B), their primitives [2n]
-    size_t off = 0;
-    auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-    const size_t o_bp = take((size_t)np * sizeof(BuildPrim)), o_counts = take((size_t)np * 8), o_bounds = take((size_t)np * 24), o_depth = take((size_t)np * 4),
-                 o_words = take(16), o_keys = take((size_t)nc * 16), o_vals = take((size_t)nc * 8), o_hist = take((size_t)hist_len * 4),
-                 o_sums = take((size_t)chunks * 4), o_cidx = take((size_t)nc * 4), o_pidx = take((size_t)nc * 4),
-                 o_cbox = take((size_t)nc * 96), o_tparent = take((size_t)nc * 12), o_tnode = take((size_t)nc * 2 * sizeof(Temp)),
-                 o_tprim = take((size_t)nc * 8);
-    TR_TRY(c->accel_build_scratch.ensure(off));
+    ScratchLayout sl;
+    const size_t o_bp = sl.take((size_t)np * sizeof(BuildPrim)), o_counts = sl.take((size_t)np * 8), o_bounds = sl.take((size_t)np * 24),
+                 o_depth = sl.take((size_t)np * 4), o_words = sl.take(16), o_keys = sl.take((size_t)nc * 16), o_vals = sl.take((size_t)nc * 8),
+                 o_hist = sl.take((size_t)hist_len * 4), o_sums = sl.take((size_t)chunks * 4), o_cidx = sl.take((size_t)nc * 4),
+                 o_pidx = sl.take((size_t)nc * 4), o_cbox = sl.take((size_t)nc * 96), o_tparent = sl.take((size_t)nc * 12),
+                 o_tnode = sl.take((size_t)nc * 2 * sizeof(Temp)), o_tprim = sl.take((size_t)nc * 8);
+    TR_TRY(c->accel_build_scratch.ensure(sl.bytes));
     TR_TRY(c->accel_blas.ensure((size_t)nn * sizeof(AccelNode)));
     TR_TRY(c->accel_tris.ensure((size_t)nc * 3 * sizeof(float4)));
     TR_TRY(c->accel_prim_table.ensure((size_t)np * sizeof(TlasPrim)));
@@ -648,28 +527,28 @@ int32_t accel_build_async(tr_ctx* c) {
     const uint32_t nu = (uint32_t)n, init_items = std::max(3 * nc, np);
     cudaStream_t s = c->stream;
 
-    build_counts_kernel<<<(np + kThreads - 1) / kThreads, kThreads, 0, s>>>(prims, np, d_tri_base, d_node_base);
+    build_counts_kernel<<<(np + kTile - 1) / kTile, kTile, 0, s>>>(prims, np, d_tri_base, d_node_base);
     launch_block_scan(d_tri_base, np, s);
     launch_block_scan(d_node_base, np, s);
-    build_init_kernel<<<(init_items + kThreads - 1) / kThreads, kThreads, 0, s>>>(prims, d_tri_base, d_node_base, d_bp, np, nu, pos, idx, bounds, depth, d_words, tparent,
-                                                                               cidx, pidx, nodes, tris, parent, arrivals, tri_src, table);
-    build_bounds_kernel<<<tiles, kThreads, 0, s>>>(d_bp, np, nu, pos, idx, bounds);
-    build_codes_kernel<<<tiles, kThreads, 0, s>>>(d_bp, np, nu, pos, idx, bounds, keys[0], vals[0]);
+    build_init_kernel<<<(init_items + kTile - 1) / kTile, kTile, 0, s>>>(prims, d_tri_base, d_node_base, d_bp, np, nu, pos, idx, bounds, depth, d_words, tparent,
+                                                                         cidx, pidx, nodes, tris, parent, arrivals, tri_src, table);
+    build_bounds_kernel<<<tiles, kTile, 0, s>>>(d_bp, np, nu, pos, idx, bounds);
+    build_codes_kernel<<<tiles, kTile, 0, s>>>(d_bp, np, nu, pos, idx, bounds, keys[0], vals[0]);
     const int passes = (int)radix_passes(np);
     for (int pass = 0; pass < passes; pass++) {
         const int in = pass & 1, shift = pass * kRadixBits;
-        build_histogram_kernel<<<tiles, kThreads, 0, s>>>(keys[in], nu, shift, hist);
+        radix_histogram_kernel<<<tiles, kTile, 0, s>>>(keys[in], nu, shift, hist);
         build_chunk_sums_kernel<<<chunks, kScanThreads, 0, s>>>(hist, hist_len, sums);
         launch_block_scan(sums, chunks, s);
         build_scan_kernel<<<chunks, kScanThreads, 0, s>>>(hist, hist_len, sums);
-        build_scatter_kernel<<<tiles, kThreads, 0, s>>>(keys[in], vals[in], nu, shift, hist, keys[in ^ 1], vals[in ^ 1]);
+        radix_scatter_kernel<<<tiles, kTile, 0, s>>>(keys[in], vals[in], nu, shift, hist, keys[in ^ 1], vals[in ^ 1]);
     }
     const int out = passes & 1;
     for (int pass = 0; pass < 2; pass++) {
-        if (pass == 1) build_reset_kernel<<<tiles, kThreads, 0, s>>>(keys[out], nu, depth, depth_limit, d_words, cidx, pidx);
-        build_hploc_kernel<<<tiles, kThreads, 0, s>>>(keys[out], vals[out], nu, d_bp, pos, idx, depth, depth_limit, pass, pidx, cidx,
+        if (pass == 1) build_reset_kernel<<<tiles, kTile, 0, s>>>(keys[out], nu, depth, depth_limit, d_words, cidx, pidx);
+        build_hploc_kernel<<<tiles, kTile, 0, s>>>(keys[out], vals[out], nu, d_bp, pos, idx, depth, depth_limit, pass, pidx, cidx,
                                                       cbox, tparent, tnode, tprim, d_words + W_COUNTER);
-        build_place_kernel<<<tiles, kThreads, 0, s>>>(nu, d_words, tnode, tparent, tprim, cbox, d_bp, vals[out], pos, idx, pass, depth,
+        build_place_kernel<<<tiles, kTile, 0, s>>>(nu, d_words, tnode, tparent, tprim, cbox, d_bp, vals[out], pos, idx, pass, depth,
                                                       nodes, tris, parent, arrivals, tri_src, table);
     }
     count_launches(async_blas_launches(np));

@@ -12,19 +12,14 @@
 //
 // Launches per update (kAsyncTlasLaunches, fixed whatever the instance count): count, scan, records, bounds, codes,
 // 4 x (histogram, scan, scatter), hierarchy, boxes = 19.
-#include "tr_device_accel.cuh"
+#include "tr_device_build.cuh"
 #include "tr_internal.h"
 
 using namespace trd;
 
 namespace {
 
-constexpr int kTile = 256;             // items per block of the count / sort kernels
-constexpr int kRadixBits = 8;
-constexpr int kRadix = 1 << kRadixBits;
 constexpr int kRadixPasses = 4;        // 30-bit codes in 8-bit digits
-constexpr int kScanThreads = 1024;
-static_assert(kTile == kRadix, "the histogram kernel keeps one digit per thread");
 
 __device__ __forceinline__ uint32_t keep_of(const tr_instance* inst, const TlasPrim* prims, uint32_t i) {
     return prims[inst[i].primitive_id].keep;
@@ -39,39 +34,16 @@ __global__ void __launch_bounds__(kTile) tlas_count_kernel(const tr_instance* __
     if (threadIdx.x == 0) block_count[blockIdx.x] = (uint32_t)total;
 }
 
-// in-place exclusive prefix sum of data[0, len) by one block
+// in-place exclusive prefix sum of data[0, len) by one block, kScanThreads entries at a time
 __global__ void __launch_bounds__(kScanThreads) tlas_scan_kernel(uint32_t* __restrict__ data, uint32_t len) {
-    __shared__ uint32_t warp_sum[kScanThreads / 32];
-    __shared__ uint32_t carry;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
+    __shared__ uint32_t warp_sum[32];
+    uint32_t carry = 0;   // the sum of the entries before base
     for (uint32_t base = 0; base < len; base += kScanThreads) {
         const uint32_t i = base + threadIdx.x;
-        const uint32_t v = i < len ? data[i] : 0u;
-        uint32_t x = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
-        }
-        if (lane == 31) warp_sum[warp] = x;
-        __syncthreads();
-        if (warp == 0) {
-            uint32_t s = warp_sum[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t y = __shfl_up_sync(0xffffffffu, s, o);
-                if (lane >= o) s += y;
-            }
-            warp_sum[lane] = s;   // inclusive over warps
-        }
-        __syncthreads();
-        const uint32_t c = carry;
-        const uint32_t excl = c + (warp ? warp_sum[warp - 1] : 0u) + x - v;
+        uint32_t total;
+        const uint32_t excl = carry + block_scan(i < len ? data[i] : 0u, warp_sum, &total);
         if (i < len) data[i] = excl;
-        __syncthreads();
-        if (threadIdx.x == kScanThreads - 1) carry = excl + v;
+        carry += total;
         __syncthreads();
     }
 }
@@ -165,36 +137,6 @@ __global__ void __launch_bounds__(kTile) tlas_codes_kernel(const AccelInstance* 
     vals[i] = i;
 }
 
-// LSD radix sort, one digit per pass: per-tile digit counts laid out digit-major, so their exclusive scan is the
-// first output slot of (digit, tile); the scatter keeps the input order within a digit (stable).
-__global__ void __launch_bounds__(kTile) tlas_histogram_kernel(const uint32_t* __restrict__ keys, uint32_t m, int shift,
-                                                               uint32_t* __restrict__ hist) {
-    __shared__ uint32_t h[kRadix];
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t i = blockIdx.x * kTile + threadIdx.x;
-    if (i < m) atomicAdd(&h[(keys[i] >> shift) & (kRadix - 1)], 1u);
-    __syncthreads();
-    hist[(size_t)threadIdx.x * gridDim.x + blockIdx.x] = h[threadIdx.x];
-}
-
-__global__ void __launch_bounds__(kTile) tlas_scatter_kernel(const uint32_t* __restrict__ keys, const uint32_t* __restrict__ vals, uint32_t m,
-                                                             int shift, const uint32_t* __restrict__ offset, uint32_t* __restrict__ keys_out,
-                                                             uint32_t* __restrict__ vals_out) {
-    __shared__ uint32_t digit[kTile];
-    const uint32_t i = blockIdx.x * kTile + threadIdx.x;
-    const uint32_t key = i < m ? keys[i] : 0u;
-    const uint32_t d = i < m ? (key >> shift) & (kRadix - 1) : 0xffffffffu;
-    digit[threadIdx.x] = d;
-    __syncthreads();
-    if (i >= m) return;
-    uint32_t rank = 0;
-    for (uint32_t j = 0; j < threadIdx.x; j++) rank += digit[j] == d;
-    const uint32_t dst = offset[(size_t)d * gridDim.x + blockIdx.x] + rank;
-    keys_out[dst] = key;
-    vals_out[dst] = vals[i];
-}
-
 // Karras 2012: the common-prefix length of the keys (code, position); positions break ties, so all keys differ.
 __device__ __forceinline__ int delta(const uint32_t* codes, int m, int i, int j) {
     if (j < 0 || j >= m) return -1;
@@ -236,36 +178,26 @@ __global__ void __launch_bounds__(kTile) tlas_hierarchy_kernel(const uint32_t* _
     arrivals[i] = 0;
 }
 
-// child `side`'s box: floats [6 side, 6 side + 6) of the node, lo then hi (the AccelNode layout)
-__device__ __forceinline__ void store_box(AccelNode* n, int side, const float* lo, const float* hi) {
-    float* b = reinterpret_cast<float*>(n) + side * 6;
-    b[0] = lo[0]; b[1] = lo[1]; b[2] = lo[2];
-    b[3] = hi[0]; b[4] = hi[1]; b[5] = hi[2];
-}
-
-// One thread per leaf (sorted position): its instance record in leaf order, then up the tree.  The first arrival at a
-// node stores its box and stops; the second stores its own, unions both and goes on.  fminf / fmaxf are exact, so the
-// boxes do not depend on the arrival order.
+// One thread per leaf (sorted position): its instance record in leaf order, then up the tree (arrive): the first arrival
+// at a node stops, the second goes on with the node's box.
 __global__ void __launch_bounds__(kTile) tlas_boxes_kernel(const AccelInstance* __restrict__ rec, const uint32_t* __restrict__ order, uint32_t m_,
                                                            AccelNode* nodes, AccelInstance* __restrict__ inst, const int32_t* __restrict__ parent,
                                                            uint32_t* arrivals) {
     const int m = (int)m_;
     const int i = blockIdx.x * kTile + threadIdx.x;
-    const float inf = __int_as_float(0x7f800000);
-    const float elo[3] = {inf, inf, inf}, ehi[3] = {-inf, -inf, -inf};
-    if (m < 2) {  // build_tree (k_accel.cu): the empty root, or one leaf wrapped in a root whose second box is empty
+    if (m < 2) {  // the special roots of build_tree (k_accel.cu)
         if (i != 0) return;
-        AccelNode* root = nodes;
-        if (m == 0) {
-            store_box(root, 0, elo, ehi);
-        } else {
+        float lo[3], hi[3];
+        empty_box(lo, hi);
+        if (m == 1) {
             const AccelInstance r = rec[order[0]];
             inst[0] = r;
-            store_box(root, 0, r.lo, r.hi);
+            for (int k = 0; k < 3; k++) {
+                lo[k] = r.lo[k];
+                hi[k] = r.hi[k];
+            }
         }
-        store_box(root, 1, elo, ehi);
-        root->c0 = root->c1 = ~0;
-        root->pad[0] = root->pad[1] = 0;
+        nodes[0] = special_root(lo, hi);
         return;
     }
     if (i >= m) return;
@@ -275,17 +207,7 @@ __global__ void __launch_bounds__(kTile) tlas_boxes_kernel(const AccelInstance* 
     int32_t child = (int32_t)~(uint32_t)i;
     int node = parent[(m - 1) + i];
     while (true) {
-        AccelNode* n = nodes + node;
-        const int side = n->c0 == child ? 0 : 1;
-        store_box(n, side, lo, hi);
-        __threadfence();
-        if (atomicAdd(&arrivals[node], 1u) == 0u) return;  // the sibling's box is not there yet: it goes on from here
-        __threadfence();
-        const float* o = reinterpret_cast<const float*>(n) + (side ^ 1) * 6;
-        for (int k = 0; k < 3; k++) {
-            lo[k] = fminf(lo[k], __ldcg(o + k));
-            hi[k] = fmaxf(hi[k], __ldcg(o + 3 + k));
-        }
+        if (!arrive(nodes, arrivals, node, nodes[node].c0 == child ? 0 : 1, lo, hi)) return;
         if (node == 0) return;
         child = node;
         node = parent[node];
@@ -316,10 +238,11 @@ int32_t accel_build_tlas_async(tr_ctx* c) {
     // scratch: records [m], keys [2][m], values [2][m], parents [2m], arrivals [m], digit counts [kRadix][tiles of m],
     // kept counts [tiles of n], centroid bounds [8]
     const uint32_t mc = m ? m : 1u, tiles_m = (mc + kTile - 1) / kTile, tiles_n = (n + kTile - 1) / kTile ? (n + kTile - 1) / kTile : 1u;
-    const size_t off_rec = 0, off_keys = off_rec + (size_t)mc * sizeof(AccelInstance), off_vals = off_keys + (size_t)mc * 8,
-                 off_parent = off_vals + (size_t)mc * 8, off_arr = off_parent + (size_t)mc * 8, off_hist = off_arr + (size_t)mc * 4,
-                 off_cnt = off_hist + (size_t)kRadix * tiles_m * 4, off_bounds = off_cnt + (size_t)tiles_n * 4, total = off_bounds + 32;
-    TR_TRY(c->accel_scratch.ensure(total));
+    ScratchLayout sl;
+    const size_t off_rec = sl.take((size_t)mc * sizeof(AccelInstance)), off_keys = sl.take((size_t)mc * 8), off_vals = sl.take((size_t)mc * 8),
+                 off_parent = sl.take((size_t)mc * 8), off_arr = sl.take((size_t)mc * 4), off_hist = sl.take((size_t)kRadix * tiles_m * 4),
+                 off_cnt = sl.take((size_t)tiles_n * 4), off_bounds = sl.take(32);
+    TR_TRY(c->accel_scratch.ensure(sl.bytes));
     TR_TRY(c->accel_tlas.ensure((size_t)(m >= 2 ? m - 1 : 1) * sizeof(AccelNode)));
     TR_TRY(c->accel_inst.ensure((size_t)mc * sizeof(AccelInstance)));
     char* base = c->accel_scratch.as<char>();
@@ -343,9 +266,9 @@ int32_t accel_build_tlas_async(tr_ctx* c) {
     tlas_codes_kernel<<<tiles_m, kTile, 0, s>>>(rec, m, bounds, keys[0], vals[0]);
     for (int pass = 0; pass < kRadixPasses; pass++) {  // an even number of passes: the sorted keys end in keys[0]
         const int in = pass & 1, shift = pass * kRadixBits;
-        tlas_histogram_kernel<<<tiles_m, kTile, 0, s>>>(keys[in], m, shift, hist);
+        radix_histogram_kernel<<<tiles_m, kTile, 0, s>>>(keys[in], m, shift, hist);
         tlas_scan_kernel<<<1, kScanThreads, 0, s>>>(hist, kRadix * tiles_m);
-        tlas_scatter_kernel<<<tiles_m, kTile, 0, s>>>(keys[in], vals[in], m, shift, hist, keys[in ^ 1], vals[in ^ 1]);
+        radix_scatter_kernel<<<tiles_m, kTile, 0, s>>>(keys[in], vals[in], m, shift, hist, keys[in ^ 1], vals[in ^ 1]);
     }
     tlas_hierarchy_kernel<<<tiles_m, kTile, 0, s>>>(keys[0], m, nodes, parent, arrivals);
     tlas_boxes_kernel<<<tiles_m, kTile, 0, s>>>(rec, vals[0], m, nodes, c->accel_inst.as<AccelInstance>(), parent, arrivals);

@@ -10,10 +10,10 @@
 //
 // Refit: the mesh keeps its topology, so every tree of tr_build_acceleration_structures keeps its nodes and leaf ranges; only
 // the triangles (gathered again from the positions in leaf order) and the boxes change.  The boxes are recomputed
-// bottom-up with per-node arrival counters, as tlas_boxes_kernel (k_accel_device.cu) does; fminf / fmaxf are exact, so
-// every inner box is the exact union of its subtree (the sign of a zero may depend on the arrival order; the slab test
-// cannot see it).  The depth is the build's, below kAccelStack.  Two launches whatever the mesh size: gather, boxes.
-#include "tr_device_accel.cuh"
+// bottom-up with per-node arrival counters (arrive, tr_device_build.cuh); fminf / fmaxf are exact, so every inner box is
+// the exact union of its subtree (the sign of a zero may depend on the arrival order; the slab test cannot see it).  The
+// depth is the build's, below kAccelStack.  Two launches whatever the mesh size: gather, boxes.
+#include "tr_device_build.cuh"
 #include "tr_internal.h"
 
 using namespace trd;
@@ -37,14 +37,9 @@ __global__ void __launch_bounds__(kChunkWarps * 32) chunk_spheres_kernel(const f
     const uint32_t chunk = blockIdx.x * kChunkWarps + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (chunk >= n_chunks) return;
-    uint32_t lo_p = 0, hi_p = n_prims;   // base[lo_p] <= chunk < base[hi_p]: the chunk's primitive is the last such lo_p
-    while (hi_p - lo_p > 1) {
-        const uint32_t mid = (lo_p + hi_p) >> 1;
-        if (__ldg(base + mid) <= chunk) lo_p = mid;
-        else hi_p = mid;
-    }
-    const tr_primitive_info pr = prims[lo_p];
-    const uint32_t tris = pr.index_count / 3u, t0 = (chunk - __ldg(base + lo_p)) * TR_CHUNK_TRIS;
+    const uint32_t p = last_at_most(n_prims, chunk, [&](uint32_t q) { return __ldg(base + q); });   // the chunk's primitive
+    const tr_primitive_info pr = prims[p];
+    const uint32_t tris = pr.index_count / 3u, t0 = (chunk - __ldg(base + p)) * TR_CHUNK_TRIS;
     const uint32_t t1 = min(t0 + TR_CHUNK_TRIS, tris);
     const uint32_t i0 = pr.first_index + t0 * 3u, i1 = pr.first_index + t1 * 3u;
     const uint32_t my0 = min(i0 + lane * 6u, i1), my1 = min(my0 + 6u, i1);
@@ -109,40 +104,17 @@ __global__ void __launch_bounds__(kRefitThreads) blas_gather_kernel(const float*
     const uint32_t i = blockIdx.x * kRefitThreads + threadIdx.x;
     if (i < n_nodes) arrivals[i] = 0u;
     if (i >= n_tris) return;
-    const uint32_t s = tri_src[i];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        const uint32_t v = __ldg(idx + s + k);
-        tris[(size_t)i * 3 + k] = make_float4(__ldg(pos + (size_t)v * 3), __ldg(pos + (size_t)v * 3 + 1), __ldg(pos + (size_t)v * 3 + 2), 0.0f);
-    }
+    const Tri t = load_tri(pos, idx, tri_src[i]);
+    for (int k = 0; k < 3; k++) tris[(size_t)i * 3 + k] = t.v[k];
 }
 
-// child `side`'s box: floats [6 side, 6 side + 6) of the node, lo then hi (the AccelNode layout)
-__device__ __forceinline__ void put_box(AccelNode* n, int side, const float* lo, const float* hi) {
-    float* b = reinterpret_cast<float*>(n) + side * 6;
-    b[0] = lo[0]; b[1] = lo[1]; b[2] = lo[2];
-    b[3] = hi[0]; b[4] = hi[1]; b[5] = hi[2];
-}
-
-// the box of a leaf's triangles, folded as the host builder folds it (box_grow per vertex, box_union per triangle)
+// the box of a leaf's triangles (up to 4: the refit also runs on trees of the host builder)
 __device__ __forceinline__ void leaf_box(const float4* __restrict__ tris, uint32_t tri_base, int32_t ref, float* lo, float* hi) {
-    const float inf = __int_as_float(0x7f800000);
     const uint32_t code = ~(uint32_t)ref, first = code & 0x0fffffffu, count = (code >> 28) + 1u;
-    lo[0] = lo[1] = lo[2] = inf;
-    hi[0] = hi[1] = hi[2] = -inf;
+    empty_box(lo, hi);
     for (uint32_t j = 0; j < count; j++) {
         const float4* t = tris + (size_t)(tri_base + first + j) * 3;
-        float tlo[3] = {inf, inf, inf}, thi[3] = {-inf, -inf, -inf};
-        for (int k = 0; k < 3; k++) {
-            const float4 p = t[k];
-            tlo[0] = fminf(tlo[0], p.x); thi[0] = fmaxf(thi[0], p.x);
-            tlo[1] = fminf(tlo[1], p.y); thi[1] = fmaxf(thi[1], p.y);
-            tlo[2] = fminf(tlo[2], p.z); thi[2] = fmaxf(thi[2], p.z);
-        }
-        for (int k = 0; k < 3; k++) {
-            lo[k] = fminf(fminf(lo[k], tlo[k]), thi[k]);
-            hi[k] = fmaxf(fmaxf(hi[k], tlo[k]), thi[k]);
-        }
+        fold_tri(Tri{{t[0], t[1], t[2]}}, lo, hi);
     }
 }
 
@@ -156,12 +128,8 @@ __global__ void __launch_bounds__(kRefitThreads) blas_boxes_kernel(AccelNode* no
                                                                    uint32_t n_prims) {
     const uint32_t i = blockIdx.x * kRefitThreads + threadIdx.x;
     if (i >= n_nodes) return;
-    uint32_t p = 0, hi_p = n_prims;   // the node's primitive: the last whose root is <= i (the trees lie in primitive order)
-    while (hi_p - p > 1) {
-        const uint32_t mid = (p + hi_p) >> 1;
-        if (table[mid].blas_root <= i) p = mid;
-        else hi_p = mid;
-    }
+    // the node's primitive: the last whose root is <= i (the trees lie in primitive order)
+    const uint32_t p = last_at_most(n_prims, i, [&](uint32_t q) { return table[q].blas_root; });
     const uint32_t tri_base = table[p].tri_base;
     AccelNode* n = nodes + i;
     const int32_t c0 = n->c0, c1 = n->c1;
@@ -169,33 +137,23 @@ __global__ void __launch_bounds__(kRefitThreads) blas_boxes_kernel(AccelNode* no
     if (c0 == c1) {   // the special roots of build_tree (k_accel.cu): the empty tree, or one leaf wrapped in a root
         if (prims[p].index_count / 3u == 0u) return;   // empty: both boxes stay empty, and so does the primitive's box
         leaf_box(tris, tri_base, c0, lo, hi);
-        put_box(n, 0, lo, hi);                          // the second box stays empty
+        store_box(n, 0, lo, hi);                        // the second box stays empty
+    } else if (c0 < 0 && c1 < 0) {   // two leaf children: the node is complete
+        float lo1[3], hi1[3];
+        leaf_box(tris, tri_base, c0, lo, hi);
+        store_box(n, 0, lo, hi);
+        leaf_box(tris, tri_base, c1, lo1, hi1);
+        store_box(n, 1, lo1, hi1);
+        for (int k = 0; k < 3; k++) {
+            lo[k] = fminf(lo[k], lo1[k]);
+            hi[k] = fmaxf(hi[k], hi1[k]);
+        }
+    } else if (c0 < 0 || c1 < 0) {   // one leaf child: its box arrives at this node as the inner child's will
+        const int side = c0 < 0 ? 0 : 1;
+        leaf_box(tris, tri_base, side ? c1 : c0, lo, hi);
+        if (!arrive(nodes, arrivals, (int)i, side, lo, hi)) return;
     } else {
-        int leaves = 0;
-        for (int side = 0; side < 2; side++) {
-            const int32_t c = side ? c1 : c0;
-            if (c >= 0) continue;
-            float llo[3], lhi[3];
-            leaf_box(tris, tri_base, c, llo, lhi);
-            put_box(n, side, llo, lhi);
-            for (int k = 0; k < 3; k++) {
-                lo[k] = leaves ? fminf(lo[k], llo[k]) : llo[k];
-                hi[k] = leaves ? fmaxf(hi[k], lhi[k]) : lhi[k];
-            }
-            leaves++;
-        }
-        if (leaves == 0) return;   // both children inner: their threads arrive here
-        if (leaves == 1) {
-            __threadfence();
-            if (atomicAdd(&arrivals[i], 1u) == 0u) return;   // the inner child's box is not there yet: it goes on from here
-            __threadfence();
-            const int other = c0 >= 0 ? 0 : 1;
-            const float* o = reinterpret_cast<const float*>(n) + other * 6;
-            for (int k = 0; k < 3; k++) {
-                lo[k] = fminf(lo[k], __ldcg(o + k));
-                hi[k] = fmaxf(hi[k], __ldcg(o + 3 + k));
-            }
-        }
+        return;   // both children inner: their threads arrive here
     }
     int32_t node = (int32_t)i;
     while (true) {   // `node` is complete and (lo, hi) is its box
@@ -208,17 +166,7 @@ __global__ void __launch_bounds__(kRefitThreads) blas_boxes_kernel(AccelNode* no
             }
             return;
         }
-        AccelNode* u = nodes + up;
-        const int side = u->c0 == node ? 0 : 1;
-        put_box(u, side, lo, hi);
-        __threadfence();
-        if (atomicAdd(&arrivals[up], 1u) == 0u) return;
-        __threadfence();
-        const float* o = reinterpret_cast<const float*>(u) + (side ^ 1) * 6;
-        for (int k = 0; k < 3; k++) {
-            lo[k] = fminf(lo[k], __ldcg(o + k));
-            hi[k] = fmaxf(hi[k], __ldcg(o + 3 + k));
-        }
+        if (!arrive(nodes, arrivals, up, nodes[up].c0 == node ? 0 : 1, lo, hi)) return;
         node = up;
     }
 }

@@ -67,25 +67,6 @@ constexpr float kSunTMax = 10000.0f;       // lighting.rs:31, 163
 //   (tests/test_gpu_accel_build.py checks it, with the fallback forced on ordinary meshes and on pathological ones).
 constexpr int kAccelStack = 64;
 
-// Morton codes of both device builders (k_accel_device.cu, k_accel_build.cu)
-TRD uint32_t spread10(uint32_t x) {  // 10 bits -> every third bit of 30
-    x &= 0x3ffu;
-    x = (x | (x << 16)) & 0x030000ffu;
-    x = (x | (x << 8)) & 0x0300f00fu;
-    x = (x | (x << 4)) & 0x030c30c3u;
-    x = (x | (x << 2)) & 0x09249249u;
-    return x;
-}
-
-// 10 bits per axis.  A zero, infinite or NaN extent, or a NaN centroid, quantises to 0 instead of an undefined
-// conversion: the codes only shape the trees, never the result.
-TRD uint32_t quantise(float c, float lo, float ext) {
-    const float t = (ext > 0.0f && ext <= 3.4e38f) ? (c - lo) / ext * 1024.0f : 0.0f;
-    if (!(t >= 0.0f)) return 0u;
-    if (t >= 1023.0f) return 1023u;
-    return (uint32_t)t;
-}
-
 struct AccelRay {
     float o[3], d[3], inv[3];
     float t_min, t_max;

@@ -48,6 +48,17 @@ struct DevBuf {
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
+// The pieces of one scratch buffer: take() returns each piece's offset, 256-byte aligned, and `bytes` is what the buffer
+// must hold (ensure) before the offsets are added to its base.
+struct ScratchLayout {
+    size_t bytes = 0;
+    size_t take(size_t n) {
+        const size_t o = bytes;
+        bytes += (n + 255) & ~(size_t)255;
+        return o;
+    }
+};
+
 struct GLayer {
     DevBuf depth, normal, uv, material_id, scale, position, duv, ddepth;
     bool has_position = false;
