@@ -723,7 +723,7 @@ def test_random_gbuffer_stress(oracle, ggx_lut):
 
 
 def test_more_lights_than_the_shared_table(oracle, ggx_lut):
-    """1 200 lights: more than the 1 024-entry shared-memory light table of the shading kernels, so the launch takes the
+    """1 200 lights: more than the 768-entry shared-memory light table of the shading kernels, so the launch takes the
     global-memory light path (the huge far clusters overflow their 128-entry lists, which both sides clamp alike)."""
     w, h = 320, 180
     cam = scenes.Camera(w, h, (0.0, 3.0, 6.0), 0.0, -15.0)
