@@ -395,6 +395,24 @@ TR_API int32_t tr_set_ggx_lut(tr_ctx* ctx, const uint8_t* rgba8, uint32_t width,
 #define TR_MAX_IMAGES 193u
 TR_API int32_t tr_set_texture(tr_ctx* ctx, uint32_t index, const uint8_t* const* levels, uint32_t n_levels,
                               uint32_t width, uint32_t height, int32_t srgb);
+/* load_texture_from_gltf + ImageManager::push_image (src/model_loading.rs:340-379): level 0 only, as RGBA8 (sRGB when
+ * srgb != 0); levels 1 .. n_levels-1 are built on the device in stream order. n_levels = 0 means the full chain
+ * floor(log2(min(w, h))) + 1.
+ * Each level is the 2x2 box of the one above it (odd sizes cropped to even), filtered in linear light in float64 and rounded
+ * back to RGBA8 bytes, as the Python ingest's scenes.make_mips does: the image samples bit for bit as tr_set_texture fed
+ * that chain.  Stream-ordered on the context stream: the frame enqueued before the call samples the old image, the next one
+ * the new.  The source follows the upload rule (pageable: copied during the call; page-locked: read in stream order).  With
+ * a page-locked source the call does not wait for the device, except when `index` is bound and its allocation must grow
+ * (as tr_set_texture, it then waits for the frame in flight); binding an index for the first time never waits.  The
+ * image's allocation keeps the RGBA8 bytes of its levels beside the decoded texels (+25 %).  tr_set_texture and this call
+ * may rebind the same index in any order.  Errors: those of tr_set_texture (index >= TR_MAX_IMAGES, a null pointer, a zero
+ * size, n_levels > 16), and n_levels greater than the full chain: TR_ERR_INVALID_ARG; a rejected call changes nothing.
+ * Each call launches n_levels kernels (the full chain's count for 0) (tr_launch_count). */
+TR_API int32_t tr_set_texture_async(tr_ctx* ctx, uint32_t index, const uint8_t* rgba8, uint32_t width, uint32_t height,
+                                    int32_t srgb, uint32_t n_levels);
+/* Parity hook: level `level` of bound image `index` as the samplers read it (RGBA32F, max(1, w >> level) x
+ * max(1, h >> level) texels, into *w / *h; null array: size only); blocking.  Not bound: TR_ERR_STATE. */
+TR_API int32_t tr_read_texture_level(tr_ctx* ctx, uint32_t index, uint32_t level, float* rgba32f, uint32_t* w, uint32_t* h);
 /* vertex bindings 0..2 + index buffer (pipelines.rs:291-307, main.rs:2516-2557). */
 TR_API int32_t tr_set_mesh(tr_ctx* ctx, const float* positions, const float* normals, const float* uvs,
                            uint32_t n_vertices, const uint32_t* indices, uint32_t n_indices);

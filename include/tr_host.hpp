@@ -372,6 +372,13 @@ public:
     void set_materials(const std::vector<tr_material_info>& v) { TR_HOST_CHECK(tr_set_materials(ctx_, v.data(), (uint32_t)v.size())); }
     void set_lights(const std::vector<tr_light>& v) { TR_HOST_CHECK(tr_set_lights(ctx_, v.empty() ? nullptr : v.data(), (uint32_t)v.size())); }
     void set_uniforms(const tr_uniforms& u) { TR_HOST_CHECK(tr_set_uniforms(ctx_, &u)); }
+    // load_texture_from_gltf + ImageManager::push_image, src/model_loading.rs:340-379: level 0 of image `index` (RGBA8,
+    // tightly packed), the mip chain built on the device in stream order (n_levels = 0: the full chain).  `rgba8` is read
+    // during the call unless it is page-locked; then it must stay alive and unchanged until the stream has passed the call.
+    void set_texture_async(uint32_t index, const std::vector<uint8_t>& rgba8, uint32_t w, uint32_t h, bool srgb, uint32_t n_levels = 0) {
+        if (rgba8.size() != (size_t)w * h * 4) throw Error(TR_ERR_INVALID_ARG, "Renderer::set_texture_async: size");
+        TR_HOST_CHECK(tr_set_texture_async(ctx_, index, rgba8.data(), w, h, srgb ? 1 : 0, n_levels));
+    }
     void set_ggx_lut(const std::vector<uint8_t>& rgba8, uint32_t w, uint32_t h) {
         if (rgba8.size() != (size_t)w * h * 4) throw Error(TR_ERR_INVALID_ARG, "Renderer::set_ggx_lut: size");
         TR_HOST_CHECK(tr_set_ggx_lut(ctx_, rgba8.data(), w, h));

@@ -509,6 +509,7 @@ int32_t tr_destroy(tr_ctx* c) {
     for (DevBuf* b : bufs) b->release();
     for (DevBuf& b : c->tex_data) b.release();
     c->tex_table.release();
+    c->tex_tables.release();
     for (int l = 0; l < 2; l++) {
         GLayer& g = c->layer[l];
         g.depth.release(); g.normal.release(); g.uv.release(); g.material_id.release(); g.scale.release(); g.position.release();
@@ -712,10 +713,26 @@ int32_t tr_set_ggx_lut(tr_ctx* c, const uint8_t* rgba8, uint32_t width, uint32_t
     return TR_OK;
 }
 
-// sRGB8 -> linear, evaluated in double and rounded once (R8G8B8A8_SRGB decode of the sampled image)
-static float srgb8_to_linear(uint8_t v) {
-    const double x = (double)v / 255.0;
-    return (float)(x <= 0.04045 ? x / 12.92 : pow((x + 0.055) / 1.055, 2.4));
+// Level texel offsets of an image (TexDesc.off) and its texel count over those levels.
+static size_t texture_layout(trd::TexDesc* d, uint32_t width, uint32_t height, uint32_t n_levels, int32_t srgb) {
+    d->w = width;
+    d->h = height;
+    d->levels = n_levels;
+    d->srgb = srgb ? 1u : 0u;
+    size_t total = 0;
+    for (uint32_t l = 0; l < n_levels; l++) {
+        d->off[l] = (uint32_t)total;
+        const uint32_t w = width >> l ? width >> l : 1u, h = height >> l ? height >> l : 1u;
+        total += (size_t)w * h;
+    }
+    return total;
+}
+
+static void bind_texture(tr_ctx* c, uint32_t index, trd::TexDesc d) {
+    d.base = c->tex_data[index].as<float4>();
+    c->h_tex[index] = d;
+    if (index + 1 > c->n_textures) c->n_textures = index + 1;
+    c->tex_table_dirty = true;
 }
 
 int32_t tr_set_texture(tr_ctx* c, uint32_t index, const uint8_t* const* levels, uint32_t n_levels, uint32_t width, uint32_t height,
@@ -723,23 +740,13 @@ int32_t tr_set_texture(tr_ctx* c, uint32_t index, const uint8_t* const* levels, 
     TR_CHECK_CTX(c);
     if (index >= TR_MAX_IMAGES) return fail(TR_ERR_INVALID_ARG, "tr_set_texture: image %u of at most %u", index, TR_MAX_IMAGES);
     if (!levels || n_levels == 0 || n_levels > 16 || !width || !height) return fail(TR_ERR_INVALID_ARG, "tr_set_texture: bad arguments");
-    float table[256], unorm[256];
-    for (int v = 0; v < 256; v++) {
-        table[v] = srgb ? srgb8_to_linear((uint8_t)v) : (float)v / 255.0f;
-        unorm[v] = (float)v / 255.0f;  // alpha stays linear in the sRGB formats
-    }
+    const TexTables& tab = texture_tables();
+    const float* table = tab.dec32[srgb ? 0 : 1];   // sRGB8 -> linear, evaluated in double and rounded once
+    const float* unorm = tab.dec32[1];              // alpha stays linear in the sRGB formats
     trd::TexDesc d{};
-    d.w = width;
-    d.h = height;
-    d.levels = n_levels;
-    d.srgb = srgb ? 1u : 0u;
-    size_t total = 0;
-    for (uint32_t l = 0; l < n_levels; l++) {
+    for (uint32_t l = 0; l < n_levels; l++)
         if (!levels[l]) return fail(TR_ERR_INVALID_ARG, "tr_set_texture: level %u is null", l);
-        d.off[l] = (uint32_t)total;
-        const uint32_t w = width >> l ? width >> l : 1u, h = height >> l ? height >> l : 1u;
-        total += (size_t)w * h;
-    }
+    const size_t total = texture_layout(&d, width, height, n_levels, srgb);
     std::vector<float> texels(total * 4);
     for (uint32_t l = 0; l < n_levels; l++) {
         const uint32_t w = width >> l ? width >> l : 1u, h = height >> l ? height >> l : 1u;
@@ -755,10 +762,42 @@ int32_t tr_set_texture(tr_ctx* c, uint32_t index, const uint8_t* const* levels, 
     TR_CUDA(cudaStreamSynchronize(c->stream));  // a frame in flight may still sample the old image
     TR_TRY(c->tex_data[index].ensure(total * 16));
     TR_CUDA(cudaMemcpy(c->tex_data[index].p, texels.data(), total * 16, cudaMemcpyHostToDevice));
-    d.base = c->tex_data[index].as<float4>();
-    c->h_tex[index] = d;
-    if (index + 1 > c->n_textures) c->n_textures = index + 1;
-    c->tex_table_dirty = true;
+    bind_texture(c, index, d);
+    return TR_OK;
+}
+
+// Level 0 as RGBA8 into the byte chain behind the image's texels, then the device builds the store and the rest of the chain
+// (k_textures.cu), all in stream order.  The allocation is the image's own: a rebind that fits it reuses it without a wait,
+// since every frame that may still read the old texels was enqueued before the kernels that overwrite them.
+int32_t tr_set_texture_async(tr_ctx* c, uint32_t index, const uint8_t* rgba8, uint32_t width, uint32_t height, int32_t srgb,
+                             uint32_t n_levels) {
+    TR_CHECK_CTX(c);
+    if (index >= TR_MAX_IMAGES) return fail(TR_ERR_INVALID_ARG, "tr_set_texture_async: image %u of at most %u", index, TR_MAX_IMAGES);
+    if (!rgba8 || !width || !height || n_levels > 16) return fail(TR_ERR_INVALID_ARG, "tr_set_texture_async: bad arguments");
+    const uint32_t full = mip_levels_for_size(width, height);
+    if (n_levels > full || (n_levels == 0 && full > 16))
+        return fail(TR_ERR_INVALID_ARG, "tr_set_texture_async: %u levels for a %ux%u image (full chain %u, at most 16)",
+                    n_levels ? n_levels : full, width, height, full);
+    trd::TexDesc d{};
+    const size_t total = texture_layout(&d, width, height, n_levels ? n_levels : full, srgb);
+    if (total > 0xffffffffull) return fail(TR_ERR_UNSUPPORTED, "tr_set_texture_async: more than 2^32 texels");
+    const size_t need = total * 20;   // RGBA32F texels, then the RGBA8 bytes of every level
+    DevBuf& buf = c->tex_data[index];
+    if (buf.p && buf.bytes < need) TR_CUDA(cudaStreamSynchronize(c->stream));   // a frame in flight may still sample the old image
+    if (!c->tex_tables.p) {
+        TR_TRY(c->tex_tables.ensure(sizeof(TexTables)));
+        TR_CUDA(cudaMemcpyAsync(c->tex_tables.p, &texture_tables(), sizeof(TexTables), cudaMemcpyHostToDevice, c->stream));
+    }
+    if (!buf.p) {   // stream-ordered: unlike cudaMalloc, it never waits for the device to reclaim freed memory
+        TR_CUDA(cudaMallocAsync(&buf.p, need, c->stream));
+        buf.bytes = need;
+    }
+    TR_TRY(buf.ensure(need));
+    uint8_t* chain = buf.as<uint8_t>() + total * 16;
+    TR_CUDA(cudaMemcpyAsync(chain, rgba8, (size_t)width * height * 4, cudaMemcpyHostToDevice, c->stream));
+    d.base = buf.as<float4>();
+    TR_TRY(launch_texture_chain(c->tex_tables.as<TexTables>(), d, chain, c->sm_count, c->stream));
+    bind_texture(c, index, d);
     return TR_OK;
 }
 
@@ -1285,6 +1324,22 @@ int32_t tr_wait_readback(tr_ctx* c) {
     TR_CHECK_CTX(c);
     if (c->copy_pending) TR_CUDA(cudaEventSynchronize(c->ev_copy_done));
     return check_device_status(c, "tr_wait_readback");  // an overflowed visibility pass must not pass for a good frame
+}
+
+int32_t tr_read_texture_level(tr_ctx* c, uint32_t index, uint32_t level, float* rgba32f, uint32_t* w, uint32_t* h) {
+    TR_CHECK_CTX(c);
+    if (index >= TR_MAX_IMAGES) return fail(TR_ERR_INVALID_ARG, "tr_read_texture_level: image %u of at most %u", index, TR_MAX_IMAGES);
+    const trd::TexDesc& d = c->h_tex[index];
+    if (!d.base) return fail(TR_ERR_STATE, "tr_read_texture_level: image %u is not bound", index);
+    if (level >= d.levels) return fail(TR_ERR_INVALID_ARG, "tr_read_texture_level: level %u of %u", level, d.levels);
+    const uint32_t lw = d.w >> level ? d.w >> level : 1u, lh = d.h >> level ? d.h >> level : 1u;
+    if (w) *w = lw;
+    if (h) *h = lh;
+    if (rgba32f) {
+        TR_CUDA(cudaMemcpyAsync(rgba32f, d.base + d.off[level], (size_t)lw * lh * 16, cudaMemcpyDeviceToHost, c->stream));
+        TR_CUDA(cudaStreamSynchronize(c->stream));
+    }
+    return TR_OK;
 }
 
 int32_t tr_mip_levels(tr_ctx* c, uint32_t* levels) {

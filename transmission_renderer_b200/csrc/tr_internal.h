@@ -85,8 +85,10 @@ struct tr_ctx {
     bool have_uniforms = false;
     tr::DevBuf lut;
     uint32_t lut_w = 0, lut_h = 0;
-    // material textures (row N2): decoded RGBA32F texels per image, descriptor table on the device
-    tr::DevBuf tex_data[TR_MAX_IMAGES], tex_table;
+    // material textures (row N2): decoded RGBA32F texels per image, descriptor table on the device.  An image bound by
+    // tr_set_texture_async also holds the RGBA8 bytes of its levels behind the texels (k_textures.cu); tex_tables is the
+    // device copy of texture_tables() those calls read, uploaded by the first one.
+    tr::DevBuf tex_data[TR_MAX_IMAGES], tex_table, tex_tables;
     trd::TexDesc h_tex[TR_MAX_IMAGES] = {};
     uint32_t n_textures = 0;          // highest bound index + 1
     bool tex_table_dirty = false;
@@ -247,6 +249,17 @@ int32_t launch_chunk_spheres(tr_ctx* c);
 int32_t accel_refit_blas(tr_ctx* c);
 constexpr int kChunkSphereLaunches = 1;
 constexpr int kRefitLaunches = 2;
+// The decode and encode tables of the material images (k_textures.cu), built once on the host: the float tables of the
+// store, which tr_set_texture uses too, and the float64 decode tables and sRGB encode thresholds of the device mip chain.
+struct TexTables {
+    double dec64[2][256];   // [0] sRGB colour -> linear, [1] v / 255.0 (alpha, UNORM)
+    double encode[256];     // encode[k - 1]: the least x whose sRGB byte is >= k; encode[255] = 2.0
+    float dec32[2][256];    // the store's texels: (float) of dec64[0], and (float)v / 255.0f
+};
+const TexTables& texture_tables();
+// tr_set_texture_async: level 0 from the bytes at `chain` (already in stream order) into d.base, then levels 1 .. d.levels - 1
+// (bytes and texels); d.levels launches
+int32_t launch_texture_chain(const TexTables* d_tables, const trd::TexDesc& d, uint8_t* chain, int sm_count, cudaStream_t s);
 int32_t launch_trace_rays(tr_ctx* c, uint32_t n, const float* d_origins, const float* d_directions, const float* d_t_max, uint8_t* d_lit);
 int32_t launch_generate_mips(uint2* pyramid, uint32_t levels, const uint32_t* w, const uint32_t* h, const uint32_t* off,
                              uint32_t* counter, int sm_count, cudaStream_t s);

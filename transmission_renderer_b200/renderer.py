@@ -117,9 +117,31 @@ class Renderer:
         _check(_lib().tr_set_texture(self._ctx, C.c_uint32(index), ptrs, C.c_uint32(len(lv)), C.c_uint32(lv[0].shape[1]),
                                      C.c_uint32(lv[0].shape[0]), C.c_int32(1 if srgb else 0)))
 
-    def set_textures(self, textures):
+    def set_texture_async(self, index, rgba8, srgb, n_levels=0):
+        """rgba8: (h, w, 4) uint8, level 0 only; levels 1 .. n_levels - 1 (0: the full chain) are built on the device in
+        stream order, bit-equal to set_texture(scenes.make_mips(rgba8, srgb)).  A page-locked array is read in stream order
+        (keep it alive and unchanged until the stream has passed the call); a pageable one is copied during the call."""
+        a = np.asarray(rgba8)
+        if a.dtype != np.uint8 or a.ndim != 3 or a.shape[2] != 4 or not a.flags.c_contiguous:
+            a = _c(a, np.uint8).reshape(a.shape[0], a.shape[1], 4)
+        _check(_lib().tr_set_texture_async(self._ctx, C.c_uint32(index), _p(a), C.c_uint32(a.shape[1]), C.c_uint32(a.shape[0]),
+                                           C.c_int32(1 if srgb else 0), C.c_uint32(n_levels)))
+
+    def read_texture_level(self, index, level):
+        """(h, w, 4) float32: level `level` of image `index` as the samplers read it (decoded to linear)."""
+        w, h = C.c_uint32(0), C.c_uint32(0)
+        _check(_lib().tr_read_texture_level(self._ctx, C.c_uint32(index), C.c_uint32(level), None, C.byref(w), C.byref(h)))
+        a = np.zeros((h.value, w.value, 4), np.float32)
+        _check(_lib().tr_read_texture_level(self._ctx, C.c_uint32(index), C.c_uint32(level), _p(a), C.byref(w), C.byref(h)))
+        return a
+
+    def set_textures(self, textures, on_device=False):
+        """on_device: bind only each levels[0] (set_texture_async) and let the device build the chains."""
         for i, t in enumerate(textures):
-            self.set_texture(i, t["levels"], t["srgb"])
+            if on_device:
+                self.set_texture_async(i, t["levels"][0], t["srgb"])
+            else:
+                self.set_texture(i, t["levels"], t["srgb"])
 
     def set_mesh(self, positions, normals, uvs, indices):
         p, n, u, i = _c(positions, np.float32), _c(normals, np.float32), _c(uvs, np.float32), _c(indices, np.uint32)
