@@ -381,9 +381,28 @@ TR_API int32_t tr_sync(tr_ctx* ctx);
 /* ------------------------------------------------------------------ */
 /* Uploads — replace the descriptor writes, src/main.rs:715-828         */
 /* ------------------------------------------------------------------ */
+/* Device sources.  tr_set_lights, tr_update_mesh_vertices and tr_update_instance_transforms also take their arrays in device
+ * memory (the context's device, another device, or managed memory), so a pose or a light set computed on the GPU goes in
+ * without a copy through the host.  A device source is read on the context stream at the point of the call: its producer
+ * must be ordered before that point, either by running on the context stream (tr_set_stream) or by an event the caller
+ * makes the context stream wait for.  It may be reused once the context stream has passed the call.  None of these calls
+ * waits for the device, and none allocates except when a buffer grows.  The members of a group are updated one by one, as
+ * for the other uploads; a source on another device of the group is read with the same copy. */
 TR_API int32_t tr_set_instances(tr_ctx* ctx, const tr_instance* instances, uint32_t n);      /* set1/b0, main.rs:2527 */
+/* The instance write of --rotate-model (src/main.rs:1263-1345) for instances whose ids do not change: replaces the transform of
+ * instances [first, first + n) and keeps their primitive_id and material_id, so unlike tr_set_instances it needs no host copy
+ * of the records.  The source may be pageable, page-locked or device memory (see "Device sources"); a host source is copied
+ * into a staging buffer of the context first (grow-only), a device one is read in place.  Stream-ordered on the context
+ * stream: the frame enqueued before the call sees the old transforms, the next one the new.  As after tr_set_instances, a
+ * traced frame then fails with TR_ERR_STATE until tr_update_top_level_acceleration_structure(_async) has run.  Non-finite
+ * values are accepted.  Errors: a range past the instance count, or a null pointer with n > 0: TR_ERR_INVALID_ARG; a rejected
+ * call changes nothing; n = 0: nothing.  Each call launches 1 kernel (tr_launch_count). */
+TR_API int32_t tr_update_instance_transforms(tr_ctx* ctx, uint32_t first, uint32_t n, const tr_packed_similarity* transforms);
 TR_API int32_t tr_set_primitives(tr_ctx* ctx, const tr_primitive_info* prims, uint32_t n);   /* set0/b7 + cull set/b0 */
 TR_API int32_t tr_set_materials(tr_ctx* ctx, const tr_material_info* materials, uint32_t n); /* set0/b2 */
+/* Host sources follow the upload rule (pageable: copied during the call; page-locked: read in stream order, ahead of the
+ * frame in flight, see INTEGRATION.md section 3).  A device source is copied on the context stream (see "Device sources"); of
+ * two calls before one frame, host or device in either order, the later one wins. */
 TR_API int32_t tr_set_lights(tr_ctx* ctx, const tr_light* lights, uint32_t n);               /* set2/b0, main.rs:472-478 */
 TR_API int32_t tr_set_uniforms(tr_ctx* ctx, const tr_uniforms* uniforms);                    /* set0/b3, main.rs:1231 */
 /* set0/b0[ggx_lut_texture_index]: RGBA8 UNORM, one mip (main.rs:295-330). */
@@ -416,10 +435,11 @@ TR_API int32_t tr_read_texture_level(tr_ctx* ctx, uint32_t index, uint32_t level
 /* vertex bindings 0..2 + index buffer (pipelines.rs:291-307, main.rs:2516-2557). */
 TR_API int32_t tr_set_mesh(tr_ctx* ctx, const float* positions, const float* normals, const float* uvs,
                            uint32_t n_vertices, const uint32_t* indices, uint32_t n_indices);
-/* Vertex animation (skinning, morph targets, cloth, procedural displacement computed on the host): replaces the positions and
- * normals [n*3] of vertices [first_vertex, first_vertex + n) of the mesh of tr_set_mesh; indices, uvs and the vertex count
- * stay.  Stream-ordered on the context stream: the frame enqueued before the call sees the old vertices, the next one the new.
- * Sources follow the upload rule (pageable: copied during the call; page-locked: read in stream order).  On the device, in
+/* Vertex animation (skinning, morph targets, cloth, procedural displacement computed on the host or the GPU): replaces the
+ * positions and normals [n*3] of vertices [first_vertex, first_vertex + n) of the mesh of tr_set_mesh; indices, uvs and the
+ * vertex count stay.  Stream-ordered on the context stream: the frame enqueued before the call sees the old vertices, the next
+ * one the new.  Host sources follow the upload rule (pageable: copied during the call; page-locked: read in stream order);
+ * device sources are read in stream order too (see "Device sources"); each pointer is classified on its own.  On the device, in
  * stream order, it recomputes the culling spheres of the binning pass and, once tr_build_acceleration_structures has run,
  * refits the bottom-level structures (same topology, new boxes and triangles); the top level then needs an update
  * (tr_update_top_level_acceleration_structure(_async)) before the next traced frame, which otherwise fails with

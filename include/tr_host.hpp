@@ -368,6 +368,15 @@ public:
         TR_HOST_CHECK(tr_update_mesh_vertices(ctx_, first_vertex, (uint32_t)(positions.size() / 3), positions.data(), normals.data()));
     }
     void set_instances(const std::vector<tr_instance>& v) { TR_HOST_CHECK(tr_set_instances(ctx_, v.data(), (uint32_t)v.size())); }
+    // the instance write of --rotate-model (src/main.rs:1263-1345) with unchanged ids: new transforms for instances
+    // [first, first + n) in stream order; with ray queries, update the top level (update_top_level_acceleration_structure_async)
+    // before the next frame.  `transforms` may also point to device memory (tr_abi.h, "Device sources").
+    void update_instance_transforms(const tr_packed_similarity* transforms, uint32_t n, uint32_t first = 0) {
+        TR_HOST_CHECK(tr_update_instance_transforms(ctx_, first, n, transforms));
+    }
+    void update_instance_transforms(const std::vector<tr_packed_similarity>& v, uint32_t first = 0) {
+        update_instance_transforms(v.empty() ? nullptr : v.data(), (uint32_t)v.size(), first);
+    }
     void set_primitives(const std::vector<tr_primitive_info>& v) { TR_HOST_CHECK(tr_set_primitives(ctx_, v.data(), (uint32_t)v.size())); }
     void set_materials(const std::vector<tr_material_info>& v) { TR_HOST_CHECK(tr_set_materials(ctx_, v.data(), (uint32_t)v.size())); }
     void set_lights(const std::vector<tr_light>& v) { TR_HOST_CHECK(tr_set_lights(ctx_, v.empty() ? nullptr : v.data(), (uint32_t)v.size())); }

@@ -20,7 +20,7 @@ _LIB = None
 # every symbol include/tr_abi.h declares (checked by tests/test_abi_symbols.py)
 EXPORTS = [
     "tr_create", "tr_destroy", "tr_resize", "tr_set_band", "tr_last_error", "tr_version", "tr_set_stream", "tr_sync",
-    "tr_set_instances", "tr_set_primitives", "tr_set_materials", "tr_set_lights", "tr_set_uniforms", "tr_set_ggx_lut", "tr_set_texture", "tr_set_texture_async",
+    "tr_set_instances", "tr_update_instance_transforms", "tr_set_primitives", "tr_set_materials", "tr_set_lights", "tr_set_uniforms", "tr_set_ggx_lut", "tr_set_texture", "tr_set_texture_async",
     "tr_read_texture_level",
     "tr_set_mesh", "tr_update_mesh_vertices", "tr_read_chunk_spheres", "tr_build_acceleration_structures", "tr_build_acceleration_structures_async",
     "tr_update_top_level_acceleration_structure", "tr_update_top_level_acceleration_structure_async", "tr_trace_shadow_rays",

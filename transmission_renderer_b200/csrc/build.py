@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 OUT = os.path.join(PKG, "libtr.so")
-SOURCES = ["tr_api.cu", "tr_comm.cu", "tr_group.cu", "k_shade.cu", "k_shade_shadow.cu", "k_accel.cu", "k_accel_device.cu", "k_accel_build.cu", "k_mesh_update.cu", "k_textures.cu", "k_mips.cu", "k_tonemap.cu", "k_eval.cu",
+SOURCES = ["tr_api.cu", "tr_comm.cu", "tr_group.cu", "k_shade.cu", "k_shade_shadow.cu", "k_accel.cu", "k_accel_device.cu", "k_accel_build.cu", "k_mesh_update.cu", "k_instances.cu", "k_textures.cu", "k_mips.cu", "k_tonemap.cu", "k_eval.cu",
            "k_cull.cu", "k_clusters.cu", "k_visibility.cu", "k_peak.cu"]
 HEADERS = ["tr_internal.h", "tr_device_math.cuh", "tr_device_pbr.cuh", "tr_device_accel.cuh", "tr_device_build.cuh",
            os.path.join("..", "..", "include", "tr_abi.h")]

@@ -505,7 +505,7 @@ int32_t tr_destroy(tr_ctx* c) {
                       &c->draws[2], &c->draws[3], &c->work_prefix, &c->slot_z, &c->slot_first, &c->block_entry, &c->chunk_spheres, &c->prim_chunk_base, &c->cluster_aabbs, &c->cluster_counts,
                       &c->cluster_indices, &c->vis[0], &c->vis[1], &c->bin_entries, &c->bin_state, &c->tri_records, &c->dev_status, &c->band_list, &c->hdr, &c->hdr_f32, &c->pyramid,
                       &c->srgb8, &c->mip_counter, &c->shade_counter, &c->accel_tlas, &c->accel_blas, &c->accel_inst, &c->accel_tris,
-                      &c->accel_prim_table, &c->accel_scratch, &c->accel_build_scratch, &c->accel_refit, &c->shadow_mask[0], &c->shadow_mask[1]};
+                      &c->accel_prim_table, &c->accel_scratch, &c->accel_build_scratch, &c->accel_refit, &c->shadow_mask[0], &c->shadow_mask[1], &c->transform_staging};
     for (DevBuf* b : bufs) b->release();
     for (DevBuf& b : c->tex_data) b.release();
     c->tex_table.release();
@@ -580,9 +580,24 @@ int32_t tr_sync(tr_ctx* c) {
 }
 
 // ------------------------------------------------------------------ uploads
-static int32_t upload(tr_ctx* c, DevBuf& b, const void* src, size_t bytes) {
+// Where a source of tr_update_mesh_vertices / tr_set_lights / tr_update_instance_transforms lives.  kLocal: memory a
+// kernel on the context's device may read in place (its own device memory, managed memory); kPeer: another device's memory,
+// which only a copy reads (peer access may be off).  Both device kinds are read on the context stream, in stream order.
+enum SourceKind { kHost, kLocal, kPeer };
+static SourceKind source_kind(const tr_ctx* c, const void* p) {
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, p) != cudaSuccess) {
+        cudaGetLastError();
+        return kHost;
+    }
+    if (attr.type == cudaMemoryTypeManaged) return kLocal;
+    if (attr.type == cudaMemoryTypeDevice) return attr.device == c->device ? kLocal : kPeer;
+    return kHost;
+}
+
+static int32_t upload(tr_ctx* c, DevBuf& b, const void* src, size_t bytes, cudaMemcpyKind kind = cudaMemcpyHostToDevice) {
     TR_TRY(b.ensure(bytes));
-    if (bytes) TR_CUDA(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, c->stream));
+    if (bytes) TR_CUDA(cudaMemcpyAsync(b.p, src, bytes, kind, c->stream));
     return TR_OK;
 }
 
@@ -622,6 +637,29 @@ int32_t tr_set_instances(tr_ctx* c, const tr_instance* instances, uint32_t n) {
     c->tri_bound_valid = false;
     c->cull_valid = false;
     c->accel_tlas_valid = false;  // src/main.rs:1263-1345: an instance write is followed by a top-level update
+    return TR_OK;
+}
+
+// Only the transforms move, so nothing the host holds about the instances changes (ids, the triangle bound, the top-level
+// count, validate_scene).  A source the kernel may read in place (device memory of this device, 16-byte aligned) is
+// scattered straight into the instance buffer; any other one is first copied contiguously into the staging buffer, on the
+// same stream: one copy of n * 32 bytes, where a 2D copy of 32-byte rows straight into the records would crawl over PCIe.
+int32_t tr_update_instance_transforms(tr_ctx* c, uint32_t first, uint32_t n, const tr_packed_similarity* transforms) {
+    TR_CHECK_CTX(c);
+    if ((uint64_t)first + n > c->n_instances)
+        return fail(TR_ERR_INVALID_ARG, "tr_update_instance_transforms: instances [%u, %u + %u) of %u", first, first, n, c->n_instances);
+    if (n == 0) return TR_OK;
+    if (!transforms) return fail(TR_ERR_INVALID_ARG, "tr_update_instance_transforms: null");
+    const SourceKind kind = source_kind(c, transforms);
+    const tr_packed_similarity* src = transforms;
+    if (kind != kLocal || ((uintptr_t)transforms & 15u)) {
+        const size_t bytes = (size_t)n * sizeof(tr_packed_similarity);
+        TR_TRY(upload(c, c->transform_staging, transforms, bytes, kind == kHost ? cudaMemcpyHostToDevice : cudaMemcpyDefault));
+        src = c->transform_staging.as<tr_packed_similarity>();
+    }
+    TR_TRY(launch_instance_transforms(c, first, n, src));
+    c->cull_valid = false;
+    c->accel_tlas_valid = false;   // as after tr_set_instances: the top level needs an update before the next traced frame
     return TR_OK;
 }
 
@@ -677,7 +715,12 @@ int32_t tr_set_materials(tr_ctx* c, const tr_material_info* materials, uint32_t 
 int32_t tr_set_lights(tr_ctx* c, const tr_light* lights, uint32_t n) {
     TR_CHECK_CTX(c);
     if (n && !lights) return fail(TR_ERR_INVALID_ARG, "tr_set_lights: null");
-    TR_TRY(upload_ahead(c, c->lights, c->lights_alt, c->lights_uploaded, c->ev_lights_ready, lights, (size_t)n * sizeof(tr_light)));
+    // A device source is copied on the context stream, after whatever produced it there, into the buffer the next frame
+    // reads: behind a run-ahead upload of this frame too, since the context stream already waits for that copy.
+    if (n && source_kind(c, lights) != kHost)
+        TR_TRY(upload(c, c->lights, lights, (size_t)n * sizeof(tr_light), cudaMemcpyDefault));
+    else
+        TR_TRY(upload_ahead(c, c->lights, c->lights_alt, c->lights_uploaded, c->ev_lights_ready, lights, (size_t)n * sizeof(tr_light)));
     c->n_lights = n;
     c->cluster_lights_valid = false;
     return TR_OK;
@@ -829,8 +872,10 @@ int32_t tr_update_mesh_vertices(tr_ctx* c, uint32_t first_vertex, uint32_t n, co
         return fail(TR_ERR_INVALID_ARG, "tr_update_mesh_vertices: vertices [%u, %u + %u) of %u", first_vertex, first_vertex, n, c->n_vertices);
     if (n == 0) return TR_OK;
     if (!positions || !normals) return fail(TR_ERR_INVALID_ARG, "tr_update_mesh_vertices: null");
-    TR_CUDA(cudaMemcpyAsync(c->mesh_pos.as<float>() + (size_t)first_vertex * 3, positions, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
-    TR_CUDA(cudaMemcpyAsync(c->mesh_nrm.as<float>() + (size_t)first_vertex * 3, normals, (size_t)n * 12, cudaMemcpyHostToDevice, c->stream));
+    const cudaMemcpyKind pk = source_kind(c, positions) == kHost ? cudaMemcpyHostToDevice : cudaMemcpyDefault;
+    const cudaMemcpyKind nk = source_kind(c, normals) == kHost ? cudaMemcpyHostToDevice : cudaMemcpyDefault;
+    TR_CUDA(cudaMemcpyAsync(c->mesh_pos.as<float>() + (size_t)first_vertex * 3, positions, (size_t)n * 12, pk, c->stream));
+    TR_CUDA(cudaMemcpyAsync(c->mesh_nrm.as<float>() + (size_t)first_vertex * 3, normals, (size_t)n * 12, nk, c->stream));
     if (c->chunks_valid) TR_TRY(launch_chunk_spheres(c));
     else TR_TRY(ensure_chunks(c));
     if (c->accel_blas_valid) {

@@ -153,6 +153,8 @@ struct tr_ctx {
     // stream, into the buffer the frame BEFORE the enqueued one read last, while the enqueued frame is still shading
     // (tr_api.cu upload_ahead).  A copy inside the compute stream costs two engine switches, ~40 us per upload.
     tr::DevBuf instances_alt, lights_alt;
+    // tr_update_instance_transforms: the contiguous copy of a host source (grow-only), read by the kernel in stream order
+    tr::DevBuf transform_staging;
     cudaStream_t upload_stream = nullptr;
     cudaEvent_t ev_frame_begin = nullptr, ev_inst_ready = nullptr, ev_lights_ready = nullptr;
     bool frame_begin_valid = false, inst_uploaded = false, lights_uploaded = false;   // the latter two: since the last tr_frame
@@ -249,6 +251,10 @@ int32_t launch_chunk_spheres(tr_ctx* c);
 int32_t accel_refit_blas(tr_ctx* c);
 constexpr int kChunkSphereLaunches = 1;
 constexpr int kRefitLaunches = 2;
+// tr_update_instance_transforms (k_instances.cu): the n similarities at `src` (device memory) into the transforms of
+// instances [first, first + n), ids kept; one launch
+int32_t launch_instance_transforms(tr_ctx* c, uint32_t first, uint32_t n, const tr_packed_similarity* src);
+constexpr int kInstanceTransformLaunches = 1;
 // The decode and encode tables of the material images (k_textures.cu), built once on the host: the float tables of the
 // store, which tr_set_texture uses too, and the float64 decode tables and sRGB encode thresholds of the device mip chain.
 struct TexTables {

@@ -30,6 +30,35 @@ def _c(a, dtype):
     return np.ascontiguousarray(a, dtype=dtype)
 
 
+def _device_rows(a, who, device, row_bytes, typestrs):
+    """(pointer, rows) of a device array (a CUDA torch tensor, or any object with `__cuda_array_interface__`) holding rows of
+    `row_bytes` bytes, or None when `a` is host data.  The array must be C-contiguous, of one of `typestrs` ('<f4': shape
+    (n, row_bytes / 4); '|u1': shape (n, row_bytes) or (n * row_bytes,)), and on `device` when it says where it lives (torch's
+    `.device.index`, CuPy's `.device.id`)."""
+    cai = getattr(a, "__cuda_array_interface__", None)
+    if cai is None:
+        return None
+    shape, typestr, strides = tuple(cai["shape"]), cai["typestr"], cai.get("strides")
+    if typestr not in typestrs:
+        raise TypeError(f"{who}: a device array of {typestr}; expected one of {', '.join(typestrs)}")
+    item = int(typestr[2:])
+    if typestr == "|u1" and len(shape) == 1 and shape[0] % row_bytes == 0:
+        rows = shape[0] // row_bytes
+    elif len(shape) == 2 and shape[1] * item == row_bytes:
+        rows = shape[0]
+    else:
+        raise ValueError(f"{who}: device array of shape {shape} and type {typestr} is not rows of {row_bytes} bytes")
+    if strides is not None and rows > 1 and tuple(strides) != tuple(item * int(np.prod(shape[k + 1:])) for k in range(len(shape))):
+        raise ValueError(f"{who}: the device array is not C-contiguous (strides {strides})")
+    dev = getattr(a, "device", None)
+    where = getattr(dev, "index", None)
+    if where is None:
+        where = getattr(dev, "id", None)
+    if where is not None and int(where) != device:
+        raise ValueError(f"{who}: the device array is on device {where}, the renderer on device {device}")
+    return (cai["data"][0] if rows else None), rows
+
+
 class _Config(C.Structure):
     _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("device", C.c_int32), ("band_y0", C.c_uint32),
                 ("band_y1", C.c_uint32), ("flags", C.c_uint32)]
@@ -51,6 +80,7 @@ class Renderer:
         cfg = _Config(self.width, self.height, device, y0, y1, abi.TR_FLAG_HDR_F32_DEBUG if f32_debug else 0)
         _check(_lib().tr_create(C.byref(cfg), C.byref(self._ctx)))
         self.f32_debug = f32_debug
+        self.device = int(device)
         self.acceleration_structure_address = 0   # the handle of the last build_acceleration_structures (RendererGroup.frame)
         self._keep = []
 
@@ -90,6 +120,20 @@ class Renderer:
         a = _c(instances, abi.instance)
         _check(_lib().tr_set_instances(self._ctx, _p(a), C.c_uint32(len(a))))
 
+    def update_instance_transforms(self, transforms, first=0):
+        """New transforms (the 32-byte packed similarity: translation_and_scale, rotation) for instances [first, first + n);
+        their primitive and material ids stay.  Stream-ordered; with ray queries, update the top level before the next
+        frame.  `transforms`: host data as (n, 8) float32, or a device array (a CUDA tensor or any object with
+        `__cuda_array_interface__`, on this renderer's device) of (n, 8) float32, (n, 32) uint8 or (n * 32,) uint8, read in
+        stream order on the context stream (order its producer before the call)."""
+        dev = _device_rows(transforms, "update_instance_transforms", self.device, 32, ("<f4", "|u1"))
+        if dev is not None:
+            ptr, n = dev
+        else:
+            a = _c(transforms, np.float32).reshape(-1, 8)
+            ptr, n = (a.ctypes.data if len(a) else None), len(a)
+        _check(_lib().tr_update_instance_transforms(self._ctx, C.c_uint32(first), C.c_uint32(n), C.c_void_p(ptr)))
+
     def set_primitives(self, primitives):
         a = _c(primitives, abi.primitive_info)
         _check(_lib().tr_set_primitives(self._ctx, _p(a), C.c_uint32(len(a))))
@@ -99,6 +143,14 @@ class Renderer:
         _check(_lib().tr_set_materials(self._ctx, _p(a), C.c_uint32(len(a))))
 
     def set_lights(self, lights):
+        """`lights`: abi.light records on the host, or a device array of their bytes (a CUDA tensor or any object with
+        `__cuda_array_interface__`, on this renderer's device): (n, 12) float32, (n, 48) uint8 or (n * 48,) uint8, copied in
+        stream order on the context stream (order its producer before the call)."""
+        dev = _device_rows(lights, "set_lights", self.device, abi.light.itemsize, ("<f4", "|u1"))
+        if dev is not None:
+            ptr, n = dev
+            _check(_lib().tr_set_lights(self._ctx, C.c_void_p(ptr), C.c_uint32(n)))
+            return
         a = _c(lights, abi.light)
         _check(_lib().tr_set_lights(self._ctx, _p(a) if len(a) else None, C.c_uint32(len(a))))
 
@@ -150,12 +202,22 @@ class Renderer:
     def update_mesh_vertices(self, positions, normals, first_vertex=0):
         """New positions and normals ((n, 3) float32 each) for vertices [first_vertex, first_vertex + n) of the mesh, in
         stream order: the culling spheres and, once built, the bottom-level acceleration structures follow on the device.
-        After it, a traced frame needs a top-level update first.  Page-locked arrays are read in stream order."""
-        p, n = _c(positions, np.float32).reshape(-1, 3), _c(normals, np.float32).reshape(-1, 3)
-        if len(p) != len(n):
-            raise ValueError(f"update_mesh_vertices: {len(p)} positions but {len(n)} normals")
-        _check(_lib().tr_update_mesh_vertices(self._ctx, C.c_uint32(first_vertex), C.c_uint32(len(p)), _p(p) if len(p) else None,
-                                              _p(n) if len(n) else None))
+        After it, a traced frame needs a top-level update first.  Page-locked arrays are read in stream order.  Either
+        array may instead be a device array ((n, 3) float32, C-contiguous, on this renderer's device: a CUDA tensor or any
+        object with `__cuda_array_interface__`), read in stream order on the context stream (order its producer before the
+        call); host and device arrays may be mixed."""
+        ptrs, counts, keep = [], [], []
+        for a in (positions, normals):
+            dev = _device_rows(a, "update_mesh_vertices", self.device, 12, ("<f4",))
+            if dev is None:
+                h = _c(a, np.float32).reshape(-1, 3)
+                keep.append(h)
+                dev = (h.ctypes.data if len(h) else None), len(h)
+            ptrs.append(C.c_void_p(dev[0]))
+            counts.append(dev[1])
+        if counts[0] != counts[1]:
+            raise ValueError(f"update_mesh_vertices: {counts[0]} positions but {counts[1]} normals")
+        _check(_lib().tr_update_mesh_vertices(self._ctx, C.c_uint32(first_vertex), C.c_uint32(counts[0]), *ptrs))
 
     def read_chunk_spheres(self):
         """(n, 4) float32: the binning pass's culling spheres (object-space centre, radius), one per 64 consecutive
