@@ -4,8 +4,9 @@
  *
  * The reference's host is one thread with one queue (src/main.rs:243, 1290-1294).  This host makes one context per visible
  * device (two on device 0 when there is only one), joins them into a group, which gives member k the k-th band of the frame,
- * and renders the frame of examples/frame.c through tr_group_frame.  The uploads go to every member, as they would go to
- * every GPU.  There is no CPU fallback: without a CUDA device tr_create fails and the program says so and exits with
+ * and renders the frame of examples/frame.c through tr_group_frame.  The scene is uploaded to member 0 only, and
+ * tr_group_replicate_scene copies it into the other members GPU to GPU, in stream order (uploading to every member, as to
+ * single contexts, works too).  There is no CPU fallback: without a CUDA device tr_create fails and the program says so and exits with
  * status 3.
  */
 #include <math.h>
@@ -111,11 +112,10 @@ int main(int argc, char** argv) {
             n++;
         }
     }
-    for (uint32_t k = 0; k < n; k++)
-        if (upload_scene(ctx[k], w, h)) return 3;
-
     tr_group* group = NULL;
     CHECK(tr_group_create(ctx, n, &group));
+    if (upload_scene(ctx[0], w, h)) return 3;
+    CHECK(tr_group_replicate_scene(group, 0, NULL));   /* no acceleration structures: no handles to collect */
 
     tr_frame_params f[MAX_MEMBERS];
     memset(f, 0, sizeof(f));

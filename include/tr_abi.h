@@ -630,7 +630,8 @@ TR_API int32_t tr_device_buffer(tr_ctx* ctx, int32_t what, void** device_ptr, si
 /* ------------------------------------------------------------------ */
 /* A group joins n contexts (at most 8) of one host thread into the bands of one frame.  Member k becomes rank k of n with
  * equal-row bands; its opaque pass stores its band into every member's mip 0 through plain device pointers (peer access
- * between distinct devices, which tr_group_create enables and leaves enabled), and CUDA events order the members, so no
+ * between distinct devices, which tr_group_create enables and leaves enabled, together with access to each device's default
+ * memory pool, from which tr_set_texture_async allocates), and CUDA events order the members, so no
  * call waits for the GPU inside a frame.  Contexts may share a device: 2..8 members on one GPU run exactly the code 8 GPUs
  * run.  Members must be distinct, of one size, and in no communicator (tr_comm_init), peer mapping (tr_peer_attach) or
  * other group.  While the group lives, tr_frame, tr_shade_opaque, tr_allgather_opaque, tr_set_band, tr_set_bands,
@@ -654,6 +655,24 @@ TR_API int32_t tr_group_frame(tr_group* g, const tr_frame_params* params);
 TR_API int32_t tr_group_sync(tr_group* g);
 /* the whole sRGB8 frame: every member's band into one width x height x 4 buffer */
 TR_API int32_t tr_group_read_srgb8(tr_group* g, uint8_t* rgba8);
+/* Copies member `source`'s scene, as its context stream sees it at the point of the call, into every other member, in
+ * stream order.  addresses[k] (n entries, may be null) receives member k's acceleration-structure handle, or 0 if the
+ * source has no valid top level.  Returns without waiting for the device, except where a destination buffer must grow,
+ * as for the other uploads.
+ * Copied: the mesh, primitives, materials, instances and lights (the buffers the source's next frame reads), uniforms,
+ * the cluster AABBs of tr_build_clusters, the GGX LUT, every bound material image (with its RGBA8 levels when bound by
+ * tr_set_texture_async), the culling spheres and, when the source has them, both acceleration-structure levels with their
+ * refit tables; also what the source holds on the host about all of these (no read-back).  A destination then behaves as
+ * a context that received the same uploads and builds: tr_update_mesh_vertices refits its trees, the top-level updates,
+ * tr_set_texture_async and tr_build_acceleration_structures_async work on it.  Not copied: frame targets, G-buffers,
+ * shadow masks, light lists, timers and streams.
+ * Ordering: each destination's stream waits for the source stream at the call, then copies (cudaMemcpyAsync, peer to
+ * peer or within one device); a frame a destination enqueued earlier reads the old scene.  The source stream then waits
+ * for every destination's copies, so uploads to the source after the call do not change what the destinations receive.
+ * No kernel is launched.  source >= n -> TR_ERR_INVALID_ARG; a source without a mesh -> TR_ERR_STATE; a rejected call
+ * changes no member; a group of one copies nothing.  A CUDA or allocation failure part-way leaves a destination with an
+ * empty scene (no mesh, no image, no structures), to be loaded again. */
+TR_API int32_t tr_group_replicate_scene(tr_group* g, uint32_t source, uint64_t* addresses);
 
 /* ------------------------------------------------------------------ */
 /* Diagnostics (benchmark support; not part of the reference surface)  */

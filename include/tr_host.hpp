@@ -496,6 +496,13 @@ public:
         TR_HOST_CHECK(tr_group_frame(group_, per_member.data()));
     }
     void sync() { TR_HOST_CHECK(tr_group_sync(group_)); }
+    // load member(source) only, then copy its scene into every other member, GPU to GPU in stream order
+    // (tr_group_replicate_scene); returns every member's acceleration-structure handle (0: the source has no valid top level)
+    std::vector<uint64_t> replicate_scene(uint32_t source = 0) {
+        std::vector<uint64_t> addresses(members_.size());
+        TR_HOST_CHECK(tr_group_replicate_scene(group_, source, addresses.data()));
+        return addresses;
+    }
     std::vector<uint8_t> read_srgb8() {   // the whole frame, every member's band
         std::vector<uint8_t> out((size_t)width_ * height_ * 4);
         TR_HOST_CHECK(tr_group_read_srgb8(group_, out.data()));

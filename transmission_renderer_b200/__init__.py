@@ -33,7 +33,7 @@ EXPORTS = [
     "tr_set_bands", "tr_comm_unique_id", "tr_comm_init", "tr_comm_destroy", "tr_peer_export", "tr_peer_attach", "tr_device_buffer",
     "tr_launch_count", "tr_raster_stats", "tr_measure_fp32_peak", "tr_measure_hbm_copy",
     "tr_group_create", "tr_group_destroy", "tr_group_set_bands", "tr_group_resize", "tr_group_frame", "tr_group_sync",
-    "tr_group_read_srgb8",
+    "tr_group_read_srgb8", "tr_group_replicate_scene",
 ]
 
 

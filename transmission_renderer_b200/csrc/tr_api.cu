@@ -771,11 +771,34 @@ static size_t texture_layout(trd::TexDesc* d, uint32_t width, uint32_t height, u
     return total;
 }
 
-static void bind_texture(tr_ctx* c, uint32_t index, trd::TexDesc d) {
+static size_t texture_texels(const trd::TexDesc& d) {
+    const uint32_t l = d.levels - 1, w = d.w >> l ? d.w >> l : 1u, h = d.h >> l ? d.h >> l : 1u;
+    return (size_t)d.off[l] + (size_t)w * h;
+}
+
+static void bind_texture(tr_ctx* c, uint32_t index, trd::TexDesc d, bool chain) {
     d.base = c->tex_data[index].as<float4>();
     c->h_tex[index] = d;
+    c->tex_chain[index] = chain;
     if (index + 1 > c->n_textures) c->n_textures = index + 1;
     c->tex_table_dirty = true;
+}
+
+// At least `need` bytes for image `index`, in stream order where it can be: a first bind allocates on the context stream
+// (unlike cudaMalloc, a stream-ordered allocation never waits for the device to reclaim freed memory); an allocation that
+// must grow waits for the frame in flight, which may still sample the old image.  The first bind takes the device's default
+// pool by name, whatever pool the host made current: that is the pool tr_group_create opens to the other members' devices
+// (peer access to pool memory follows cudaMemPoolSetAccess, not cudaDeviceEnablePeerAccess).
+static int32_t ensure_texture(tr_ctx* c, uint32_t index, size_t need) {
+    DevBuf& buf = c->tex_data[index];
+    if (buf.p && buf.bytes < need) TR_CUDA(cudaStreamSynchronize(c->stream));
+    if (!buf.p) {
+        cudaMemPool_t pool;
+        TR_CUDA(cudaDeviceGetDefaultMemPool(&pool, c->device));
+        TR_CUDA(cudaMallocFromPoolAsync(&buf.p, need, pool, c->stream));
+        buf.bytes = need;
+    }
+    return buf.ensure(need);
 }
 
 int32_t tr_set_texture(tr_ctx* c, uint32_t index, const uint8_t* const* levels, uint32_t n_levels, uint32_t width, uint32_t height,
@@ -805,7 +828,7 @@ int32_t tr_set_texture(tr_ctx* c, uint32_t index, const uint8_t* const* levels, 
     TR_CUDA(cudaStreamSynchronize(c->stream));  // a frame in flight may still sample the old image
     TR_TRY(c->tex_data[index].ensure(total * 16));
     TR_CUDA(cudaMemcpy(c->tex_data[index].p, texels.data(), total * 16, cudaMemcpyHostToDevice));
-    bind_texture(c, index, d);
+    bind_texture(c, index, d, false);
     return TR_OK;
 }
 
@@ -825,22 +848,17 @@ int32_t tr_set_texture_async(tr_ctx* c, uint32_t index, const uint8_t* rgba8, ui
     const size_t total = texture_layout(&d, width, height, n_levels ? n_levels : full, srgb);
     if (total > 0xffffffffull) return fail(TR_ERR_UNSUPPORTED, "tr_set_texture_async: more than 2^32 texels");
     const size_t need = total * 20;   // RGBA32F texels, then the RGBA8 bytes of every level
-    DevBuf& buf = c->tex_data[index];
-    if (buf.p && buf.bytes < need) TR_CUDA(cudaStreamSynchronize(c->stream));   // a frame in flight may still sample the old image
     if (!c->tex_tables.p) {
         TR_TRY(c->tex_tables.ensure(sizeof(TexTables)));
         TR_CUDA(cudaMemcpyAsync(c->tex_tables.p, &texture_tables(), sizeof(TexTables), cudaMemcpyHostToDevice, c->stream));
     }
-    if (!buf.p) {   // stream-ordered: unlike cudaMalloc, it never waits for the device to reclaim freed memory
-        TR_CUDA(cudaMallocAsync(&buf.p, need, c->stream));
-        buf.bytes = need;
-    }
-    TR_TRY(buf.ensure(need));
+    TR_TRY(ensure_texture(c, index, need));
+    DevBuf& buf = c->tex_data[index];
     uint8_t* chain = buf.as<uint8_t>() + total * 16;
     TR_CUDA(cudaMemcpyAsync(chain, rgba8, (size_t)width * height * 4, cudaMemcpyHostToDevice, c->stream));
     d.base = buf.as<float4>();
     TR_TRY(launch_texture_chain(c->tex_tables.as<TexTables>(), d, chain, c->sm_count, c->stream));
-    bind_texture(c, index, d);
+    bind_texture(c, index, d, true);
     return TR_OK;
 }
 
@@ -895,6 +913,122 @@ int32_t tr_read_chunk_spheres(tr_ctx* c, float* spheres, uint32_t capacity, uint
     TR_CUDA(cudaStreamSynchronize(c->stream));
     return TR_OK;
 }
+
+}  // extern "C"
+
+// ------------------------------------------------------------------ scene replication (tr_group_replicate_scene)
+// The host state of an empty scene: no counts, no bound image, nothing valid that a frame or a build would read.  The
+// device buffers stay allocated (grow-only).
+static void clear_scene(tr_ctx* c) {
+    c->n_vertices = c->n_indices = c->n_primitives = c->n_materials = c->n_instances = c->n_lights = 0;
+    c->have_uniforms = c->clusters_valid = c->cluster_lights_valid = false;
+    c->lut_w = c->lut_h = 0;
+    c->prims_alpha_clip = c->materials_textured = false;
+    for (uint32_t i = 0; i < TR_MAX_IMAGES; i++) {
+        c->h_tex[i] = trd::TexDesc{};
+        c->tex_chain[i] = false;
+    }
+    c->n_textures = 0;
+    c->tex_table_dirty = true;
+    for (std::vector<uint32_t>* v : {&c->h_prim_tris, &c->h_inst_prim, &c->h_inst_mat, &c->h_prim_first, &c->h_prim_count,
+                                     &c->h_chunk_base, &c->h_prim_root, &c->h_prim_tri_base, &c->h_prim_bucket})
+        v->clear();
+    c->n_chunks = 0;
+    c->chunks_valid = c->chunk_cull = false;
+    c->scene_checked = c->tri_bound_valid = c->cull_valid = false;
+    c->max_triangles = 0;
+    c->accel_blas_nodes = c->accel_n_tris = c->accel_n_instances = 0;
+    c->accel_blas_valid = c->accel_tlas_valid = false;
+}
+
+// One destination: every device buffer a frame reads is copied byte for byte on dst's stream (cudaMemcpyDefault: a peer
+// device or the same one), and the host state that describes those buffers is copied on the host, so dst ends as a context
+// that received the same uploads and builds.  The trees hold node and triangle indices, never pointers, so they are valid
+// at dst's addresses as they are; the texture descriptors hold absolute bases, so dst's table is rebuilt.  What is dst's
+// own stays: frame targets, G-buffers, shadow masks, light lists, cull outputs, timers, streams, scratch and the run-ahead
+// bookkeeping.  dst's host state is first set to an empty scene: a buffer that grows is freed before it is reallocated, so
+// a failure part-way (an allocation) leaves dst empty, to be loaded again, and never describing memory it no longer owns.
+int32_t tr::replicate_scene(tr_ctx* dst, const tr_ctx* src) {
+    const cudaMemcpyKind k = cudaMemcpyDefault;
+    clear_scene(dst);
+    TR_TRY(upload(dst, dst->mesh_pos, src->mesh_pos.p, (size_t)src->n_vertices * 12, k));
+    TR_TRY(upload(dst, dst->mesh_nrm, src->mesh_nrm.p, (size_t)src->n_vertices * 12, k));
+    TR_TRY(upload(dst, dst->mesh_uv, src->mesh_uv.p, (size_t)src->n_vertices * 8, k));
+    TR_TRY(upload(dst, dst->mesh_idx, src->mesh_idx.p, (size_t)src->n_indices * 4, k));
+    TR_TRY(upload(dst, dst->primitives, src->primitives.p, (size_t)src->n_primitives * sizeof(tr_primitive_info), k));
+    TR_TRY(upload(dst, dst->materials, src->materials.p, (size_t)src->n_materials * sizeof(tr_material_info), k));
+    TR_TRY(upload(dst, dst->instances, src->instances.p, (size_t)src->n_instances * sizeof(tr_instance), k));
+    TR_TRY(upload(dst, dst->lights, src->lights.p, (size_t)src->n_lights * sizeof(tr_light), k));
+    if (src->lut_w) TR_TRY(upload(dst, dst->lut, src->lut.p, (size_t)src->lut_w * src->lut_h * 2, k));
+    if (src->clusters_valid)
+        TR_TRY(upload(dst, dst->cluster_aabbs, src->cluster_aabbs.p, (size_t)src->n_clusters * sizeof(tr_cluster_aabb), k));
+    if (src->chunks_valid) {
+        TR_TRY(upload(dst, dst->prim_chunk_base, src->prim_chunk_base.p, src->h_chunk_base.size() * 4, k));
+        TR_TRY(upload(dst, dst->chunk_spheres, src->chunk_spheres.p, (size_t)src->n_chunks * 16, k));
+    }
+    if (src->accel_blas_valid) {
+        const size_t nn = src->accel_blas_nodes, nt = src->accel_n_tris;
+        TR_TRY(upload(dst, dst->accel_blas, src->accel_blas.p, nn * sizeof(trd::AccelNode), k));
+        TR_TRY(upload(dst, dst->accel_tris, src->accel_tris.p, nt * 3 * sizeof(float4), k));
+        TR_TRY(upload(dst, dst->accel_prim_table, src->accel_prim_table.p, (size_t)src->n_primitives * sizeof(trd::TlasPrim), k));
+        TR_TRY(upload(dst, dst->accel_refit, src->accel_refit.p, (nn * 2 + nt) * 4, k));   // parents, arrivals, triangle sources
+        if (src->accel_tlas_valid) {
+            const size_t m = src->accel_n_instances;
+            TR_TRY(upload(dst, dst->accel_tlas, src->accel_tlas.p, (m >= 2 ? m - 1 : 1) * sizeof(trd::AccelNode), k));
+            TR_TRY(upload(dst, dst->accel_inst, src->accel_inst.p, m * sizeof(trd::AccelInstance), k));
+        }
+    }
+    for (uint32_t i = 0; i < src->n_textures; i++) {   // an image unbound on the source stays unbound here (clear_scene)
+        const trd::TexDesc& d = src->h_tex[i];
+        if (!d.base) continue;
+        const size_t bytes = texture_texels(d) * (src->tex_chain[i] ? 20 : 16);
+        TR_TRY(ensure_texture(dst, i, bytes));
+        TR_CUDA(cudaMemcpyAsync(dst->tex_data[i].p, src->tex_data[i].p, bytes, k, dst->stream));
+        bind_texture(dst, i, d, src->tex_chain[i]);
+    }
+    dst->n_textures = src->n_textures;
+    dst->tex_table_dirty = true;
+
+    dst->n_vertices = src->n_vertices;
+    dst->n_indices = src->n_indices;
+    dst->n_primitives = src->n_primitives;
+    dst->n_materials = src->n_materials;
+    dst->n_instances = src->n_instances;
+    dst->n_lights = src->n_lights;
+    dst->uniforms = src->uniforms;
+    dst->have_uniforms = src->have_uniforms;
+    dst->n_clusters = src->n_clusters;
+    dst->clusters_valid = src->clusters_valid;
+    dst->cluster_lights_valid = false;   // as after tr_set_lights: the next frame assigns the new lights
+    dst->lut_w = src->lut_w;
+    dst->lut_h = src->lut_h;
+    dst->prims_alpha_clip = src->prims_alpha_clip;
+    dst->materials_textured = src->materials_textured;
+    dst->h_prim_tris = src->h_prim_tris;
+    dst->h_inst_prim = src->h_inst_prim;
+    dst->h_inst_mat = src->h_inst_mat;
+    dst->h_prim_first = src->h_prim_first;
+    dst->h_prim_count = src->h_prim_count;
+    dst->h_chunk_base = src->h_chunk_base;
+    dst->n_chunks = src->n_chunks;
+    dst->chunks_valid = src->chunks_valid;
+    dst->chunk_cull = src->chunk_cull;
+    dst->scene_checked = src->scene_checked;
+    dst->max_triangles = src->max_triangles;
+    dst->tri_bound_valid = src->tri_bound_valid;
+    dst->cull_valid = false;
+    dst->h_prim_root = src->h_prim_root;
+    dst->h_prim_tri_base = src->h_prim_tri_base;
+    dst->h_prim_bucket = src->h_prim_bucket;
+    dst->accel_blas_nodes = src->accel_blas_nodes;
+    dst->accel_n_tris = src->accel_n_tris;
+    dst->accel_n_instances = src->accel_n_instances;
+    dst->accel_blas_valid = src->accel_blas_valid;
+    dst->accel_tlas_valid = src->accel_blas_valid && src->accel_tlas_valid;
+    return TR_OK;
+}
+
+extern "C" {
 
 // ------------------------------------------------------------------ ray-queried shadows
 int32_t tr_build_acceleration_structures(tr_ctx* c, uint64_t* address) {

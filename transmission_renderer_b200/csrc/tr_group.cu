@@ -12,8 +12,14 @@
 //                 (its K6 no longer samples its mip 0, which r's K4 is about to write); K4; record r's FRONT event
 //       back   r: wait for every other member's FRONT event of this frame (every band is in r's mip 0); K5, K6; record
 //                 r's BACK event; K7
-//     Every wait names an event whose record call this thread has already made (the first frame's waits name events never
-//     recorded, which CUDA treats as complete), so no enqueued work depends on work not yet enqueued: nothing can deadlock.
+//   * replication (tr_group_replicate_scene): the source records its REPLICA event; each destination d waits for it, copies
+//     the scene on its own stream (tr_api.cu replicate_scene: copy engines only, from a peer device or the same one) and
+//     records d's REPLICA event; then the source waits for every destination's REPLICA event, so that a later upload to
+//     the source cannot overwrite what a copy is still reading.  A frame a destination enqueued before the call reads the
+//     old scene, its next frame the new one.
+//     Every wait, the frame's and the replication's, names an event whose record call this thread has already made (the
+//     first frame's waits name events never recorded, which CUDA treats as complete), so no enqueued work depends on work
+//     not yet enqueued: nothing can deadlock.
 #include <string.h>
 
 #include <new>
@@ -30,7 +36,10 @@ int32_t set_device(const tr_ctx* c) {
 }
 
 // Distinct devices store into each other's frames: peer access both ways.  "Already enabled" (by torch, or an earlier
-// group) is success; access stays enabled after the group, since the host process may rely on it.
+// group) is success; access stays enabled after the group, since the host process may rely on it.  Stream-ordered pool
+// memory does not follow cudaDeviceEnablePeerAccess: the images tr_set_texture_async allocates from each device's default
+// pool (tr_api.cu ensure_texture), which tr_group_replicate_scene copies across devices, so that pool is opened to the
+// other device too (read and write, both ways; it stays open, like peer access).
 int32_t enable_peer_access(int a, int b) {
     int ab = 0, ba = 0;
     TR_CUDA(cudaDeviceCanAccessPeer(&ab, a, b));
@@ -45,6 +54,13 @@ int32_t enable_peer_access(int a, int b) {
         if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();   // clears it
         else if (e != cudaSuccess)
             return fail(TR_ERR_CUDA, "tr_group_create: cudaDeviceEnablePeerAccess(%d -> %d): %s", from, to, cudaGetErrorString(e));
+        cudaMemPool_t pool;
+        TR_CUDA(cudaDeviceGetDefaultMemPool(&pool, to));
+        cudaMemAccessDesc access{};
+        access.location.type = cudaMemLocationTypeDevice;
+        access.location.id = from;
+        access.flags = cudaMemAccessFlagsProtReadWrite;
+        TR_CUDA(cudaMemPoolSetAccess(pool, &access, 1));   // `from` reads and writes `to`'s pool
     }
     return TR_OK;
 }
@@ -71,7 +87,8 @@ void destroy_events(tr_group* g) {
         cudaSetDevice(g->members[k]->device);
         if (g->ev_front[k]) cudaEventDestroy(g->ev_front[k]);
         if (g->ev_back[k]) cudaEventDestroy(g->ev_back[k]);
-        g->ev_front[k] = g->ev_back[k] = nullptr;
+        if (g->ev_replica[k]) cudaEventDestroy(g->ev_replica[k]);
+        g->ev_front[k] = g->ev_back[k] = g->ev_replica[k] = nullptr;
     }
 }
 
@@ -111,7 +128,8 @@ int32_t tr_group_create(tr_ctx* const* ctxs, uint32_t n, tr_group** out_group) {
         // a frame still in flight samples its own mip 0, which the other members' first opaque passes will write
         if (st == TR_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) st = fail(TR_ERR_CUDA, "tr_group_create: member %u's stream failed", k);
         if (st == TR_OK && (cudaEventCreateWithFlags(&g->ev_front[k], cudaEventDisableTiming) != cudaSuccess ||
-                            cudaEventCreateWithFlags(&g->ev_back[k], cudaEventDisableTiming) != cudaSuccess))
+                            cudaEventCreateWithFlags(&g->ev_back[k], cudaEventDisableTiming) != cudaSuccess ||
+                            cudaEventCreateWithFlags(&g->ev_replica[k], cudaEventDisableTiming) != cudaSuccess))
             st = fail(TR_ERR_CUDA, "tr_group_create: cudaEventCreate failed");
     }
     if (st != TR_OK) {
@@ -197,6 +215,41 @@ int32_t tr_group_frame(tr_group* g, const tr_frame_params* params) {
         TR_TRY(frame_back(c, &params[r], g->ev_back[r]));
     }
     return TR_OK;
+}
+
+int32_t tr_group_replicate_scene(tr_group* g, uint32_t source, uint64_t* addresses) {
+    if (!g) return fail(TR_ERR_INVALID_ARG, "tr_group_replicate_scene: null");
+    if (source >= (uint32_t)g->n) return fail(TR_ERR_INVALID_ARG, "tr_group_replicate_scene: source %u of %d members", source, g->n);
+    tr_ctx* s = g->members[source];
+    if (!s->mesh_pos.p) return fail(TR_ERR_STATE, "tr_group_replicate_scene: member %u has no mesh (tr_set_mesh)", source);
+    int32_t st = TR_OK;
+    if (g->n > 1) {
+        TR_TRY(set_device(s));
+        TR_CUDA(cudaEventRecord(g->ev_replica[source], s->stream));
+        int issued = 0;   // destinations [0, issued) may have copies in flight that read the source
+        for (int k = 0; k < g->n && st == TR_OK; k++) {
+            if (k == (int)source) continue;
+            tr_ctx* d = g->members[k];
+            st = set_device(d);
+            if (st == TR_OK && cudaStreamWaitEvent(d->stream, g->ev_replica[source], 0) != cudaSuccess)
+                st = fail(TR_ERR_CUDA, "tr_group_replicate_scene: member %d cannot wait for the source", k);
+            if (st != TR_OK) break;
+            st = replicate_scene(d, s);
+            issued = k + 1;
+            if (cudaEventRecord(g->ev_replica[k], d->stream) != cudaSuccess && st == TR_OK)
+                st = fail(TR_ERR_CUDA, "tr_group_replicate_scene: cudaEventRecord on member %d failed", k);
+        }
+        // later work on the source (an upload into a buffer a copy is still reading) waits for every copy
+        TR_TRY(set_device(s));
+        for (int k = 0; k < issued; k++)
+            if (k != (int)source) TR_CUDA(cudaStreamWaitEvent(s->stream, g->ev_replica[k], 0));
+    }
+    if (addresses)
+        for (int k = 0; k < g->n; k++) {
+            const tr_ctx* m = g->members[k];
+            addresses[k] = m->accel_blas_valid && m->accel_tlas_valid ? (uint64_t)(uintptr_t)m->accel_tlas.p : 0;
+        }
+    return st;
 }
 
 int32_t tr_group_sync(tr_group* g) {

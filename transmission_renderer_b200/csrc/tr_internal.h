@@ -90,6 +90,7 @@ struct tr_ctx {
     // device copy of texture_tables() those calls read, uploaded by the first one.
     tr::DevBuf tex_data[TR_MAX_IMAGES], tex_table, tex_tables;
     trd::TexDesc h_tex[TR_MAX_IMAGES] = {};
+    bool tex_chain[TR_MAX_IMAGES] = {};   // the image's allocation holds its RGBA8 levels behind the texels (bound async)
     uint32_t n_textures = 0;          // highest bound index + 1
     bool tex_table_dirty = false;
     bool prims_alpha_clip = false;    // some primitive uses draw buffer 1 or 3 (alpha clip): the rasteriser runs the alpha test
@@ -187,6 +188,8 @@ struct tr_group {
     tr_ctx* members[tr::kMaxPeers] = {};
     cudaEvent_t ev_front[tr::kMaxPeers] = {};  // recorded after member k's opaque pass (its band is in every mip 0)
     cudaEvent_t ev_back[tr::kMaxPeers] = {};   // recorded after member k's transmissive pass (done reading its mip 0)
+    // tr_group_replicate_scene: on the source, the point of the call; on a destination, the end of its copies
+    cudaEvent_t ev_replica[tr::kMaxPeers] = {};
 };
 
 namespace tr {
@@ -288,6 +291,9 @@ int32_t validate_scene(tr_ctx* c, const char* who);  // instance -> primitive / 
 void mat4_inverse_f64(const tr_mat4& m, tr_mat4* out);
 int32_t ensure_layer(tr_ctx* c, int layer, bool with_position);
 int32_t upload_texture_table(tr_ctx* c);  // descriptor table of the bound images -> device (if it changed)
+// tr_group_replicate_scene (tr_group.cu): src's scene into dst on dst's stream, which must already wait for the point of the
+// call on src's stream; copies only, no kernel
+int32_t replicate_scene(tr_ctx* dst, const tr_ctx* src);
 void band_of(const tr_ctx* c, int r, uint32_t* y0, uint32_t* y1);   // rows of rank r (tr_comm.cu)
 
 // tr_frame in pieces (tr_api.cu), shared with tr_group_frame (tr_group.cu):

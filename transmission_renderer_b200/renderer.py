@@ -628,6 +628,19 @@ class RendererGroup:
     def sync(self):
         _check(_lib().tr_group_sync(self._g))
 
+    # -- scene -------------------------------------------------------------------------------------------
+    def replicate_scene(self, source=0):
+        """Copies member `source`'s scene (everything its uploads and builds made, as its stream sees it now) into every
+        other member, GPU to GPU in stream order, without waiting for the device unless a buffer grows: load one member,
+        then replicate.  Returns every member's acceleration-structure handle (0 where the source has no valid top level),
+        which also becomes each member's `acceleration_structure_address`."""
+        n = len(self.renderers)
+        out = (C.c_uint64 * n)()
+        _check(_lib().tr_group_replicate_scene(self._g, C.c_uint32(source), out))
+        for r, a in zip(self.renderers, out):
+            r.acceleration_structure_address = int(a)
+        return [int(a) for a in out]
+
     # -- whole-frame reads ---------------------------------------------------------------------------
     def read_srgb8(self, out=None):
         a = np.zeros((self.height, self.width, 4), dtype=np.uint8) if out is None else out
